@@ -7,6 +7,7 @@ device-resident sampler kernel per GPU.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                   [--workload auto|config2|config3] [--scaling strong|weak] [--n-steps S] [--n-burn B]
+                  [--dump-outputs DIR]
 
   --gpus 1 (default)  BASELINE configs[1] = "config 2": 299 cells x 1 chain, n_burn=10000, n_steps=200000 (dram_kernel: one
                       CTA per chain).  Secondary legs in the same line: config 3 on one GPU (the N > 1 workload, and one fit
@@ -24,6 +25,10 @@ libtcmcmc); `e2e` = the same through the public call with HOST buffers, max-over
 
 --impl reference times the CPU restatement of the reference algorithm (oracle/, a C port: the reference is MATLAB +
 un-vendored mcmcstat and cannot run here) on the box's host cores on a bounded sample of the same workload.
+
+--dump-outputs DIR writes what the last timed fit returned to its caller as DIR/<name>.npy (float64): the per-chain
+posterior means and standard deviations, the sigma summaries and the decision counters.  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import glob
@@ -39,6 +44,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 GOLDEN = os.path.join(ROOT, "tests", "golden", "cells.npz")
 CSRC = [os.path.join(ROOT, "transcriptioncycleinference_b200", "csrc", f) for f in ("tc_mcmc.cu", "tc_device.cuh", "tc_warp.cuh")]
 METRIC = "mcmc_chain_steps_per_s"
@@ -70,7 +76,12 @@ def parse():
     ap.add_argument("--no-config5", action="store_true", help="skip the secondary N = 400 leg")
     ap.add_argument("--no-config3", action="store_true", help="skip the secondary config-3 legs of the one-GPU line")
     ap.add_argument("--no-writeback", action="store_true", help="skip the raw-chain write-back leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed fit to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if a.workload == "auto":
         a.workload = "config2" if world == 1 else "config3"
@@ -311,6 +322,8 @@ def run_ours(args, g):
             dt, ks, out = one_fit()
             e2e_s.append(dt); kernel_s.append(ks)
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs, _lib)
     tk, te = float(np.sum(kernel_s)), float(np.sum(e2e_s))
     if world > 1:
         tt = torch.tensor([tk, te], dtype=torch.float64, device="cuda")
@@ -396,6 +409,16 @@ def run_ours(args, g):
         dist.barrier()
         dist.destroy_process_group()
     return line if rank == 0 else None
+
+
+def dump_outputs(out, d, _lib):
+    """The summaries Cells.mcmc_run returned for every chain of the fit (gathered over the ranks under strong scaling; rank
+    0's own chains under weak scaling), as float64.  Counters past CNT_STATUS are SM cycle readings, not results, and are
+    left out; the others are exact in float64.  The largest workload, config3, comes to about 42 MB."""
+    os.makedirs(d, exist_ok=True)
+    arrs = dict(mean=out["mean"], std=out["std"], sig=out["sig"], counters=out["counters"][:, :_lib.CNT_STATUS + 1])
+    for name, a in arrs.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def config3_leg(cells, g, device, peak_dfma, flush, torch, n_steps, n_burn, fits):

@@ -15,19 +15,34 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
 
 
+def load_golden(stem):
+    """tests/golden/<stem>.npz merged with its parts <stem>.1.npz, <stem>.2.npz, ... (a fixture is split to keep every
+    file under 1 MB, tests/golden/make_golden.py); an array present in several parts is concatenated along its first
+    axis, in part order."""
+    out, path, k = {}, os.path.join(GOLDEN, stem + ".npz"), 1
+    while True:
+        with np.load(path) as z:
+            for key in z.files:
+                out[key] = np.concatenate([out[key], z[key]]) if key in out else z[key]
+        path = os.path.join(GOLDEN, "%s.%d.npz" % (stem, k))
+        if not os.path.exists(path):
+            return out
+        k += 1
+
+
 @pytest.fixture(scope="session")
 def cells_npz():
-    return dict(np.load(os.path.join(GOLDEN, "cells.npz")))
+    return load_golden("cells")
 
 
 @pytest.fixture(scope="session")
 def results_npz():
-    return dict(np.load(os.path.join(GOLDEN, "results.npz")))
+    return load_golden("results")
 
 
 @pytest.fixture(scope="session")
 def chains_npz():
-    return dict(np.load(os.path.join(GOLDEN, "chains.npz")))
+    return load_golden("chains")
 
 
 @pytest.fixture(scope="session")

@@ -1,14 +1,19 @@
 #!/usr/bin/env python
 """Generate the committed golden fixtures from the reference's own .mat files.
 
-Run HERE (the dev container, where /root/reference is mounted); the GPU box has
-no /root/reference, so the tests, smoke() and bench.py only ever read the .npz
-files this script writes next to itself.
+  python tests/golden/make_golden.py <checkout of the reference project>
 
-Sources (all MAT v5, read with scipy.io.loadmat):
-  /root/reference/TestScripts/TestData.mat                     -> cells.npz
-  /root/reference/TestScripts/28-Oct-2020-TestData.mat         -> results.npz
-  /root/reference/TestScripts/28-Oct-2020-TestData_RawChain.mat-> chains.npz
+The tests, smoke() and bench.py only ever read the .npz files this script writes
+next to itself, so they need no copy of the reference.
+
+Sources (all MAT v5, read with scipy.io.loadmat), relative to the reference checkout:
+  TestScripts/TestData.mat                      -> cells.npz
+  TestScripts/28-Oct-2020-TestData.mat          -> results.npz, results.1.npz
+  TestScripts/28-Oct-2020-TestData_RawChain.mat -> chains.npz, chains.1.npz
+
+A fixture larger than 1 MB is stored in parts, <stem>.npz, <stem>.1.npz, ...;
+tests/conftest.py:load_golden merges them back, concatenating an array that is
+split over several parts along its first axis.
 
 Layout of the packed ("ragged") arrays: cell c owns [off[c], off[c]+N[c]) of
 every per-timepoint array, off = exclusive cumulative sum of N.
@@ -30,8 +35,9 @@ import sys
 import numpy as np
 import scipy.io as sio
 
-REF = "/root/reference/TestScripts"
 HERE = os.path.dirname(os.path.abspath(__file__))
+RESULTS_PART1 = ("MS2_plot", "PP7_plot", "simMS2", "simPP7")     # stored in results.1.npz
+CHAINS_SPLIT = 150                                                # theta of cells [0, 150) in chains.npz, the rest in chains.1.npz
 
 SCALAR_FIELDS = [
     "mean_v", "sigma_v", "mean_ton", "sigma_ton", "mean_A", "sigma_A", "mean_tau",
@@ -41,11 +47,25 @@ SCALAR_FIELDS = [
 ]
 
 
-def main():
-    if not os.path.isdir(REF):
-        sys.exit("reference fixtures not mounted at " + REF)
+def save_results(out):
+    """results.npz + results.1.npz: the same arrays as one file would hold, each file under 1 MB."""
+    np.savez_compressed(os.path.join(HERE, "results.npz"), **{k: v for k, v in out.items() if k not in RESULTS_PART1})
+    np.savez_compressed(os.path.join(HERE, "results.1.npz"), **{k: out[k] for k in RESULTS_PART1})
 
-    d = sio.loadmat(os.path.join(REF, "TestData.mat"), mat_dtype=True)["data"]
+
+def save_chains(out):
+    """chains.npz + chains.1.npz: theta split by cell, each file under 1 MB."""
+    first = dict(out, theta=out["theta"][:CHAINS_SPLIT])
+    np.savez_compressed(os.path.join(HERE, "chains.npz"), **first)
+    np.savez_compressed(os.path.join(HERE, "chains.1.npz"), theta=out["theta"][CHAINS_SPLIT:])
+
+
+def main():
+    if len(sys.argv) != 2 or not os.path.isdir(os.path.join(sys.argv[1], "TestScripts")):
+        sys.exit("usage: make_golden.py <checkout of the reference project (with TestScripts/)>")
+    ref = os.path.join(sys.argv[1], "TestScripts")
+
+    d = sio.loadmat(os.path.join(ref, "TestData.mat"), mat_dtype=True)["data"]
     nc = d.shape[1]
     N = np.array([d[0, c]["time"].shape[1] for c in range(nc)], dtype=np.int32)
     off = np.zeros(nc + 1, dtype=np.int64)
@@ -57,7 +77,7 @@ def main():
     np.savez_compressed(os.path.join(HERE, "cells.npz"), N=N, off=off, t=t, ms2=ms2,
                         pp7=pp7, name=name)
 
-    r = sio.loadmat(os.path.join(REF, "28-Oct-2020-TestData.mat"), mat_dtype=True)
+    r = sio.loadmat(os.path.join(ref, "28-Oct-2020-TestData.mat"), mat_dtype=True)
     res, plot = r["MCMCresults"], r["MCMCplot"]
     out = {}
     for f in SCALAR_FIELDS:
@@ -69,9 +89,9 @@ def main():
     out["DatasetName"] = str(r["DatasetName"][0])
     out["field_order"] = np.array(res.dtype.names)
     out["plot_field_order"] = np.array(plot.dtype.names)
-    np.savez_compressed(os.path.join(HERE, "results.npz"), N=N, off=off, **out)
+    save_results(dict(N=N, off=off, **out))
 
-    ch = sio.loadmat(os.path.join(REF, "28-Oct-2020-TestData_RawChain.mat"),
+    ch = sio.loadmat(os.path.join(ref, "28-Oct-2020-TestData_RawChain.mat"),
                      mat_dtype=True)["MCMCchain"]
     nrow = ch[0, 0]["v_chain"].shape[0]
     npmax = 7 + int(N.max())
@@ -84,9 +104,8 @@ def main():
             theta[c, :, k] = ch[0, c][f][:, 0]
         theta[c, :, 7:7 + N[c]] = ch[0, c]["dR_chain"]
         s2[c] = ch[0, c]["s2chain"][:, 0]
-    np.savez_compressed(os.path.join(HERE, "chains.npz"), N=N, theta=theta, s2chain=s2,
-                        chain_field_order=np.array(ch.dtype.names))
-    for f in ("cells.npz", "results.npz", "chains.npz"):
+    save_chains(dict(N=N, theta=theta, s2chain=s2, chain_field_order=np.array(ch.dtype.names)))
+    for f in ("cells.npz", "results.npz", "results.1.npz", "chains.npz", "chains.1.npz"):
         print(f, os.path.getsize(os.path.join(HERE, f)), "bytes")
 
 
