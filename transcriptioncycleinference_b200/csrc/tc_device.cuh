@@ -411,11 +411,6 @@ __device__ __noinline__ void scan_counts_sequential(Cell cv, Vec th, double R, d
 // within 1e-7 of an integer — where a different association could flip a floor — lane 0 redoes the sum
 // sequentially.  Error bound of either order: (N-1) * eps * max(c) < 400 * 1.1e-16 * 3e4 << 1e-7, so the two paths
 // agree otherwise.
-#ifndef TC_SS_UNR
-#define TC_SS_UNR 1         // time points per lane per pass of the forward model (unroll-and-jam factor).  1: the smallest code — ss_eval
-                            // is 13 KB of SASS instead of 18.6 KB with 2, and the samplers' round (bounds, ss_eval, resolve, flush: ~33 KB with 2)
-                            // runs against a 32 KB instruction cache: config 2 +2 %, config 3 +1 % (measured); 4 doubles the code for no gain
-#endif
 template <class Cell, class Vec>
 __device__ __forceinline__ void scan_counts(const Cell &cv, const Vec &th, double R, double ton, const Work &w,
                                             bool force_sequential, bool want_n)
@@ -616,33 +611,27 @@ __device__ __noinline__ double ss_eval(const ConsX &C, Cell cv, Vec th, Work w, 
             //            that wanders to v -> 0, where the ramp spans every lag, is no slower than any other)
             //   plateau, lags [lb, min(lL-1, j)]:  whole polymerases -> exact count
             //   Branch-free: a part that is absent gets the index pair (0, 0), i.e. an empty prefix difference.
+            //   One time point per lane per pass, for the instruction cache: two made ss_eval 18.6 KB of SASS instead of 13 KB,
+            //   measured 2 % slower on config 2 and 1 % on config 3; four doubled the code for no gain.
 #pragma unroll 1
-            for (int jb = lane; jb < N; jb += 32 * TC_SS_UNR) {
-#pragma unroll
-                for (int u = 0; u < TC_SS_UNR; ++u) {
-                    const int j = jb + 32 * u;
-                    const bool in = j < N;
-                    const int jj = in ? j : 0;
-                    const double dj = (double)jj;
-                    const int lh1 = min(le1 - 1, jj), lh2 = min(le2 - 1, jj);
-                    const bool r1ok = lh1 >= la1, r2ok = lh2 >= la2;
-                    const bool p1ok = jj >= lb1 && lb1 < lL1, p2ok = jj >= lb2 && lb2 < lL2;
-                    const int a1i = r1ok ? jj - la1 + 1 : 0, b1i = r1ok ? jj - lh1 : 0;
-                    const int a2i = r2ok ? jj - la2 + 1 : 0, b2i = r2ok ? jj - lh2 : 0;
-                    const int p1a = p1ok ? jj - lb1 + 1 : 0, p1b = p1ok ? max(jj - lL1 + 1, 0) : 0;
-                    const int p2a = p2ok ? jj - lb2 + 1 : 0, p2b = p2ok ? max(jj - lL2 + 1, 0) : 0;
-                    const int *ks = tc_smem_i();
-                    const double dK1 = (double)(ks[w.K + a1i] - ks[w.K + b1i]), dS1 = (double)(ks[w.S + a1i] - ks[w.S + b1i]);
-                    const double dK2 = (double)(ks[w.K + a2i] - ks[w.K + b2i]), dS2 = (double)(ks[w.S + a2i] - ks[w.S + b2i]);
-                    const double pl1 = (double)(ks[w.K + p1a] - ks[w.K + p1b]), pl2 = (double)(ks[w.K + p2a] - ks[w.K + p2b]);
-                    double c1 = fma(f1, pl1, sc1 * (vd * (dj * dK1 - dS1) - s1 * dK1));
-                    double c2 = fma(f2, pl2, sc2 * (vd * (dj * dK2 - dS2) - s2 * dK2));
-                    if (s > 0) { c1 += tc_smem[w.F1 + jj]; c2 += tc_smem[w.F2 + jj]; }
-                    if (in) {
-                        tc_smem[w.F1 + j] = c1 < b1 ? b1 : c1;                  // :57
-                        tc_smem[w.F2 + j] = c2 < b2 ? b2 : c2;                  // :69
-                    }
-                }
+            for (int j = lane; j < N; j += 32) {
+                const double dj = (double)j;
+                const int lh1 = min(le1 - 1, j), lh2 = min(le2 - 1, j);
+                const bool r1ok = lh1 >= la1, r2ok = lh2 >= la2;
+                const bool p1ok = j >= lb1 && lb1 < lL1, p2ok = j >= lb2 && lb2 < lL2;
+                const int a1i = r1ok ? j - la1 + 1 : 0, b1i = r1ok ? j - lh1 : 0;
+                const int a2i = r2ok ? j - la2 + 1 : 0, b2i = r2ok ? j - lh2 : 0;
+                const int p1a = p1ok ? j - lb1 + 1 : 0, p1b = p1ok ? max(j - lL1 + 1, 0) : 0;
+                const int p2a = p2ok ? j - lb2 + 1 : 0, p2b = p2ok ? max(j - lL2 + 1, 0) : 0;
+                const int *ks = tc_smem_i();
+                const double dK1 = (double)(ks[w.K + a1i] - ks[w.K + b1i]), dS1 = (double)(ks[w.S + a1i] - ks[w.S + b1i]);
+                const double dK2 = (double)(ks[w.K + a2i] - ks[w.K + b2i]), dS2 = (double)(ks[w.S + a2i] - ks[w.S + b2i]);
+                const double pl1 = (double)(ks[w.K + p1a] - ks[w.K + p1b]), pl2 = (double)(ks[w.K + p2a] - ks[w.K + p2b]);
+                double c1 = fma(f1, pl1, sc1 * (vd * (dj * dK1 - dS1) - s1 * dK1));
+                double c2 = fma(f2, pl2, sc2 * (vd * (dj * dK2 - dS2) - s2 * dK2));
+                if (s > 0) { c1 += tc_smem[w.F1 + j]; c2 += tc_smem[w.F2 + j]; }
+                tc_smem[w.F1 + j] = c1 < b1 ? b1 : c1;                          // :57
+                tc_smem[w.F2 + j] = c2 < b2 ? b2 : c2;                          // :69
             }
         } else {
             SS_MARK(1);
@@ -660,27 +649,17 @@ __device__ __noinline__ double ss_eval(const ConsX &C, Cell cv, Vec th, Work w, 
     //     SumofSquares...m:51-64
     double acc = 0.0;
 #pragma unroll 1
-    for (int jb = lane; jb < N; jb += 32 * TC_SS_UNR) {
-        double pa[TC_SS_UNR];
-#pragma unroll
-        for (int u = 0; u < TC_SS_UNR; ++u) pa[u] = 0.0;
-#pragma unroll
-        for (int u = 0; u < TC_SS_UNR; ++u) {
-            const int j = jb + 32 * u;
-            const int jj = j < N ? j : 0;
-            const int k = j < N ? cv.ik(jj) : -1;                               // -1: outside the model grid (interp1 -> NaN)
-            const int kk = k >= 0 ? k : 0;
-            const double wj = cv.iw(jj);
-            const double m1 = A * tc_smem[w.F1 + kk], m1n = A * tc_smem[w.F1 + kk + 1];
-            double r1 = cv.ms2(jj) - (m1 + wj * (m1n - m1));
-            const double f2k = tc_smem[w.F2 + kk];
-            double r2 = cv.pp7(jj) - (f2k + wj * (tc_smem[w.F2 + kk + 1] - f2k));
-            r1 = (k >= 0 && r1 == r1) ? r1 : 0.0;                               // nansum
-            r2 = (k >= 0 && r2 == r2) ? r2 : 0.0;
-            pa[u] = fma(r2, r2, fma(r1, r1, pa[u]));
-        }
-#pragma unroll
-        for (int u = 0; u < TC_SS_UNR; ++u) acc += pa[u];
+    for (int j = lane; j < N; j += 32) {
+        const int k = cv.ik(j);                                                 // -1: outside the model grid (interp1 -> NaN)
+        const int kk = k >= 0 ? k : 0;
+        const double wj = cv.iw(j);
+        const double m1 = A * tc_smem[w.F1 + kk], m1n = A * tc_smem[w.F1 + kk + 1];
+        double r1 = cv.ms2(j) - (m1 + wj * (m1n - m1));
+        const double f2k = tc_smem[w.F2 + kk];
+        double r2 = cv.pp7(j) - (f2k + wj * (tc_smem[w.F2 + kk + 1] - f2k));
+        r1 = (k >= 0 && r1 == r1) ? r1 : 0.0;                                   // nansum
+        r2 = (k >= 0 && r2 == r2) ? r2 : 0.0;
+        acc += fma(r2, r2, fma(r1, r1, 0.0));               // the point's two squares, then one add (folding acc into the fma rounds differently)
     }
     SS_MARK(3);
     acc = warp_sum(acc);

@@ -53,19 +53,10 @@ struct DeviceGuard {
 #define RING 16            // ring of proposal increments: generated GEN_M steps at a time, ahead of use
 #define SS_WARPS 8
 #define SS_THREADS (32 * SS_WARPS)
-#ifndef SS_MIN_CTAS
 #define SS_MIN_CTAS 4          // 64 registers: 32 warps per SM hide the latency of streaming theta (measured +12 % over 2)
-#endif
-#ifndef TC_WARP_MIN_CHAINS_PER_SM
 #define TC_WARP_MIN_CHAINS_PER_SM 13  // chain-per-warp kernel from this many chains per SM on (measured crossover on B200: ~1 900 chains)
-#endif
-#ifndef TC_SOLO_LAG
 #define TC_SOLO_LAG 2       // dram_kernel: slices a chain must lag the mean progress by to get its SM to itself (0: never)
 #define TC_SOLO_NSEG 128    // ... and the number of time slices per chain then
-#endif
-#ifndef TC_CB_UNR
-#define TC_CB_UNR 1         // unroll factor of the bounds / prior loop of a round (phase A): 1 = smallest code (measured: +1 % on config 2 against 4)
-#endif
 #define COV_CR 32          // weighted rows of the covariance block staged per pass of the scatter update
 
 // development aid: cycle counts of sub-phases, chain 0 only (build with -DTC_SUBPROF; see scripts/subprof.py)
@@ -969,19 +960,6 @@ __device__ __noinline__ void emit_s2(const RunArgs &a, const ChainCtx &cx, S2Sta
 #define GENB_MAXT 7        // column tiles per warp: npar <= 8 * 8 * 7 = 448
 #define GENB_NS 4          // ring stages
 #define GENB_RPS 32        // tile rows per stage, at most (the short rows at the bottom of the triangle pack many to a stage)
-#ifndef GENB_COOP
-#define GENB_COOP 0        // 0: one bulk copy per stage by thread 0 (TmaRing); 1: stages filled by all threads with cp.async.cg
-                           // (CoopRing) — measured 12 % slower here: a stage of R is one contiguous 16-32 KB piece, ideal for a bulk copy
-#endif
-#if GENB_COOP
-#define GENB_RING CoopRing
-#define GENB_PRODUCER true
-#define GENB_FILL(g, src, n) { ring.begin(g); ring.copy(g, 0, src, (n) / 2); ring.commit(g); }
-#else
-#define GENB_RING TmaRing
-#define GENB_PRODUCER (tid == 0)
-#define GENB_FILL(g, src, n) ring.issue(g, src, 8u * (unsigned)(n));
-#endif
 // one k-step for the NA column tiles that still have rows: accumulator j belongs to the j-th tile from the TOP (so the live
 // ones are always a prefix and the code is straight-line: a conditional mma.sync costs a WARPSYNC each); `bt` = B fragment
 // of the top tile, tile j sits 256 j doubles before it.  EDGE: the lowest live tile (j = NA-1) is in its last k-step,
@@ -1035,7 +1013,7 @@ __device__ __noinline__ void gen_increments_tma(const ChainCtx &cx, int g0, int 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, npar = cx.npar;
     const int nt4 = (npar + 3) >> 2, NT = (npar + 7) >> 3;
     const int ar = lane >> 2, ak = lane & 3, th = ar >> 2, inner = 4 * ak + (ar & 3);
-    GENB_RING<GENB_NS> ring;
+    TmaRing<GENB_NS> ring;      // a bulk copy per stage (one contiguous 16-32 KB piece): cp.async.cg fills measured 12 % slower here
     // the stages fill the per-warp areas (Z lives in the ring slots); one tile of room before the first stage and two after
     // the last row of a stage: the fragment reads of a half-stored tile pair fall there and are discarded
     const int sst = ((SPEC * cx.wsz - 16) / GENB_NS) & ~1, cap = sst - 32;
@@ -1047,11 +1025,11 @@ __device__ __noinline__ void gen_increments_tma(const ChainCtx &cx, int g0, int 
     {                                                                                                       \
         int kend__ = pk, used__ = 0;                                                                        \
         while (kend__ < nt4 && kend__ - pk < GENB_RPS && used__ + 16 * (nt4 - kend__) <= cap) { used__ += 16 * (nt4 - kend__); ++kend__; } \
-        GENB_FILL(pg, src, used__)                      /* consecutive tile rows are contiguous: ONE segment */ \
+        ring.issue(pg, src, 8u * (unsigned)used__);     /* consecutive tile rows are contiguous: ONE segment */ \
         src += used__; pk = kend__;                                                                         \
         ++pg;                                                                                               \
     }
-    if (GENB_PRODUCER)
+    if (tid == 0)
         while (pk < nt4 && pg < GENB_NS - 2) GENB_ISSUE()
     double acc[GENB_MAXT][4];
 #pragma unroll
@@ -1068,7 +1046,7 @@ __device__ __noinline__ void gen_increments_tma(const ChainCtx &cx, int g0, int 
 #pragma unroll 1
     for (int g = 0; kk < nt4; ++g) {
         GSP_T0;
-        if (GENB_PRODUCER && pk < nt4) GENB_ISSUE()
+        if (tid == 0 && pk < nt4) GENB_ISSUE()
         GSP(28);
         int kend = kk, used = 0;                                    // the rows of stage g: the producer's packing rule
         while (kend < nt4 && kend - kk < GENB_RPS && used + 16 * (nt4 - kend) <= cap) { used += 16 * (nt4 - kend); ++kend; }
@@ -1120,14 +1098,8 @@ __device__ __noinline__ void gen_increments_tma(const ChainCtx &cx, int g0, int 
 //      FP64 tensor cores ([8 x npar] x [npar x npar] as mma.sync m8n8k4, A rows = the new steps, 4 interleaved
 //      accumulator sets).  Every element of R is needed exactly once per call, so R is not staged as a matrix:
 //      each lane pulls its own B elements HBM/L2 -> shared memory with 8-byte cp.async into private staging slots,
-//      two groups of 8 k-steps in flight.
-#ifndef TC_TMA_ALL
-#define TC_TMA_ALL 0        // development switch: 1 = the TMA-staged increments for the regular layout too (measured 5 % slower at N = 120:
-                            // R is 76 KB there, and the per-lane cp.async stream needs no CTA-wide stage hand-over)
-#endif
-#ifndef TC_NOLOAD
-#define TC_NOLOAD 0        // development switch: 1 = skip the loads of R (isolates the MMA loop in scripts/subprof.py)
-#endif
+//      two groups of 8 k-steps in flight.  (The big layout's TMA-staged version, gen_increments_tma, measured 5 % slower
+//      here at N = 120: R is 76 KB, and the per-lane cp.async stream needs no CTA-wide stage hand-over.)
 __device__ __forceinline__ void warp_sum2(double &p, double &q)
 {
 #pragma unroll
@@ -1140,7 +1112,7 @@ __device__ __noinline__ void generate(const RunArgs &a, const ChainCtx &cx, int 
     // big layout: row sidx of Z is the ring slot of step g0 + sidx itself (the increments overwrite it at the end), which
     // leaves the per-warp areas to the TMA stages of R
     const bool big = a.big != 0;
-#define ZROW(sidx) ((big || TC_TMA_ALL) ? cx.slot_d(g0 + (sidx)) : cx.U + (size_t)(sidx) * zs)
+#define ZROW(sidx) (big ? cx.slot_d(g0 + (sidx)) : cx.U + (size_t)(sidx) * zs)
     SUBP_BEGIN;
 #ifdef TC_SUBPROF
     if (tid == 0 && cx.ch == 0) { tc_subprof[26] += 1; tc_subprof[27] += nnew; }
@@ -1217,7 +1189,7 @@ __device__ __noinline__ void generate(const RunArgs &a, const ChainCtx &cx, int 
     if (r_diag) {
         // big layout: Z lives in the ring slots and is scaled IN PLACE below, while the warps above may still be reading it
         // for the norms (the regular layout keeps Z apart, and gen_increments_tma starts with a barrier of its own)
-        if (big || TC_TMA_ALL) __syncthreads();
+        if (big) __syncthreads();
 #pragma unroll 1
         for (int sidx = 0; sidx < nnew; ++sidx) {
             const double2 *dz = reinterpret_cast<const double2 *>(ZROW(sidx));
@@ -1226,7 +1198,7 @@ __device__ __noinline__ void generate(const RunArgs &a, const ChainCtx &cx, int 
             double2 zz[(7 + 414 + DRAM_THREADS - 1) / DRAM_THREADS];
 #pragma unroll
             for (int m = 0; m < (int)(sizeof(zz) / sizeof(zz[0])); ++m) { const int j = tid + m * DRAM_THREADS; if (j < npar) zz[m] = dz[j]; }
-            if (big || TC_TMA_ALL) __syncthreads();
+            if (big) __syncthreads();
 #pragma unroll
             for (int m = 0; m < (int)(sizeof(zz) / sizeof(zz[0])); ++m) {
                 const int j = tid + m * DRAM_THREADS;
@@ -1236,7 +1208,7 @@ __device__ __noinline__ void generate(const RunArgs &a, const ChainCtx &cx, int 
                 }
             }
         }
-    } else if (big || TC_TMA_ALL) {
+    } else if (big) {
         gen_increments_tma(cx, g0, nnew);
         SUBP(2);
     } else {
@@ -1273,7 +1245,7 @@ __device__ __noinline__ void generate(const RunArgs &a, const ChainCtx &cx, int 
             // (commit / wait_group order the arrivals; a register pipeline would have to share the warp's 6 scoreboards)
 #define GEN_ISSUE(slot, live)                                                                               \
     {                                                                                                       \
-        if ((live) && il <= bj && !TC_NOLOAD) asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(sstg + 256u * (unsigned)(slot)), "l"(pl) : "memory"); \
+        if ((live) && il <= bj) asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(sstg + 256u * (unsigned)(slot)), "l"(pl) : "memory"); \
         else tc_smem[ostg + 32 * (slot)] = 0.0;                                                             \
         pl += dpl; dpl -= 16; il += 1;                                                                      \
     }
@@ -1341,13 +1313,7 @@ __device__ __forceinline__ void cand_bounds_t(const ChainCtx &cx, int k, int C, 
         const int o1 = cx.slot_i(k + c), o2 = o1 + cx.s1;
         double pr1 = 0.0, pr2 = 0.0;
         unsigned oob = 0;
-#if TC_CB_UNR == 4
-#pragma unroll 4
-#elif TC_CB_UNR == 2
-#pragma unroll 2
-#else
-#pragma unroll 1
-#endif
+#pragma unroll 1                                                    // the smallest code: measured +1 % on config 2 against unroll 4
         for (int j = lane; j < npar; j += 32) {
             const double xj = tc_smem[ox + j], a1 = xj + tc_smem[o1 + j], a2 = xj + tc_smem[o2 + j];
             double lo, hi, mu, pinv;
@@ -1373,15 +1339,15 @@ __device__ __noinline__ void cand_bounds(const ChainCtx &cx, int k, int C, Cand 
     else { if (cx.uni) cand_bounds_t<false, true>(cx, k, C, cand); else cand_bounds_t<false, false>(cx, k, C, cand); }
 }
 
-// Round phase D, part 2: the delayed-rejection arithmetic of ONE step (one lane) whose first stage rejected, from state
-// (ss, pri) seeing sigma2 = s2p.  The three exponentials are evaluated in one interleaved body (an unused one may see
-// garbage or Inf: it is never read):
+// The delayed-rejection decision of ONE step (one lane) whose first stage rejected, from state (ss, pri) seeing sigma2 = s2p;
+// q1 = -1/2 (|z1 - z2/drscale|^2 - |z1|^2) and the uniform u2 are the step's (generate()).  Both samplers decide through it:
+// dram_kernel in round phase D, dram_warp_kernel in its step loop.  The three exponentials are evaluated in one interleaved
+// body (an unused one may see garbage or Inf: it is never read):
 //   a12 = exp(-1/2 ((ss1-ss)/s2 + pr1-pri)), a32 = exp(-1/2 ((ss1-ss2)/s2 + pr1-pr2)), exp(l2 + q1)
 //                                                                             mcmcstat DRAM: SURVEY.md 3.2
-__device__ __noinline__ int resolve_dr(const double *sc, bool o1, double x12, double pr1, double pr2, double ss1, double ss2,
+__device__ __noinline__ int resolve_dr(double q1, double u2, bool o1, double x12, double pr1, double pr2, double ss1, double ss2,
                                        double ss, double pri, double is2p)            // is2p = 1 / sigma2 of the step
 {
-    const double q1 = -0.5 * (sc[3] - sc[4]);
     double e12, e32, e13;
     tc_exp3(x12, -0.5 * ((ss1 - ss2) * is2p + pr1 - pr2), -0.5 * ((ss2 - ss) * is2p + pr2 - pri) + q1, e12, e32, e13);
     const double a12 = o1 ? 0.0 : e12;
@@ -1393,7 +1359,7 @@ __device__ __noinline__ int resolve_dr(const double *sc, bool o1, double x12, do
     // denominator that rounds to 0 keeps the quotient's answer: +Inf -> accept when num > 0, 0/0 -> reject.
     const double num = e13 * (1.0 - a32), den = 1.0 - a12;
     if (!(den > 0.0)) return num > 0.0 ? 1 : 0;
-    return (num >= den || num > sc[1] * den) ? 1 : 0;
+    return (num >= den || num > u2 * den) ? 1 : 0;
 }
 
 // dst[e] = src[e] * sc, e < n 16-byte units, src in HBM/L2: 8 independent loads in flight per thread (written as one loop
@@ -1963,7 +1929,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                     if (o2) { so_.fl |= TC_FL_OOB2; ++so_.noob; }
                     else {
                         ++so_.nev;
-                        if (resolve_dr(scp, o1, x12, pr1, pr2, ss1, ss2, ss, pri, is2p)) { so_.acc = 2; so_.fl |= TC_FL_STAGE2; so_.ssn = ss2; so_.prin = pr2; }
+                        if (resolve_dr(-0.5 * (scp[3] - scp[4]), scp[1], o1, x12, pr1, pr2, ss1, ss2, ss, pri, is2p)) { so_.acc = 2; so_.fl |= TC_FL_STAGE2; so_.ssn = ss2; so_.prin = pr2; }
                     }
                 }
             }
@@ -2122,22 +2088,6 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             atomicExch(a.cstate + ch, nseg);                        // finished (also ends a chain whose ss(x0) failed)
         }
     }
-}
-
-// delayed-rejection decision from values (the chain-per-warp kernel keeps the step's scalars in L2)
-__device__ __noinline__ int resolve_dr_v(double q1, double u2, bool o1, double x12, double pr1, double pr2, double ss1, double ss2,
-                                         double ss, double pri, double is2p)            // is2p = 1 / sigma2 of the step
-{
-    // the arithmetic of resolve_dr(), from values
-    double e12, e32, e13;
-    tc_exp3(x12, -0.5 * ((ss1 - ss2) * is2p + pr1 - pr2), -0.5 * ((ss2 - ss) * is2p + pr2 - pri) + q1, e12, e32, e13);
-    const double a12 = o1 ? 0.0 : e12;
-    double a32 = e32;
-    a32 = a32 > 1.0 ? 1.0 : a32;
-    if (!(a32 >= 0.0)) a32 = 0.0;
-    const double num = e13 * (1.0 - a32), den = 1.0 - a12;
-    if (!(den > 0.0)) return num > 0.0 ? 1 : 0;
-    return (num >= den || num > u2 * den) ? 1 : 0;
 }
 
 #include "tc_warp.cuh"

@@ -123,20 +123,6 @@ __device__ __forceinline__ double wk_ld_keep(const double *p, unsigned long long
     return v;
 }
 
-// FP32 -> FP64 (exact).  WK_INTWIDEN: with integer instructions instead of the conversion unit (normal or zero values only:
-// radius * cos/sin of Box-Muller is never denormal) — a development switch
-__device__ __forceinline__ double wk_widen(float f)
-{
-#ifndef WK_INTWIDEN                                                  // measured: no faster than F2F on B200 (generate 28.2 k vs 27.0 k cycles/step)
-    return (double)f;
-#else
-    const unsigned b = __float_as_uint(f);
-    const unsigned hi = (b & 0x7f800000u) ? ((b & 0x80000000u) | (((b >> 3) & 0x0fffffffu) + 0x38000000u)) : (b & 0x80000000u);
-    return __hiloint2double((int)hi, (int)(b << 29));
-#endif
-}
-__device__ __forceinline__ double wk_widen(double f) { return f; }
-
 template <typename ZT>
 __device__ __forceinline__ void wk_increments(const WkCtx &c, int nnew)
 {
@@ -192,7 +178,8 @@ __device__ __forceinline__ void wk_increments(const WkCtx &c, int nnew)
 #pragma unroll
             for (int u = 0; u < 8; ++u) {
                 const int kc = min(4 * (kk + u), ldz - 4);
-                const double a1 = wk_widen(za1p[kc]), a2 = wk_widen(za2p[kc]);
+                // FP32 Z widens exactly through F2F: integer-instruction widening measured no faster (28.2 k vs 27.0 k cycles per step)
+                const double a1 = za1p[kc], a2 = za2p[kc];
                 dmma_m8n8k4(acc[u & 3][0], acc[u & 3][1], a1, bv[u]);
                 dmma_m8n8k4(acc[u & 3][2], acc[u & 3][3], a2, bv[u]);
             }
@@ -868,25 +855,19 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
         int k = seg == 0 ? 1 : seg * a.seglen;
         rden = tc_rcp(n0s20 + ss);                                  // (a function of ss alone: recomputed, not parked)
         int next_adapt = a.adaptint > 0 ? ((k + a.adaptint) / a.adaptint) * a.adaptint : 0x7fffffff;
-#ifdef WK_BAR_EVERY
-        int wk_batch = 0;
-#endif
 #pragma unroll 1
         while (k < k_end) {                                             // the same trip count for every warp of the CTA
             const int g0 = k, gen_upto = min(k + genmax, min(k_end, next_adapt));
-#ifdef WK_BAR_EVERY                                                  // development switch: align the phases only every n-th batch.  Measured
-            if ((wk_batch++ % WK_BAR_EVERY) == 0)                       // (9 568 chains): n = 1 / 2 / 4 -> 55.5 k / 62.9 k / 72.7 k cycles per step
-#endif
-            __syncthreads();                                            // phase alignment: generation
+            // phase alignment: generation.  Every batch: aligning every 2nd / 4th measured 62.9 k / 72.7 k cycles per step
+            // against 55.5 k (9 568 chains)
+            __syncthreads();
             if (active) {
                 WK_PHASE(3);
                 wk_generate(a, c, g0, gen_upto - g0, r_diag != 0);
                 wk_stage_cell(a.cells, cid, cv);
                 WK_PHASE(0);
             }
-#if !defined(WK_NOBAR2) && !defined(WK_BAR_EVERY)
             __syncthreads();                                            // phase alignment: the step loop
-#endif
             if (active) WK_PHASE(3);
 #pragma unroll 1
             for (; k < gen_upto && active; ++k) {
@@ -920,7 +901,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                         const double ss2 = ss_eval(a.cons, cv, SmemVecA{ob}, w, a.algo, false, nullptr, nullptr);
                         WK_T1(7);
                         ++nev;
-                        if (resolve_dr_v(-0.5 * (s_n1 - s_n0), s_u2, o1, x12, pr1, pr2, ss1, ss2, ss, pri, is2)) { acc = 2; fl |= TC_FL_STAGE2; ssn = ss2; prin = pr2; }
+                        if (resolve_dr(-0.5 * (s_n1 - s_n0), s_u2, o1, x12, pr1, pr2, ss1, ss2, ss, pri, is2)) { acc = 2; fl |= TC_FL_STAGE2; ssn = ss2; prin = pr2; }
                     }
                 }
                 // ---- commit
@@ -1024,8 +1005,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 cn[TC_CNT_CYCLES0 + 4] = st.pc[5]; cn[TC_CNT_CYCLES0 + 5] = st.pc[2]; cn[TC_CNT_CYCLES0 + 6] = st.pc[6];
 #ifdef WK_SUBPROF
                 cn[TC_CNT_CYCLES0 + 7] = st.pc[7];
-#endif
-#ifndef WK_SUBPROF
+#else
                 cn[TC_CNT_CYCLES0 + 7] = st.n_ss;                       // no speculation: every evaluation is committed
 #endif
             }
