@@ -110,11 +110,17 @@ enum { TC_LAYOUT_AUTO = 0, TC_LAYOUT_BIG = 1, TC_LAYOUT_WARP = 2, TC_LAYOUT_CTA 
 enum {
     TC_CNT_SS_EVALS = 0, TC_CNT_ACC_STAGE1 = 1, TC_CNT_ACC_STAGE2 = 2, TC_CNT_OUT_OF_BOUNDS = 3,
     TC_CNT_ADAPTATIONS = 4, TC_CNT_CHOL_FAIL = 5, TC_CNT_DR_TRIES = 6, TC_CNT_STATUS = 7,
-    /* SM cycles thread 0 of the chain's CTA spent per phase of the speculative batch loop:
-       +0 generation (randomness + tensor-core increments), +1 speculation (SPEC steps in parallel),
-       +2 rows of rejected steps, +3 accept/copy, +4 per-row scalars + state update, +5 adaptation
-       (covariance block update + Cholesky), +6 spare; +7 = forward-model evaluations executed
-       including the speculative ones that were discarded (TC_CNT_SS_EVALS counts only the committed) */
+    /* TC_CNT_CYCLES0 + i: SM cycles the chain spent per phase (clock readings, not results), by sampler.
+       One CTA per chain (TC_LAYOUT_CTA / _BIG), cycles of thread 0:
+         +0 generation (randomness + proposal increments), +1 bounds checks + the speculative evaluations of a
+         round, +2 decisions + commit of a round, +3 +4 +6 always 0, +5 adaptation (covariance update + Cholesky);
+         +7 is a count: forward-model evaluations executed, including the discarded speculative ones
+         (TC_CNT_SS_EVALS counts only the committed).
+       One warp per chain (TC_LAYOUT_WARP), cycles of lane 0:
+         +0 generation, +1 the step loop, +2 waits at the barriers that keep the CTA's warps in one phase,
+         +3 the randomness part of +0, +4 the scatter-update part of +5, +5 adaptation, +6 the scatter-update +
+         factorisation part of +5; +7 = TC_CNT_SS_EVALS (no speculation: every evaluation is committed; a
+         -DWK_SUBPROF development build puts the cycles of the forward-model evaluations there instead). */
     TC_CNT_CYCLES0 = 8,
     TC_NCOUNTERS = 16
 };

@@ -179,6 +179,7 @@ def test_time_slices_are_transparent(gpu_cells, cells_npz, orc):
     inputs = _setup(gpu_cells, chain_cell, 51)
     opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, seed=seed, **SHORT)
     out = gpu_cells.mcmc_run(opts, chain_cell, *inputs, chain_uid=uid, want_flags=True)
+    assert np.all(out["counters"][:, [_lib.CNT_CYCLES0 + 3, _lib.CNT_CYCLES0 + 4, _lib.CNT_CYCLES0 + 6]] == 0)   # phases dram_kernel does not time
     for i, c in enumerate(chain_cell):
         N = int(cells_npz["N"][c]); npar = 7 + N
         d = _lib.rng_dump(seed, int(uid[i]), npar, 1 + 2 * N, nsimu)
@@ -385,6 +386,7 @@ def test_warp_kernel_production_path(gpu_cells, cells_npz, orc):
         res[layout] = gpu_cells.mcmc_run(opts, cc, *inputs, chain_uid=uid, want_flags=True)
     assert np.array_equal(res[2]["flags"], res[0]["flags"])
     assert np.array_equal(res[2]["counters"][:, :8], res[0]["counters"][:, :8])
+    assert np.array_equal(res[2]["counters"][:, _lib.CNT_CYCLES0 + 7], res[2]["counters"][:, _lib.CNT_SS_EVALS])
     np.testing.assert_allclose(res[2]["mean"], res[0]["mean"], rtol=0, atol=1e-6)
     np.testing.assert_allclose(res[2]["sig"], res[0]["sig"], rtol=1e-9)
     for i in (0, 17, 36):

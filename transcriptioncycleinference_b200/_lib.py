@@ -17,6 +17,7 @@ NCOUNTERS = 16
 ALGO_PAIRS, ALGO_TOEPLITZ = 0, 1
 CNT_SS_EVALS, CNT_ACC_STAGE1, CNT_ACC_STAGE2, CNT_OUT_OF_BOUNDS = 0, 1, 2, 3
 CNT_ADAPTATIONS, CNT_CHOL_FAIL, CNT_DR_TRIES, CNT_STATUS = 4, 5, 6, 7
+CNT_CYCLES0 = 8       # + 0..7: per-phase clock readings (include/tcmcmc.h)
 FL_ACCEPT, FL_STAGE2, FL_OOB1, FL_DR, FL_OOB2 = 1, 2, 4, 8, 16
 
 EXPORTS = [

@@ -858,26 +858,133 @@ __device__ __noinline__ bool chol_global(int nt4, int npar, const double *gA, do
 struct Cand { double pr1, pr2; int oob, pad; };
 // outcome of one step under the hypothesis "every earlier step of the round rejected" (registers of lane = step)
 struct StepOut { double ssn, prin; int acc, fl, nev, noob; };
-// s2chain statistics over ALL rows (TranscriptionCycleMCMC.m:302-303), thread 0, shared memory
-struct S2Stats { double sum, sq_sum, cnt, pad; };      // sum s2, sum sqrt(s2), rows
+
+// ---- chain book-keeping shared by dram_kernel and dram_warp_kernel (tc_warp.cuh)
+
+// Constants of a chain that both samplers derive their per-step arithmetic from
+struct ChainConsts {
+    unsigned long long uid;                             // Philox identity
+    int first_row, nstore;                              // first row of the summaries and of the stored chain (n_burn - 1), rows stored
+    double inv_dr, adascale, chi_d, chi_c;              // chi_d, chi_c: Marsaglia-Tsang constants of chi2(N0 + 2 N)
+};
+__device__ __forceinline__ ChainConsts chain_consts(const RunArgs &a, int ch, int N)
+{
+    ChainConsts k;
+    k.uid = a.chain_uid ? a.chain_uid[ch] : (unsigned long long)ch;
+    k.first_row = a.n_burn - 1;
+    k.nstore = a.nsimu - (a.n_burn - 1);
+    k.inv_dr = 1.0 / a.drscale;
+    k.adascale = a.adascale > 0.0 ? a.adascale : 2.4 / sqrt((double)(7 + N));
+    chi2_consts(a.N0 + 2.0 * N, k.chi_d, k.chi_c);
+    return k;
+}
+
+// Phase clocks: pc[i] of the tally is returned as counter TC_CNT_CYCLES0 + i; include/tcmcmc.h says what each sampler times in
+// each slot (PH_COMMIT: dram_kernel, PH_WAIT, PH_RAND, PH_SCATTER, PH_FACTOR: dram_warp_kernel, PH_EVAL: its WK_SUBPROF build)
+enum { PH_GEN = 0, PH_STEPS = 1, PH_COMMIT = 2, PH_WAIT = 2, PH_RAND = 3, PH_SCATTER = 4, PH_ADAPT = 5, PH_FACTOR = 6, PH_EVAL = 7 };
+
+// What a chain counts and sums, in shared memory (one thread writes each field); parked with the chain between slices
+struct Tally {
+    long long n_ss, n_acc1, n_acc2, n_oob, n_adapt, n_cholfail, n_dr;   // counters TC_CNT_SS_EVALS .. TC_CNT_DR_TRIES
+    long long n_spec;                                   // dram_kernel: evaluations including the discarded speculative ones
+    long long rej, reju;                                // rejected steps: in all, since the last adaptation
+    double s2sum, s2sq, s2cnt;                          // s2chain over ALL rows (TranscriptionCycleMCMC.m:302-303): sum s2, sum sqrt(s2), rows
+    double wcnt, cov_n;                                 // rows in the Welford summaries, rows in the covariance
+    long long pc[8];                                    // phase clocks (PH_*)
+};
+
+// A chain between two time slices: its slot of gState (state_doubles(ld) doubles) holds this record, then the vectors
+// x | wmean | wM2 | rdiag, ld doubles each (dram_warp_kernel keeps the last three there all along).  16-byte aligned: the vectors
+// after it stay aligned, and it moves through L2 as 16-byte words.
+struct __align__(16) ParkedChain {
+    double ss, pri, sigma2;
+    double rsig;                                        // 1 / sigma2 as the next step sees it (chi2 of the last row * rden)
+    int r_diag;
+    int bad0;                                           // ss(x0) was not finite (dram_warp_kernel: the later slices skip the chain)
+    Tally t;
+};
+constexpr int ST_VEC0 = sizeof(ParkedChain) / sizeof(double);
+__host__ __device__ inline int state_doubles(int ld) { return ST_VEC0 + 4 * ld; }
+
+// the next slice may run on another SM: past L1 both ways
+__device__ __forceinline__ void park_chain(double *gst, const ParkedChain &p)
+{
+    const double2 *src = reinterpret_cast<const double2 *>(&p);
+#pragma unroll
+    for (int i = 0; i < (int)(sizeof(ParkedChain) / 16); ++i) __stcg(reinterpret_cast<double2 *>(gst) + i, src[i]);
+}
+__device__ __forceinline__ ParkedChain resume_chain(const double *gst)
+{
+    ParkedChain p;
+    double2 *dst = reinterpret_cast<double2 *>(&p);
+#pragma unroll
+    for (int i = 0; i < (int)(sizeof(ParkedChain) / 16); ++i) dst[i] = __ldcg(reinterpret_cast<const double2 *>(gst) + i);
+    return p;
+}
+
+// The optional per-row outputs of row r: s2chain (store_chain), flags and sschain (replay / parity harness)
+__device__ __forceinline__ void store_row(const RunArgs &a, int ch, int r, double s2, int fl, double ss)
+{
+    const size_t g = (size_t)ch * a.nsimu + r;
+    if (a.store_chain && a.s2chain) a.s2chain[g] = s2;
+    if (a.flags) a.flags[g] = fl;
+    if (a.sschain) a.sschain[g] = ss;
+}
+// Row 0 = x0 with a finite ss0: s2 = sigma2_0 (TranscriptionCycleMCMC.m:259), no flags.  One thread.
+__device__ __forceinline__ void record_row0(const RunArgs &a, int ch, double ss0, Tally &t)
+{
+    t.s2sum += a.sigma2_0; t.s2sq += sqrt(a.sigma2_0); t.s2cnt += 1.0;
+    store_row(a, ch, 0, a.sigma2_0, 0, ss0);
+}
+
+// a Welford vector: shared memory (dram_kernel) or L2 (dram_warp_kernel: written by other SMs, so past L1)
+__device__ __forceinline__ double ld_welford(const double *p) { return __isGlobal(p) ? __ldcg(p) : *p; }
+// Outputs of a finished chain (TranscriptionCycleMCMC.m:286-303): mean / std of the stored rows by the threads i0 = 0 .. nthr-1,
+// sig and the counters by thread i0 = 0.  slot7 = counter TC_CNT_CYCLES0 + 7, the one slot whose meaning the caller decides.
+// A chain whose ss(x0) is not finite (bad0) reports zeros and status 1.
+__device__ void write_outputs(const RunArgs &a, int ch, int npar, const double *wmean, const double *wM2, const Tally &t,
+                              long long slot7, bool bad0, int i0, int nthr)
+{
+    const double wcnt = t.wcnt;
+#pragma unroll 1
+    for (int i = i0; i < npar; i += nthr) {
+        if (a.mean) a.mean[(size_t)ch * a.ld + i] = bad0 ? 0.0 : ld_welford(wmean + i);
+        if (a.std) a.std[(size_t)ch * a.ld + i] = (!bad0 && wcnt > 0) ? sqrt(ld_welford(wM2 + i) / wcnt) : 0.0;
+    }
+    if (i0 != 0) return;
+    if (a.sig) {
+        // sqrt(mean(s2chain)); std(sqrt(s2chain),1) = sqrt(E[s2] - E[sqrt(s2)]^2)   (:302-303)
+        const double m2 = t.s2sum / t.s2cnt, m1 = t.s2sq / t.s2cnt;
+        a.sig[2 * (size_t)ch] = bad0 ? 0.0 : sqrt(m2);
+        a.sig[2 * (size_t)ch + 1] = bad0 ? 0.0 : sqrt(fmax(m2 - m1 * m1, 0.0));
+    }
+    if (a.counters) {
+        long long *c = a.counters + (size_t)ch * TC_NCOUNTERS;
+        c[TC_CNT_SS_EVALS] = t.n_ss; c[TC_CNT_ACC_STAGE1] = t.n_acc1; c[TC_CNT_ACC_STAGE2] = t.n_acc2;
+        c[TC_CNT_OUT_OF_BOUNDS] = t.n_oob; c[TC_CNT_ADAPTATIONS] = t.n_adapt;
+        c[TC_CNT_CHOL_FAIL] = t.n_cholfail; c[TC_CNT_DR_TRIES] = t.n_dr; c[TC_CNT_STATUS] = bad0 ? 1 : 0;
+        for (int i = 0; i < 7; ++i) c[TC_CNT_CYCLES0 + i] = t.pc[i];
+        c[TC_CNT_CYCLES0 + 7] = slot7;
+    }
+}
 
 // Mutable chain state (uniform across the CTA) in shared memory.  Written by thread 0 in the commit phase
 // (between the post-speculation barrier and the end-of-round barrier), read by everyone at the top of a round.
+// In the commit phase thread 0 and lane 0 of warp SPEC-1 write disjoint fields.
 struct ChainState {
-    double ss, pri, sigma2, cov_n, wcnt;
+    double ss, pri, sigma2;
     double rden, rsig;                                  // 1 / (N0 S20 + ss) and 1 / sigma2 as the next step sees it (= chi2 of the last row * rden)
     int r_diag, bad0, run_r0, ndist;
-    long long n_ss, n_acc1, n_acc2, n_oob, n_adapt, n_cholfail, n_dr, n_spec, rej, reju;
-    long long pc[8], tprev;
+    Tally t;
+    long long tprev;
 };
 
 // Immutable per-chain context, built once in shared memory so that the out-of-line phases below
 // (kept out of line to keep the hot loop inside the instruction cache) can share it.
 struct ChainCtx {
-    int N, npar, npad, ld, slot_sz, s1, wsz, ch, first_row, nstore, ring_mask, uni;
+    int N, npar, npad, ld, slot_sz, s1, wsz, ch, ring_mask, uni;
     double blk[4];                                      // uni: common lo, hi, mu, 1/sig of the parameters >= 7 (the dR block)
-    unsigned long long uid;
-    double adascale, inv_dr, chi_d, chi_c;              // chi_d, chi_c: Marsaglia-Tsang constants of chi2(N0 + 2 N)
+    ChainConsts cc;
     SmemCell cv;
     int o_x, o_ring, o_U;                               // offsets (doubles) into tc_smem
     int o_lo, o_pinv, o_wmean, o_wM2, o_mb;             // hot per-parameter vectors by offset (tc_smem + offset compiles to LDS/STS, the
@@ -900,7 +1007,7 @@ __device__ __noinline__ void flush_run(const RunArgs &a, const ChainCtx &cx, int
     // threads t0 .. DRAM_THREADS-1 take part (t0 = 32 at an accept: warp 0 writes the per-row scalars meanwhile)
     const int tid = (int)threadIdx.x - t0, nthr = DRAM_THREADS - t0, npar = cx.npar;
     if (tid < 0) return;
-    const int m_c = r1 - r0, rs = max(r0, cx.first_row), m_w = r1 - rs;
+    const int m_c = r1 - r0, rs = max(r0, cx.cc.first_row), m_w = r1 - rs;
     const bool cov = a.do_cov && m_c > 0;
     // Welford weights m_w / nn and wcnt m_w / nn through ONE reciprocal (every thread computes them: two quotients were ~300
     // cycles at the head of every accept)
@@ -915,7 +1022,7 @@ __device__ __noinline__ void flush_run(const RunArgs &a, const ChainCtx &cx, int
             tc_smem[owm + i] = fma(d1, f1, wm);
             tc_smem[ow2 + i] = fma(d1 * d1, f2, tc_smem[ow2 + i]);
             if (a.store_chain && a.chain) {
-                double *dst = a.chain + ((size_t)cx.ch * cx.nstore + (rs - cx.first_row)) * cx.ld + i;
+                double *dst = a.chain + ((size_t)cx.ch * cx.cc.nstore + (rs - cx.cc.first_row)) * cx.ld + i;
 #pragma unroll 1
                 for (int r = 0; r < m_w; ++r) dst[(size_t)r * cx.ld] = xo;
             }
@@ -927,27 +1034,6 @@ __device__ __noinline__ void flush_run(const RunArgs &a, const ChainCtx &cx, int
         if (so >= 0) tc_smem[ox + i] = xo + tc_smem[so + i];
     }
     if (cov && tid == 0) cx.gWts[ndist] = (double)m_c;
-}
-
-// Per-row scalars of `cnt` committed rows r0.. by the lanes of warp 0 (one row per lane, cnt <= SPEC):
-// sigma2 of the row, s2chain statistics (sum s2, sum sqrt(s2)) and the optional per-step outputs.
-// Rows before `first` keep (ss_old); row `first` (if < cnt) carries the accepted (ss_new).
-__device__ __noinline__ void emit_s2(const RunArgs &a, const ChainCtx &cx, S2Stats *st, int fl, int r0, int cnt,
-                                     int first, double ss_old, double ss_new, double sigma2_fixed)
-{
-    const int lane = threadIdx.x & 31;
-    double s2 = 0.0, sq = 0.0;
-    if (lane < cnt) {
-        const int r = r0 + lane;
-        const double ssr = lane < first ? ss_old : ss_new;
-        s2 = (a.updatesigma && r > 0) ? (a.N0 * a.S20 + ssr) / cx.slot_sc(r)[2] : sigma2_fixed;
-        sq = sqrt(s2);
-        if (a.store_chain && a.s2chain) a.s2chain[(size_t)cx.ch * a.nsimu + r] = s2;
-        if (a.flags) a.flags[(size_t)cx.ch * a.nsimu + r] = fl;
-        if (a.sschain) a.sschain[(size_t)cx.ch * a.nsimu + r] = ssr;
-    }
-    s2 = warp_sum(s2); sq = warp_sum(sq);
-    if (lane == 0) { st->sum += s2; st->sq_sum += sq; st->cnt += cnt; }
 }
 
 #define GEN_M 8
@@ -1078,7 +1164,7 @@ __device__ __noinline__ void gen_increments_tma(const ChainCtx &cx, int g0, int 
     __syncthreads();                                                // every warp is done reading Z: the increments overwrite it
     if (ar < nnew) {
         const int oo = cx.slot_i(g0 + ar), o2 = oo + cx.s1;
-        const double inv_dr = cx.inv_dr;
+        const double inv_dr = cx.cc.inv_dr;
 #pragma unroll
         for (int j = 0; j < GENB_MAXT; ++j) {
             const int jc = 8 * (warp + SPEC * (mcnt - 1 - j)) + 2 * ak;     // accumulator j = the j-th tile from the top
@@ -1141,10 +1227,10 @@ __device__ __noinline__ void generate(const RunArgs &a, const ChainCtx &cx, int 
         if (warp == 0 && lane < nnew) {
             const int st = g0 + lane;
             double *sc = cx.slot_sc(st);
-            const u32x4 ru = draw(a.seed, cx.uid, st, RK_U, 0);
+            const u32x4 ru = draw(a.seed, cx.cc.uid, st, RK_U, 0);
             sc[0] = u01(ru.x, ru.y);
             sc[1] = u01(ru.z, ru.w);
-            sc[2] = a.updatesigma ? chi2_draw_dc(a.seed, cx.uid, st, cx.chi_d, cx.chi_c) : 1.0;
+            sc[2] = a.updatesigma ? chi2_draw_dc(a.seed, cx.cc.uid, st, cx.cc.chi_d, cx.cc.chi_c) : 1.0;
             sc[5] = tc_log(sc[0]);                                  // stage 1 is decided in the log domain
         }
         __syncwarp();
@@ -1162,7 +1248,7 @@ __device__ __noinline__ void generate(const RunArgs &a, const ChainCtx &cx, int 
             if (it < nitems) {
                 const int sidx = (int)(((float)it + 0.5f) * inv_np), q2 = it - sidx * npairs;
                 double *dz = ZROW(sidx);
-                const double4 z = normal_quad(a.seed, cx.uid, g0 + sidx, q2);
+                const double4 z = normal_quad(a.seed, cx.cc.uid, g0 + sidx, q2);
                 *reinterpret_cast<double2 *>(dz + 4 * q2) = make_double2(z.x, z.z);          // (z1, z2) of parameter 2q
                 if (2 * q2 + 1 < npar) *reinterpret_cast<double2 *>(dz + 4 * q2 + 2) = make_double2(z.y, z.w);
             }
@@ -1178,7 +1264,7 @@ __device__ __noinline__ void generate(const RunArgs &a, const ChainCtx &cx, int 
 #pragma unroll 1
         for (int i = lane; i < npar; i += 32) {
             const double2 zz = dz[i];
-            const double d = zz.x - zz.y * cx.inv_dr;
+            const double d = zz.x - zz.y * cx.cc.inv_dr;
             n1 = fma(d, d, n1);
             n0 = fma(zz.x, zz.x, n0);
         }
@@ -1204,7 +1290,7 @@ __device__ __noinline__ void generate(const RunArgs &a, const ChainCtx &cx, int 
                 const int j = tid + m * DRAM_THREADS;
                 if (j < npar) {
                     const double r = cx.rdiag[j];
-                    tc_smem[o1 + j] = zz[m].x * r; tc_smem[o2 + j] = zz[m].y * (r * cx.inv_dr);
+                    tc_smem[o1 + j] = zz[m].x * r; tc_smem[o2 + j] = zz[m].y * (r * cx.cc.inv_dr);
                 }
             }
         }
@@ -1215,7 +1301,7 @@ __device__ __noinline__ void generate(const RunArgs &a, const ChainCtx &cx, int 
         const int NT = (npar + 7) >> 3;                              // column tiles of 8
         const int ar = lane >> 2, ak = lane & 3;                     // A[row = step][k], B[k][col]
         const double *gR = cx.gRb;
-        const double inv_dr = cx.inv_dr;
+        const double inv_dr = cx.cc.inv_dr;
         // Column tiles are dealt to the warps in serpentine order (longest k-range first: balances the triangle):
         // tile of round r = NT-1 - (8 r + (r odd ? 7-w : w)).
         const int oa = cx.o_U + ar * zs;                              // A row of this lane (offset into tc_smem); rows >= nnew hold
@@ -1509,7 +1595,7 @@ __device__ __noinline__ int adapt(const RunArgs &a, const ChainCtx &cx, int isim
             if (!ok && !a.qcovadj_always) ok = chol_global(nt4, npar, cx.gM2, invn, a.qcovadj, gW, o_ws, ws_d);
             SUBP(11);
             if (ok) {
-                scaled_copy_cg(reinterpret_cast<double2 *>(cx.gRb), reinterpret_cast<const double2 *>(gW), 8 * T4, cx.adascale);
+                scaled_copy_cg(reinterpret_cast<double2 *>(cx.gRb), reinterpret_cast<const double2 *>(gW), 8 * T4, cx.cc.adascale);
                 fence_async_proxy();                                // generate() reads R back with bulk copies
             }
             __syncthreads();
@@ -1547,7 +1633,7 @@ __device__ __noinline__ int adapt(const RunArgs &a, const ChainCtx &cx, int isim
             {
                 const double2 *src = reinterpret_cast<const double2 *>(W);
                 double2 *dst = reinterpret_cast<double2 *>(cx.gRb);
-                const double sc = cx.adascale;
+                const double sc = cx.cc.adascale;
 #pragma unroll 8
                 for (int e = tid; e < 8 * T4; e += DRAM_THREADS) { const double2 v = src[e]; dst[e] = make_double2(v.x * sc, v.y * sc); }
             }
@@ -1574,12 +1660,6 @@ __device__ __noinline__ int adapt(const RunArgs &a, const ChainCtx &cx, int isim
 // Book-keeping works on RUNS (an accepted state and the rejections that follow it): a rejected step
 // only lengthens the current run; summaries, chain storage and the covariance block see a run once,
 // with its length as weight.
-//
-// Saved state of a chain between two time slices (doubles):
-//   [0..15] scalars | [16..47] counters (long long) | x | wmean | wM2 | rdiag
-#define ST_VEC0 48         // first vector: 16 scalars + up to 32 counters (17 used: 9 counts + 8 phase clocks)
-__host__ __device__ inline int state_doubles(int ld) { return ST_VEC0 + 4 * ld; }
-
 __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_constant__ RunArgs ga)
 {
     // The out-of-line phases take the launch arguments by reference: a reference to the kernel parameter
@@ -1596,7 +1676,6 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
     __shared__ Cand s_cand[RING];
     __shared__ double s_ssv[2 * RING];
     __shared__ ChainCtx cx;
-    __shared__ S2Stats s_s2;
     __shared__ int s_item, s_done, s_sum, s_own;
     __shared__ unsigned s_min;
     __shared__ ChainState st;
@@ -1699,12 +1778,8 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             o += o & 1;
             if (tid == 0) {
                 cx.N = N; cx.npar = npar; cx.npad = (npar + 3) & ~3; cx.ld = a.ld;
-                cx.slot_sz = dram_slot(N); cx.s1 = dram_s1(N); cx.wsz = a.wsz; cx.ch = ch; cx.first_row = a.n_burn - 1;
-                cx.nstore = a.nsimu - (a.n_burn - 1);
-                cx.uid = a.chain_uid ? a.chain_uid[ch] : (unsigned long long)ch;
-                cx.adascale = a.adascale > 0.0 ? a.adascale : 2.4 / sqrt((double)npar);
-                cx.inv_dr = 1.0 / a.drscale;
-                chi2_consts(a.N0 + 2.0 * N, cx.chi_d, cx.chi_c);
+                cx.slot_sz = dram_slot(N); cx.s1 = dram_s1(N); cx.wsz = a.wsz; cx.ch = ch;
+                cx.cc = chain_consts(a, ch, N);
                 cx.cv = cv; cx.cv.d = a.cells.dmean[cid];
                 o |= 1;                                             // x at an ODD offset: x[7] is 16-byte aligned (SumVec::get4)
                 cx.o_x = o;
@@ -1791,30 +1866,26 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
         }
         if (tid == 0) {
             if (seg == 0) {
-                st.ss = 0.0; st.pri = 0.0; st.sigma2 = a.sigma2_0; st.cov_n = 0.0; st.wcnt = 0.0; st.r_diag = 1; st.bad0 = 0;
-                st.n_ss = 1; st.n_acc1 = 0; st.n_acc2 = 0; st.n_oob = 0; st.n_adapt = 0; st.n_cholfail = 0; st.n_dr = 0; st.n_spec = 0;
-                st.rej = 0; st.reju = 0;
-                for (int i = 0; i < 8; ++i) st.pc[i] = 0;
-                s_s2.sum = 0.0; s_s2.sq_sum = 0.0; s_s2.cnt = 0.0;
+                st.sigma2 = a.sigma2_0; st.r_diag = 1;              // (ss, pri, rden, rsig: row 0 below)
+                st.t = Tally{};
+                st.t.n_ss = 1;                                      // ss(x0)
                 st.run_r0 = 0;
             } else {
-                st.ss = __ldcg(gst + 0); st.pri = __ldcg(gst + 1); st.sigma2 = __ldcg(gst + 2); st.cov_n = __ldcg(gst + 3);
-                st.wcnt = __ldcg(gst + 4); st.r_diag = __ldcg(gst + 5) != 0.0; st.bad0 = 0;
-                st.rden = __ldcg(gst + 10); st.rsig = __ldcg(gst + 11);
-                s_s2.sum = __ldcg(gst + 6); s_s2.sq_sum = __ldcg(gst + 7); s_s2.cnt = __ldcg(gst + 9);
-                const long long *gc = reinterpret_cast<const long long *>(gst + 16);
-                st.n_ss = __ldcg(gc + 0); st.n_acc1 = __ldcg(gc + 1); st.n_acc2 = __ldcg(gc + 2); st.n_oob = __ldcg(gc + 3);
-                st.n_adapt = __ldcg(gc + 4); st.n_cholfail = __ldcg(gc + 5); st.n_dr = __ldcg(gc + 6); st.n_spec = __ldcg(gc + 7);
-                st.rej = __ldcg(gc + 8); st.reju = 0;
-                for (int i = 0; i < 8; ++i) st.pc[i] = __ldcg(gc + 9 + i);
+                // (the tally's reju comes back as parked, which is 0: a slice ends on an adaptation boundary, or adaptation
+                // is off and nothing reads it)
+                const ParkedChain p = resume_chain(gst);
+                st.ss = p.ss; st.pri = p.pri; st.sigma2 = p.sigma2; st.rsig = p.rsig; st.r_diag = p.r_diag;
+                st.rden = tc_rcp(a.N0 * a.S20 + p.ss);
+                st.t = p.t;
                 st.run_r0 = seg * a.seglen;
             }
+            st.bad0 = 0;
             st.ndist = 0;
             st.tprev = clock64();
         }
         __syncthreads();
         // phase clocks (TC_CNT_CYCLES0..).  (Sampling them every 8th round was measured: no gain — 66.7 M against 67.5 M.)
-#define TC_PHASE(i) do { if (tid == 0) { const long long tn__ = clock64(); st.pc[i] += tn__ - st.tprev; st.tprev = tn__; } } while (0)
+#define TC_PHASE(i) do { if (tid == 0) { const long long tn__ = clock64(); st.t.pc[i] += tn__ - st.tprev; st.tprev = tn__; } } while (0)
 
         if (seg == 0) {
             // ---- row 0: x0 (opens the first run)
@@ -1824,8 +1895,10 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             for (int i = lane; i < npar; i += 32) { const double e = (cx.x[i] - cx.mu[i]) * cx.pinv[i]; sp += e * e; }
             sp = warp_sum(sp);
             const bool bad = !isfinite(ss0);
-            if (tid == 0) { st.ss = ss0; st.pri = sp; st.bad0 = bad ? 1 : 0; st.rden = tc_rcp(a.N0 * a.S20 + ss0); st.rsig = 1.0 / a.sigma2_0; }
-            if (!bad && warp == 0) emit_s2(a, cx, &s_s2, 0, 0, 1, 1, ss0, ss0, a.sigma2_0);
+            if (tid == 0) {
+                st.ss = ss0; st.pri = sp; st.bad0 = bad ? 1 : 0; st.rden = tc_rcp(a.N0 * a.S20 + ss0); st.rsig = 1.0 / a.sigma2_0;
+                if (!bad) record_row0(a, ch, ss0, st.t);
+            }
             __syncthreads();
         }
 
@@ -1841,7 +1914,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             // is the last one that may use the current R
             const int bound = min(k_end, next_adapt);                       // exclusive step bound
             // chain state of this round (thread 0 rewrites st only in the commit phase, after two barriers)
-            const double ss = st.ss, pri = st.pri, sig2 = st.sigma2, wcnt = st.wcnt;
+            const double ss = st.ss, pri = st.pri, sig2 = st.sigma2, wcnt = st.t.wcnt;
             const int run_r0 = st.run_r0, ndist = st.ndist;
             // 1 / sigma2 of the candidate steps, started here so that the divisions are off the critical path of phase D:
             // step k sees sig2, step k + w sees (N0 S20 + ss) / chi2_{k+w-1}, i.e. 1/sigma2 = chi2_{k+w-1} * rden.  (A product
@@ -1856,7 +1929,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                 generate(a, cx, gen_upto, glim - gen_upto, st.r_diag != 0);
                 gen_upto = glim;
             }
-            TC_PHASE(0);
+            TC_PHASE(PH_GEN);
 
             // ---- one round = SPEC forward-model evaluations, one per warp, over as many future steps as they cover.
             // A. bounds + prior of both proposals of every ready step (an out-of-bounds proposal needs no evaluation)
@@ -1892,7 +1965,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             SUBP(18);
             __syncthreads();
             SUBP(19);
-            TC_PHASE(1);
+            TC_PHASE(PH_STEPS);
             // D. accept/reject of every covered step under the hypothesis "the steps before it rejected" (lane = step; the
             //    sigma2 a step sees is the draw made at the end of the previous step from the unchanged ss).  Every warp
             //    computes the same outcomes, so no barrier is needed before the commit (and a warp running this alone is
@@ -1955,7 +2028,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                     const double ss_new = accd ? ssn_a : ss;
                     if (accd) {
                         st.ss = ss_new; st.pri = prin_a;
-                        st.wcnt = wcnt + max(0, r_acc - max(run_r0, cx.first_row));
+                        st.t.wcnt = wcnt + max(0, r_acc - max(run_r0, cx.cc.first_row));
                         if (a.do_cov && r_acc > run_r0) st.ndist = ndist + 1;
                         st.run_r0 = r_acc;
                     }
@@ -1975,9 +2048,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                     const double ssr = lane < first ? ss : ss_new;
                     s2 = a.updatesigma ? (a.N0 * a.S20 + ssr) * tc_rcp(cx.slot_sc(r)[2]) : sig2;
                     sq = sqrt(s2);
-                    if (a.store_chain && a.s2chain) a.s2chain[(size_t)cx.ch * a.nsimu + r] = s2;
-                    if (a.flags) a.flags[(size_t)cx.ch * a.nsimu + r] = so_.fl;
-                    if (a.sschain) a.sschain[(size_t)cx.ch * a.nsimu + r] = ssr;
+                    store_row(a, cx.ch, r, s2, so_.fl, ssr);
                 }
 #pragma unroll
                 for (int o = RING / 2; o > 0; o >>= 1) { s2 += __shfl_xor_sync(0xffffffffu, s2, o); sq += __shfl_xor_sync(0xffffffffu, sq, o); }
@@ -1986,11 +2057,11 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                 const int d_dr = __reduce_add_sync(0xffffffffu, (lane < ncommit && (so_.fl & TC_FL_DR)) ? 1 : 0);
                 const int d_spec = __shfl_sync(0xffffffffu, inc, nsteps - 1);       // evaluations of this round
                 if (lane == 0) {
-                    s_s2.sum += s2; s_s2.sq_sum += sq; s_s2.cnt += ncommit;
+                    st.t.s2sum += s2; st.t.s2sq += sq; st.t.s2cnt += ncommit;
                     const int nrej = accd ? first : nsteps;
-                    st.n_ss += d_ss; st.n_oob += d_oob; st.n_dr += d_dr; st.n_spec += d_spec;
-                    st.rej += nrej; st.reju += nrej;
-                    if (accd) { if (acc_t == 1) ++st.n_acc1; else ++st.n_acc2; }
+                    st.t.n_ss += d_ss; st.t.n_oob += d_oob; st.t.n_dr += d_dr; st.t.n_spec += d_spec;
+                    st.t.rej += nrej; st.t.reju += nrej;
+                    if (accd) { if (acc_t == 1) ++st.t.n_acc1; else ++st.t.n_acc2; }
                 }
             }
             SUBP(22);
@@ -2000,30 +2071,30 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
 #ifdef TC_SUBPROF
             if (tid == 0 && cx.ch == 0) { tc_subprof[24] += 1; tc_subprof[25] += ncommit; }
 #endif
-            TC_PHASE(2);
+            TC_PHASE(PH_COMMIT);
 
             // adaptation after the step with isimu = k, a multiple of adaptint
             if (k == next_adapt) {
                 const int rr0 = st.run_r0, nd0 = st.ndist;
-                const double wc0 = st.wcnt;
+                const double wc0 = st.t.wcnt;
                 flush_run(a, cx, rr0, k, wc0, nd0, -1, 0);                     // close the run at the block boundary
                 const int nd = nd0 + ((a.do_cov && k > rr0) ? 1 : 0);
-                const double rate = a.burnin_cumulative ? (double)st.rej / k : (double)st.reju / a.adaptint;
-                const double cov_n = st.cov_n;
+                const double rate = a.burnin_cumulative ? (double)st.t.rej / k : (double)st.t.reju / a.adaptint;
+                const double cov_n = st.t.cov_n;
                 const bool rdg = st.r_diag != 0;
                 __syncthreads();
                 const int rc = adapt(a, cx, k, cov_n, rate, rdg, nd);
                 if (tid == 0) {
-                    st.wcnt = wc0 + max(0, k - max(rr0, cx.first_row));
+                    st.t.wcnt = wc0 + max(0, k - max(rr0, cx.cc.first_row));
                     st.run_r0 = k; st.ndist = 0;
-                    if (a.do_cov) st.cov_n = cov_n + a.adaptint;
-                    if (rc == 1) { st.r_diag = 0; ++st.n_adapt; }
-                    else if (rc == 2) ++st.n_cholfail;
-                    st.reju = 0;
+                    if (a.do_cov) st.t.cov_n = cov_n + a.adaptint;
+                    if (rc == 1) { st.r_diag = 0; ++st.t.n_adapt; }
+                    else if (rc == 2) ++st.t.n_cholfail;
+                    st.t.reju = 0;
                 }
                 __syncthreads();
                 next_adapt += a.adaptint;
-                TC_PHASE(5);
+                TC_PHASE(PH_ADAPT);
             }
         }
 
@@ -2031,10 +2102,10 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
         if (!bad0 && st.run_r0 < k) {
             // close the last run (the fit or the slice does not end on an adaptation boundary)
             const int rr0 = st.run_r0;
-            const double wc0 = st.wcnt;
+            const double wc0 = st.t.wcnt;
             flush_run(a, cx, rr0, k, wc0, st.ndist, -1, 0);
             __syncthreads();
-            if (tid == 0) { st.wcnt = wc0 + max(0, k - max(rr0, cx.first_row)); st.run_r0 = k; }
+            if (tid == 0) { st.t.wcnt = wc0 + max(0, k - max(rr0, cx.cc.first_row)); st.run_r0 = k; }
             __syncthreads();
         }
         if (!last_seg && !bad0) {
@@ -2046,44 +2117,16 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                 gst[ST_VEC0 + 2 * a.ld + i] = cx.wM2[i];
                 gst[ST_VEC0 + 3 * a.ld + i] = cx.rdiag[i];
             }
-            if (tid == 0) {
-                gst[0] = st.ss; gst[1] = st.pri; gst[2] = st.sigma2; gst[3] = st.cov_n; gst[4] = st.wcnt; gst[5] = st.r_diag ? 1.0 : 0.0;
-                gst[6] = s_s2.sum; gst[7] = s_s2.sq_sum; gst[8] = 0.0; gst[9] = s_s2.cnt; gst[10] = st.rden; gst[11] = st.rsig;
-                long long *gc = reinterpret_cast<long long *>(gst + 16);
-                gc[0] = st.n_ss; gc[1] = st.n_acc1; gc[2] = st.n_acc2; gc[3] = st.n_oob; gc[4] = st.n_adapt; gc[5] = st.n_cholfail;
-                gc[6] = st.n_dr; gc[7] = st.n_spec; gc[8] = st.rej;
-                for (int i = 0; i < 8; ++i) gc[9 + i] = st.pc[i];
-            }
+            if (tid == 0) park_chain(gst, ParkedChain{st.ss, st.pri, st.sigma2, st.rsig, st.r_diag, 0, st.t});
             __threadfence();
             __syncthreads();
             if (tid == 0) atomicExch(a.cstate + ch, seg + 1);      // release: next slice, not running
             continue;
         }
 
-        // ---- summaries (TranscriptionCycleMCMC.m:286-303); a chain whose ss(x0) is not finite ends here
-        {
-            const double wcnt = st.wcnt;
-#pragma unroll 1
-            for (int i = tid; i < npar; i += DRAM_THREADS) {
-                if (a.mean) a.mean[(size_t)ch * a.ld + i] = bad0 ? 0.0 : cx.wmean[i];
-                if (a.std) a.std[(size_t)ch * a.ld + i] = (!bad0 && wcnt > 0) ? sqrt(cx.wM2[i] / wcnt) : 0.0;
-            }
-        }
+        // ---- summaries; a chain whose ss(x0) is not finite ends here
+        write_outputs(a, ch, npar, cx.wmean, cx.wM2, st.t, st.t.n_spec, bad0, tid, DRAM_THREADS);
         if (tid == 0) {
-            if (a.sig) {
-                // sqrt(mean(s2chain)); std(sqrt(s2chain),1) = sqrt(E[s2] - E[sqrt(s2)]^2)   (:302-303)
-                const double m2 = s_s2.sum / s_s2.cnt, m1 = s_s2.sq_sum / s_s2.cnt;
-                a.sig[2 * (size_t)ch] = bad0 ? 0.0 : sqrt(m2);
-                a.sig[2 * (size_t)ch + 1] = bad0 ? 0.0 : sqrt(fmax(m2 - m1 * m1, 0.0));
-            }
-            if (a.counters) {
-                long long *c = a.counters + (size_t)ch * TC_NCOUNTERS;
-                c[TC_CNT_SS_EVALS] = st.n_ss; c[TC_CNT_ACC_STAGE1] = st.n_acc1; c[TC_CNT_ACC_STAGE2] = st.n_acc2;
-                c[TC_CNT_OUT_OF_BOUNDS] = st.n_oob; c[TC_CNT_ADAPTATIONS] = st.n_adapt;
-                c[TC_CNT_CHOL_FAIL] = st.n_cholfail; c[TC_CNT_DR_TRIES] = st.n_dr; c[TC_CNT_STATUS] = bad0 ? 1 : 0;
-                for (int i = 0; i < 7; ++i) c[TC_CNT_CYCLES0 + i] = st.pc[i];
-                c[TC_CNT_CYCLES0 + 7] = st.n_spec;
-            }
             __threadfence();
             atomicExch(a.cstate + ch, nseg);                        // finished (also ends a chain whose ss(x0) failed)
         }

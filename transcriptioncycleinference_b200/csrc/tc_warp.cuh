@@ -44,15 +44,13 @@ __host__ __device__ inline int wk_region(int N) { return 2 * wk_ldp(N) + 2 + wk_
 
 // per-warp mutable book-keeping in shared memory (lane 0 writes; everything hot lives in registers)
 struct WkState {
-    double cov_n, wcnt, s2sum, s2sq, s2cnt;
-    long long n_ss, n_acc1, n_acc2, n_oob, n_adapt, n_cholfail, n_dr, rej, reju;
-    long long pc[8], tprev;                                         // phase clocks: 0 generate, 1 steps, 2 adapt, 3 barrier waits; 4-7 sub-phases
+    Tally t;
+    long long tprev;
 };
 // per-warp chain context (written by lane 0 when a slice is claimed)
 struct WkCtx {
-    int N, npar, ld, ldp, ch, first_row, nstore, o_s0, o_ov, o_work;
-    unsigned long long uid;
-    double inv_dr, adascale, chi_d, chi_c;
+    int N, npar, ld, ldp, ch, o_s0, o_ov, o_work;
+    ChainConsts cc;
     const double *lo, *hi, *mu, *pinv;
     double *gInc, *gSc, *gWs;                                        // this warp slot's scratch
     double *gR, *gM2, *gRows, *gWts, *cmean, *mb, *wmean, *wM2, *rdiag;
@@ -131,7 +129,7 @@ __device__ __forceinline__ void wk_increments(const WkCtx &c, int nnew)
     const ZT *Z1 = reinterpret_cast<const ZT *>(tc_smem + c.o_ov), *Z2 = Z1 + rows * ldz;
     const int NT = (npar + 7) >> 3, nt4 = (npar + 3) >> 2, inner = 4 * ak + (ar & 3);
     const bool rowok = ar < nnew;
-    const double inv_dr = c.inv_dr;
+    const double inv_dr = c.cc.inv_dr;
     // rows >= nnew of Z hold stale data: their results are dropped; columns >= npar are zero (wk_generate)
     const ZT *za1p = Z1 + (ar < rows ? ar : 0) * ldz + ak, *za2p = Z2 + (ar < rows ? ar : 0) * ldz + ak;
     double2 *out = reinterpret_cast<double2 *>(c.gInc) + (size_t)ar * c.ldp;
@@ -216,15 +214,15 @@ __device__ __noinline__ void wk_generate(const RunArgs &a, const WkCtx &c, int g
             const size_t g = (size_t)c.ch * a.nsimu + st;
             u1 = a.u1[g]; u2 = a.u2[g]; x2 = a.chi2[g];
         } else {
-            const u32x4 ru = draw(a.seed, c.uid, st, RK_U, 0);
+            const u32x4 ru = draw(a.seed, c.cc.uid, st, RK_U, 0);
             u1 = u01(ru.x, ru.y); u2 = u01(ru.z, ru.w);
-            x2 = a.updatesigma ? chi2_draw_dc(a.seed, c.uid, st, c.chi_d, c.chi_c) : 1.0;
+            x2 = a.updatesigma ? chi2_draw_dc(a.seed, c.cc.uid, st, c.cc.chi_d, c.cc.chi_c) : 1.0;
         }
         double *sc = c.gSc + 8 * lane;
         __stcg(sc + 0, u1); __stcg(sc + 1, u2); __stcg(sc + 2, x2); __stcg(sc + 5, tc_log(u1));
     }
     __syncwarp();
-    const double inv_dr = c.inv_dr;
+    const double inv_dr = c.cc.inv_dr;
     if (rep) {
         double *Z1 = tc_smem + c.o_ov, *Z2 = Z1 + WK_GENR * ldz;
 #pragma unroll 1
@@ -260,7 +258,7 @@ __device__ __noinline__ void wk_generate(const RunArgs &a, const WkCtx &c, int g
                 for (int u = 0; u < 4; ++u) {
                     const int q = q0 + lane + 32 * (u & 1), ss = s + (u >> 1);
                     on[u] = q < npairs && ss < nnew;
-                    z[u] = normal_quad_inl(a.seed, c.uid, g0 + ss, on[u] ? q : 0);   // (z1[2q], z1[2q+1], z2[2q], z2[2q+1]): FP32 values
+                    z[u] = normal_quad_inl(a.seed, c.cc.uid, g0 + ss, on[u] ? q : 0);   // (z1[2q], z1[2q+1], z2[2q], z2[2q+1]): FP32 values
                 }
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
@@ -292,7 +290,7 @@ __device__ __noinline__ void wk_generate(const RunArgs &a, const WkCtx &c, int g
         }
     }
     __syncwarp();
-    if (lane == 0) { WkState &st = wk_st[threadIdx.x >> 5]; st.pc[4] += clock64() - st.tprev; }    // sub-phase: randomness (tprev is not moved)
+    if (lane == 0) { WkState &st = wk_st[threadIdx.x >> 5]; st.t.pc[PH_RAND] += clock64() - st.tprev; }    // sub-phase: randomness (tprev is not moved)
     if (r_diag) {
         double2 *out = reinterpret_cast<double2 *>(c.gInc);
         const unsigned long long pol_k = wk_policy_keep();
@@ -397,7 +395,7 @@ __device__ __forceinline__ bool wk_propose2(const WkCtx &c, int ox, int ob, doub
 __device__ __noinline__ void wk_flush(const RunArgs &a, const WkCtx &c, int ox, int r0, int r1, double wcnt, int ndist)
 {
     const int lane = threadIdx.x & 31, npar = c.npar;
-    const int m_c = r1 - r0, rs = max(r0, c.first_row), m_w = r1 - rs;
+    const int m_c = r1 - r0, rs = max(r0, c.cc.first_row), m_w = r1 - rs;
     const bool cov = a.do_cov && m_c > 0;
     const double nn = wcnt + m_w, rnn = m_w > 0 ? tc_rcp(nn) : 0.0, f1 = m_w * rnn, f2 = wcnt * m_w * rnn;     // as flush_run()
     double *grow = cov ? c.gRows + (size_t)ndist * c.ld : nullptr;
@@ -409,7 +407,7 @@ __device__ __noinline__ void wk_flush(const RunArgs &a, const WkCtx &c, int ox, 
             __stcg(c.wmean + i, fma(d1, f1, wm));
             __stcg(c.wM2 + i, fma(d1 * d1, f2, __ldcg(c.wM2 + i)));
             if (a.store_chain && a.chain) {
-                double *dst = a.chain + ((size_t)c.ch * c.nstore + (rs - c.first_row)) * c.ld + i;
+                double *dst = a.chain + ((size_t)c.ch * c.cc.nstore + (rs - c.cc.first_row)) * c.ld + i;
 #pragma unroll 1
                 for (int r = 0; r < m_w; ++r) dst[(size_t)r * c.ld] = xo;
             }
@@ -623,7 +621,7 @@ __device__ __noinline__ int wk_adapt(const RunArgs &a, const WkCtx &c, int o_mb,
         cov_n += m;
         __syncwarp();
     }
-    if (lane == 0) { WkState &st = wk_st[threadIdx.x >> 5]; st.pc[5] += clock64() - st.tprev; }    // sub-phase: scatter update
+    if (lane == 0) { WkState &st = wk_st[threadIdx.x >> 5]; st.t.pc[PH_SCATTER] += clock64() - st.tprev; }    // sub-phase: scatter update
     if (isimu < a.burnintime) {
         double f = 1.0;
         if (rate > 0.95) f = 1.0 / a.burnin_scale;
@@ -644,11 +642,11 @@ __device__ __noinline__ int wk_adapt(const RunArgs &a, const WkCtx &c, int o_mb,
     // mcmcstat: chol(cov) first, chol(cov + qcovadj I) only when that fails [U]; qcovadj_always = 1 adds it at once
     bool ok = wk_chol(nt4, npar, c.gM2, invn, a.qcovadj_always ? a.qcovadj : 0.0, c.gWs, c.o_ov);
     if (!ok && !a.qcovadj_always) ok = wk_chol(nt4, npar, c.gM2, invn, a.qcovadj, c.gWs, c.o_ov);
-    if (lane == 0) { WkState &st = wk_st[threadIdx.x >> 5]; st.pc[6] += clock64() - st.tprev; }    // sub-phase: scatter + factorisation
+    if (lane == 0) { WkState &st = wk_st[threadIdx.x >> 5]; st.t.pc[PH_FACTOR] += clock64() - st.tprev; }    // sub-phase: scatter + factorisation
     if (ok) {
         const double2 *src = reinterpret_cast<const double2 *>(c.gWs);
         double2 *dst = reinterpret_cast<double2 *>(c.gR);
-        const double sc = c.adascale;
+        const double sc = c.cc.adascale;
 #pragma unroll 8
         for (int e = lane; e < 8 * T4; e += 32) { const double2 v = __ldcg(src + e); __stcg(dst + e, make_double2(v.x * sc, v.y * sc)); }
     }
@@ -745,13 +743,9 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
             N = a.cells.N[cid]; npar = 7 + N;
             gst = a.gState + (size_t)ch * state_doubles(a.ld);
             if (lane == 0) {
-                c.N = N; c.npar = npar; c.ld = a.ld; c.ldp = ldp; c.ch = ch; c.first_row = a.n_burn - 1;
-                c.nstore = a.nsimu - (a.n_burn - 1);
+                c.N = N; c.npar = npar; c.ld = a.ld; c.ldp = ldp; c.ch = ch;
                 c.o_s0 = o_reg + 1; c.o_ov = o_reg + 2 * ldp + 2; c.o_work = c.o_ov + wk_cell_sz(a.ld - 7);
-                c.uid = a.chain_uid ? a.chain_uid[ch] : (unsigned long long)ch;
-                c.inv_dr = 1.0 / a.drscale;
-                c.adascale = a.adascale > 0.0 ? a.adascale : 2.4 / sqrt((double)npar);
-                chi2_consts(a.N0 + 2.0 * N, c.chi_d, c.chi_c);
+                c.cc = chain_consts(a, ch, N);
                 c.lo = a.low + (size_t)ch * a.ld; c.hi = a.upp + (size_t)ch * a.ld; c.mu = a.pmu + (size_t)ch * a.ld;
                 c.pinv = a.gPinv + (size_t)ch * a.ld;
                 c.gInc = a.gInc + (size_t)slot * (2 * WK_GEN * ldp); c.gSc = a.gSc + (size_t)slot * (8 * WK_GEN);
@@ -790,9 +784,8 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                     for (int i = lane; i < 16 * (nt4 * (nt4 + 1) / 2); i += 32) __stcg(c.gM2 + i, 0.0);
                 }
                 if (lane == 0) {
-                    st.cov_n = 0.0; st.wcnt = 0.0; st.s2sum = 0.0; st.s2sq = 0.0; st.s2cnt = 0.0;
-                    st.n_ss = 1; st.n_acc1 = 0; st.n_acc2 = 0; st.n_oob = 0; st.n_adapt = 0; st.n_cholfail = 0; st.n_dr = 0; st.rej = 0; st.reju = 0;
-                    for (int i = 0; i < 8; ++i) st.pc[i] = 0;
+                    st.t = Tally{};
+                    st.t.n_ss = 1;                                      // ss(x0)
                 }
                 __syncwarp();
                 // row 0: x0
@@ -802,27 +795,15 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 for (int i = lane; i < npar; i += 32) { const double e = (tc_smem[ox + i] - __ldg(c.mu + i)) * __ldcg(c.pinv + i); sp += e * e; }
                 pri = warp_sum(sp);
                 bad0 = !isfinite(ss);
-                if (!bad0 && lane == 0) {
-                    st.s2sum = a.sigma2_0; st.s2sq = sqrt(a.sigma2_0); st.s2cnt = 1.0;
-                    if (a.store_chain && a.s2chain) a.s2chain[(size_t)ch * a.nsimu] = a.sigma2_0;
-                    if (a.flags) a.flags[(size_t)ch * a.nsimu] = 0;
-                    if (a.sschain) a.sschain[(size_t)ch * a.nsimu] = ss;
-                }
+                if (!bad0 && lane == 0) record_row0(a, ch, ss, st.t);
             } else {
 #pragma unroll 1
                 for (int i = lane; i < npar; i += 32) tc_smem[ox + i] = __ldcg(gst + ST_VEC0 + i);
-                ss = __ldcg(gst + 0); pri = __ldcg(gst + 1); sig2 = __ldcg(gst + 2); is2 = __ldcg(gst + 11);
-                r_diag = __ldcg(gst + 5) != 0.0;
-                bad0 = __ldcg(gst + 8) != 0.0;                          // ss(x0) was not finite: reported at slice 0, nothing left to do
+                const ParkedChain p = resume_chain(gst);
+                ss = p.ss; pri = p.pri; sig2 = p.sigma2; is2 = p.rsig; r_diag = p.r_diag;
+                bad0 = p.bad0 != 0;                                     // ss(x0) was not finite: reported at slice 0, nothing left to do
                 run_r0 = seg * a.seglen;
-                if (lane == 0) {
-                    st.cov_n = __ldcg(gst + 3); st.wcnt = __ldcg(gst + 4);
-                    st.s2sum = __ldcg(gst + 6); st.s2sq = __ldcg(gst + 7); st.s2cnt = __ldcg(gst + 9);
-                    const long long *gc = reinterpret_cast<const long long *>(gst + 16);
-                    st.n_ss = __ldcg(gc + 0); st.n_acc1 = __ldcg(gc + 1); st.n_acc2 = __ldcg(gc + 2); st.n_oob = __ldcg(gc + 3);
-                    st.n_adapt = __ldcg(gc + 4); st.n_cholfail = __ldcg(gc + 5); st.n_dr = __ldcg(gc + 6); st.rej = __ldcg(gc + 8); st.reju = __ldcg(gc + 7);
-                    for (int i = 0; i < 8; ++i) st.pc[i] = __ldcg(gc + 9 + i);
-                }
+                if (lane == 0) st.t = p.t;
             }
             // bounds / prior in the reference's structure?  (every slice: four vectors read once)
             {
@@ -845,12 +826,12 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
         const bool active = valid && !bad0;
 #ifdef WK_SUBPROF
 #define WK_T0 const long long t0__ = clock64()
-#define WK_T1(i) do { if (lane == 0) st.pc[i] += clock64() - t0__; } while (0)
+#define WK_T1(i) do { if (lane == 0) st.t.pc[i] += clock64() - t0__; } while (0)
 #else
 #define WK_T0
 #define WK_T1(i)
 #endif
-#define WK_PHASE(i) do { if (lane == 0) { const long long tn__ = clock64(); st.pc[i] += tn__ - st.tprev; st.tprev = tn__; } } while (0)
+#define WK_PHASE(i) do { if (lane == 0) { const long long tn__ = clock64(); st.t.pc[i] += tn__ - st.tprev; st.tprev = tn__; } } while (0)
 
         int k = seg == 0 ? 1 : seg * a.seglen;
         rden = tc_rcp(n0s20 + ss);                                  // (a function of ss alone: recomputed, not parked)
@@ -862,13 +843,13 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
             // against 55.5 k (9 568 chains)
             __syncthreads();
             if (active) {
-                WK_PHASE(3);
+                WK_PHASE(PH_WAIT);
                 wk_generate(a, c, g0, gen_upto - g0, r_diag != 0);
                 wk_stage_cell(a.cells, cid, cv);
-                WK_PHASE(0);
+                WK_PHASE(PH_GEN);
             }
             __syncthreads();                                            // phase alignment: the step loop
-            if (active) WK_PHASE(3);
+            if (active) WK_PHASE(PH_WAIT);
 #pragma unroll 1
             for (; k < gen_upto && active; ++k) {
                 const int row = k - g0;
@@ -884,7 +865,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 else {
                     WK_T0;
                     ss1 = ss_eval(a.cons, cv, SmemVecA{ob}, w, a.algo, false, nullptr, nullptr);
-                    WK_T1(7);
+                    WK_T1(PH_EVAL);
                     nev = 1;
                     x12 = -0.5 * ((ss1 - ss) * is2 + pr1 - pri);
                     if (x12 >= 0.0 || x12 > s_logu) acc = 1;
@@ -899,7 +880,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                     else {
                         WK_T0;
                         const double ss2 = ss_eval(a.cons, cv, SmemVecA{ob}, w, a.algo, false, nullptr, nullptr);
-                        WK_T1(7);
+                        WK_T1(PH_EVAL);
                         ++nev;
                         if (resolve_dr(-0.5 * (s_n1 - s_n0), s_u2, o1, x12, pr1, pr2, ss1, ss2, ss, pri, is2)) { acc = 2; fl |= TC_FL_STAGE2; ssn = ss2; prin = pr2; }
                     }
@@ -907,9 +888,9 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 // ---- commit
                 if (acc) {
                     fl |= TC_FL_ACCEPT;
-                    const double wcnt = st.wcnt;
+                    const double wcnt = st.t.wcnt;
                     wk_flush(a, c, ox, run_r0, k, wcnt, ndist);          // close the run of the old state at row k
-                    if (lane == 0) st.wcnt = wcnt + max(0, k - max(run_r0, c.first_row));
+                    if (lane == 0) st.t.wcnt = wcnt + max(0, k - max(run_r0, c.cc.first_row));
                     if (a.do_cov && k > run_r0) ++ndist;
                     run_r0 = k;
                     const int t_ = ox; ox = ob; ob = t_;                 // the proposal becomes the state
@@ -918,39 +899,37 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 }
                 const double s2 = a.updatesigma ? (n0s20 + ss) * tc_rcp(s_chi) : sig2;
                 if (lane == 0) {
-                    st.s2sum += s2; st.s2sq += sqrt(s2); st.s2cnt += 1.0;
-                    st.n_ss += nev; st.n_oob += noob; if (fl & TC_FL_DR) ++st.n_dr;
-                    if (acc == 1) ++st.n_acc1; else if (acc == 2) ++st.n_acc2; else { ++st.rej; ++st.reju; }
-                    if (a.store_chain && a.s2chain) a.s2chain[(size_t)ch * a.nsimu + k] = s2;
-                    if (a.flags) a.flags[(size_t)ch * a.nsimu + k] = fl;
-                    if (a.sschain) a.sschain[(size_t)ch * a.nsimu + k] = ss;
+                    st.t.s2sum += s2; st.t.s2sq += sqrt(s2); st.t.s2cnt += 1.0;
+                    st.t.n_ss += nev; st.t.n_oob += noob; if (fl & TC_FL_DR) ++st.t.n_dr;
+                    if (acc == 1) ++st.t.n_acc1; else if (acc == 2) ++st.t.n_acc2; else { ++st.t.rej; ++st.t.reju; }
+                    store_row(a, ch, k, s2, fl, ss);
                 }
                 if (a.updatesigma) { sig2 = s2; is2 = s_chi * rden; }
                 __syncwarp();
             }
             k = gen_upto;
-            if (active) WK_PHASE(1);
+            if (active) WK_PHASE(PH_STEPS);
             if (k == next_adapt) {
                 __syncthreads();                                        // phase alignment: adaptation
                 if (active) {
-                    WK_PHASE(3);
-                    const double wc0 = st.wcnt, cov_n = st.cov_n;
+                    WK_PHASE(PH_WAIT);
+                    const double wc0 = st.t.wcnt, cov_n = st.t.cov_n;
                     wk_flush(a, c, ox, run_r0, k, wc0, ndist);           // close the run at the block boundary
                     const int nd = ndist + ((a.do_cov && k > run_r0) ? 1 : 0);
-                    const double rate = a.burnin_cumulative ? (double)st.rej / k : (double)st.reju / a.adaptint;
+                    const double rate = a.burnin_cumulative ? (double)st.t.rej / k : (double)st.t.reju / a.adaptint;
                     __syncwarp();
                     const int rc = wk_adapt(a, c, ob, k, cov_n, rate, r_diag != 0, nd);
                     if (lane == 0) {
-                        st.wcnt = wc0 + max(0, k - max(run_r0, c.first_row));
-                        if (a.do_cov) st.cov_n = cov_n + a.adaptint;
-                        if (rc == 1) ++st.n_adapt; else if (rc == 2) ++st.n_cholfail;
-                        st.reju = 0;
+                        st.t.wcnt = wc0 + max(0, k - max(run_r0, c.cc.first_row));
+                        if (a.do_cov) st.t.cov_n = cov_n + a.adaptint;
+                        if (rc == 1) ++st.t.n_adapt; else if (rc == 2) ++st.t.n_cholfail;
+                        st.t.reju = 0;
                     }
                     if (rc == 1) r_diag = 0;
                     run_r0 = k; ndist = 0;
                     __syncwarp();
                     wk_stage_cell(a.cells, cid, cv);
-                    WK_PHASE(2);
+                    WK_PHASE(PH_ADAPT);
                 }
                 next_adapt += a.adaptint;
             }
@@ -958,9 +937,9 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
         if (valid) {
         __syncwarp();
         if (!bad0 && run_r0 < k) {
-            const double wc0 = st.wcnt;
+            const double wc0 = st.t.wcnt;
             wk_flush(a, c, ox, run_r0, k, wc0, ndist);
-            if (lane == 0) st.wcnt = wc0 + max(0, k - max(run_r0, c.first_row));
+            if (lane == 0) st.t.wcnt = wc0 + max(0, k - max(run_r0, c.cc.first_row));
             run_r0 = k;
             __syncwarp();
         }
@@ -970,46 +949,17 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
             // ---- park
 #pragma unroll 1
             for (int i = lane; i < npar; i += 32) __stcg(gst + ST_VEC0 + i, tc_smem[ox + i]);
-            if (lane == 0) {
-                gst[0] = ss; gst[1] = pri; gst[2] = sig2; gst[3] = st.cov_n; gst[4] = st.wcnt; gst[5] = r_diag ? 1.0 : 0.0;
-                gst[6] = st.s2sum; gst[7] = st.s2sq; gst[8] = 0.0; gst[9] = st.s2cnt; gst[11] = is2;
-                long long *gc = reinterpret_cast<long long *>(gst + 16);
-                gc[0] = st.n_ss; gc[1] = st.n_acc1; gc[2] = st.n_acc2; gc[3] = st.n_oob; gc[4] = st.n_adapt; gc[5] = st.n_cholfail;
-                gc[6] = st.n_dr; gc[7] = st.reju; gc[8] = st.rej;
-                for (int i = 0; i < 8; ++i) gc[9 + i] = st.pc[i];
-            }
+            if (lane == 0) park_chain(gst, ParkedChain{ss, pri, sig2, is2, r_diag, 0, st.t});
             __syncwarp();
         } else {
-        // ---- summaries (TranscriptionCycleMCMC.m:286-303)
-        {
-            const double wcnt = st.wcnt;
-#pragma unroll 1
-            for (int i = lane; i < npar; i += 32) {
-                if (a.mean) a.mean[(size_t)ch * a.ld + i] = bad0 ? 0.0 : __ldcg(c.wmean + i);
-                if (a.std) a.std[(size_t)ch * a.ld + i] = (!bad0 && wcnt > 0) ? sqrt(__ldcg(c.wM2 + i) / wcnt) : 0.0;
-            }
-        }
-        if (lane == 0) {
-            if (bad0) gst[8] = 1.0;
-            if (a.sig) {
-                const double m2 = st.s2sum / st.s2cnt, m1 = st.s2sq / st.s2cnt;
-                a.sig[2 * (size_t)ch] = bad0 ? 0.0 : sqrt(m2);
-                a.sig[2 * (size_t)ch + 1] = bad0 ? 0.0 : sqrt(fmax(m2 - m1 * m1, 0.0));
-            }
-            if (a.counters) {
-                long long *cn = a.counters + (size_t)ch * TC_NCOUNTERS;
-                cn[TC_CNT_SS_EVALS] = st.n_ss; cn[TC_CNT_ACC_STAGE1] = st.n_acc1; cn[TC_CNT_ACC_STAGE2] = st.n_acc2;
-                cn[TC_CNT_OUT_OF_BOUNDS] = st.n_oob; cn[TC_CNT_ADAPTATIONS] = st.n_adapt;
-                cn[TC_CNT_CHOL_FAIL] = st.n_cholfail; cn[TC_CNT_DR_TRIES] = st.n_dr; cn[TC_CNT_STATUS] = bad0 ? 1 : 0;
-                cn[TC_CNT_CYCLES0 + 0] = st.pc[0]; cn[TC_CNT_CYCLES0 + 1] = st.pc[1]; cn[TC_CNT_CYCLES0 + 2] = st.pc[3]; cn[TC_CNT_CYCLES0 + 3] = st.pc[4];
-                cn[TC_CNT_CYCLES0 + 4] = st.pc[5]; cn[TC_CNT_CYCLES0 + 5] = st.pc[2]; cn[TC_CNT_CYCLES0 + 6] = st.pc[6];
+            // ---- summaries
+            if (bad0 && lane == 0) reinterpret_cast<ParkedChain *>(gst)->bad0 = 1;
 #ifdef WK_SUBPROF
-                cn[TC_CNT_CYCLES0 + 7] = st.pc[7];
+            const long long slot7 = st.t.pc[PH_EVAL];
 #else
-                cn[TC_CNT_CYCLES0 + 7] = st.n_ss;                       // no speculation: every evaluation is committed
+            const long long slot7 = st.t.n_ss;                          // no speculation: every evaluation is committed
 #endif
-            }
-        }
+            write_outputs(a, ch, npar, c.wmean, c.wM2, st.t, slot7, bad0, lane, 32);
         }
         }
         // ---- release the group: its next slice may run on any CTA
