@@ -13,6 +13,7 @@ from . import build as _build
 MAX_SETS = 8
 MAX_GPUS = 8
 TC_EDIM = -4          # numel(t(1):dt:t(end)) != numel(t)
+TC_ESTATE = -6        # ss(theta0) not finite for a chain
 NCOUNTERS = 16
 ALGO_PAIRS, ALGO_TOEPLITZ = 0, 1
 CNT_SS_EVALS, CNT_ACC_STAGE1, CNT_ACC_STAGE2, CNT_OUT_OF_BOUNDS = 0, 1, 2, 3

@@ -160,6 +160,7 @@ struct RunArgs {
     unsigned long long seed;
     // chains
     int nchains, ld, ldR, do_cov, wsz, big;
+    int blk_rows;                                       // rows of the largest adaptation block: the distinct-row buffer of a chain
     const int *chain_cell;
     const unsigned long long *chain_uid;
     const double *theta0, *qcov_diag, *low, *upp, *pmu, *psig;
@@ -888,10 +889,23 @@ struct Tally {
     long long n_ss, n_acc1, n_acc2, n_oob, n_adapt, n_cholfail, n_dr;   // counters TC_CNT_SS_EVALS .. TC_CNT_DR_TRIES
     long long n_spec;                                   // dram_kernel: evaluations including the discarded speculative ones
     long long rej, reju;                                // rejected steps: in all, since the last adaptation
-    double s2sum, s2sq, s2cnt;                          // s2chain over ALL rows (TranscriptionCycleMCMC.m:302-303): sum s2, sum sqrt(s2), rows
+    double s2sum, s2cnt;                                // s2chain over ALL rows (TranscriptionCycleMCMC.m:302-303): sum s2, rows
+    double sqmean, sqM2;                                // ... mean of sqrt(s2) and sum of squared deviations from it (tally_s2)
     double wcnt, cov_n;                                 // rows in the Welford summaries, rows in the covariance
     long long pc[8];                                    // phase clocks (PH_*)
 };
+
+// Fold nb more rows of s2chain into the tally: sum s2b of their s2, mean mb and sum of squared deviations M2b of their sqrt(s2),
+// merged with Chan et al.'s update.  std(sqrt(s2chain),1) from two running sums, sqrt(E[s2] - E[sqrt(s2)]^2), cancels: with
+// sigma2 fixed it is ~1e-6 sqrt(sigma2) after 2e5 rows instead of 0.  One thread.  Out of line: inlined, it costs
+// dram_warp_kernel (at its 128-register cap) spill traffic on every step.
+__device__ __noinline__ void tally_s2(Tally &t, double nb, double s2b, double mb, double M2b)
+{
+    const double n = t.s2cnt + nb, d = mb - t.sqmean, f = nb * tc_rcp(n);
+    t.sqmean = fma(d, f, t.sqmean);
+    t.sqM2 += fma(d * d, t.s2cnt * f, M2b);
+    t.s2sum += s2b; t.s2cnt = n;
+}
 
 // A chain between two time slices: its slot of gState (state_doubles(ld) doubles) holds this record, then the vectors
 // x | wmean | wM2 | rdiag, ld doubles each (dram_warp_kernel keeps the last three there all along).  16-byte aligned: the vectors
@@ -933,7 +947,7 @@ __device__ __forceinline__ void store_row(const RunArgs &a, int ch, int r, doubl
 // Row 0 = x0 with a finite ss0: s2 = sigma2_0 (TranscriptionCycleMCMC.m:259), no flags.  One thread.
 __device__ __forceinline__ void record_row0(const RunArgs &a, int ch, double ss0, Tally &t)
 {
-    t.s2sum += a.sigma2_0; t.s2sq += sqrt(a.sigma2_0); t.s2cnt += 1.0;
+    tally_s2(t, 1.0, a.sigma2_0, sqrt(a.sigma2_0), 0.0);
     store_row(a, ch, 0, a.sigma2_0, 0, ss0);
 }
 
@@ -953,10 +967,9 @@ __device__ void write_outputs(const RunArgs &a, int ch, int npar, const double *
     }
     if (i0 != 0) return;
     if (a.sig) {
-        // sqrt(mean(s2chain)); std(sqrt(s2chain),1) = sqrt(E[s2] - E[sqrt(s2)]^2)   (:302-303)
-        const double m2 = t.s2sum / t.s2cnt, m1 = t.s2sq / t.s2cnt;
-        a.sig[2 * (size_t)ch] = bad0 ? 0.0 : sqrt(m2);
-        a.sig[2 * (size_t)ch + 1] = bad0 ? 0.0 : sqrt(fmax(m2 - m1 * m1, 0.0));
+        // sqrt(mean(s2chain)); std(sqrt(s2chain),1) = sqrt(M2 / rows) of the running (mean, M2) of sqrt(s2)   (:302-303)
+        a.sig[2 * (size_t)ch] = bad0 ? 0.0 : sqrt(t.s2sum / t.s2cnt);
+        a.sig[2 * (size_t)ch + 1] = bad0 ? 0.0 : sqrt(t.sqM2 / t.s2cnt);
     }
     if (a.counters) {
         long long *c = a.counters + (size_t)ch * TC_NCOUNTERS;
@@ -1465,8 +1478,8 @@ __device__ __forceinline__ void scaled_copy_cg(double2 *dst, const double2 *src,
     for (; e < n; e += DRAM_THREADS) { const double2 v = __ldcg(src + e); dst[e] = make_double2(v.x * sc, v.y * sc); }
 }
 
-// Adaptation after the step with isimu (a multiple of adaptint).  The block of the last adaptint chain rows
-// arrives as `ndist` DISTINCT rows with integer weights (a rejected step repeats the previous row): the
+// Adaptation after the step with isimu (a multiple of adaptint).  The block of chain rows since the last adaptation (adaptint
+// of them; the first block is rows 0 .. isimu-1, which is 2 rows when adaptint = 1) arrives as `ndist` DISTINCT rows with integer weights (a rejected step repeats the previous row): the
 // scatter of the block is sum_d w_d (x_d - mb)(x_d - mb)', folded into the running scatter matrix with
 // Chan's mean-shift term as one more weighted row, in 4x4 register tiles.  Then either burn-in scaling or
 // R = chol(cov + qcovadj I) * adascale.  Returns 0: R unchanged / scaled, 1: new full factor, 2: Cholesky failed.
@@ -1478,7 +1491,7 @@ __device__ __noinline__ int adapt(const RunArgs &a, const ChainCtx &cx, int isim
                                                        // (offset arithmetic on tc_smem compiles to LDS / STS, cx.ring would be generic)
     SUBP_BEGIN;
     if (a.do_cov) {
-        const int m = a.adaptint;
+        const int m = isimu - (int)cov_n;                              // rows of the block: adaptint (rows 0 and 1 when adaptint = 1)
         const double fcorr = cov_n * m / (cov_n + m);
         const int nrows = ndist + (cov_n > 0.0 ? 1 : 0);              // + the mean-shift row
 #pragma unroll 1
@@ -1803,8 +1816,8 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                 cx.U = tc_smem + o;
                 cx.gRb = a.gR + (size_t)ch * a.ldR;                 // the factor R lives in HBM/L2 (4x4 tiles)
                 cx.gM2 = a.gM2 ? a.gM2 + (size_t)ch * a.ldR : nullptr;
-                cx.gRows = a.gRows ? a.gRows + (size_t)ch * (size_t)a.adaptint * a.ld : nullptr;
-                cx.gWts = a.gWts ? a.gWts + (size_t)ch * (size_t)a.adaptint : nullptr;
+                cx.gRows = a.gRows ? a.gRows + (size_t)ch * (size_t)a.blk_rows * a.ld : nullptr;
+                cx.gWts = a.gWts ? a.gWts + (size_t)ch * (size_t)a.blk_rows : nullptr;
                 cx.cmean = a.gCmean ? a.gCmean + (size_t)ch * a.ld : nullptr;
             }
             load_cell(a.cells, cid, cv);
@@ -2050,14 +2063,21 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                     sq = sqrt(s2);
                     store_row(a, cx.ch, r, s2, so_.fl, ssr);
                 }
+                // the round's sum of s2, and mean of sqrt(s2) and squared deviations from it (rows = lanes < ncommit <= RING / 2)
+                double s2b = s2, mb = sq;
 #pragma unroll
-                for (int o = RING / 2; o > 0; o >>= 1) { s2 += __shfl_xor_sync(0xffffffffu, s2, o); sq += __shfl_xor_sync(0xffffffffu, sq, o); }
+                for (int o = RING / 2; o > 0; o >>= 1) { s2b += __shfl_xor_sync(0xffffffffu, s2b, o); mb += __shfl_xor_sync(0xffffffffu, mb, o); }
+                mb *= tc_rcp((double)ncommit);
+                double dq = lane < ncommit ? sq - mb : 0.0;
+                dq *= dq;
+#pragma unroll
+                for (int o = RING / 2; o > 0; o >>= 1) dq += __shfl_xor_sync(0xffffffffu, dq, o);
                 const int d_ss = __reduce_add_sync(0xffffffffu, lane < ncommit ? so_.nev : 0);
                 const int d_oob = __reduce_add_sync(0xffffffffu, lane < ncommit ? so_.noob : 0);
                 const int d_dr = __reduce_add_sync(0xffffffffu, (lane < ncommit && (so_.fl & TC_FL_DR)) ? 1 : 0);
                 const int d_spec = __shfl_sync(0xffffffffu, inc, nsteps - 1);       // evaluations of this round
                 if (lane == 0) {
-                    st.t.s2sum += s2; st.t.s2sq += sq; st.t.s2cnt += ncommit;
+                    tally_s2(st.t, ncommit, s2b, mb, dq);
                     const int nrej = accd ? first : nsteps;
                     st.t.n_ss += d_ss; st.t.n_oob += d_oob; st.t.n_dr += d_dr; st.t.n_spec += d_spec;
                     st.t.rej += nrej; st.t.reju += nrej;
@@ -2087,7 +2107,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                 if (tid == 0) {
                     st.t.wcnt = wc0 + max(0, k - max(rr0, cx.cc.first_row));
                     st.run_r0 = k; st.ndist = 0;
-                    if (a.do_cov) st.t.cov_n = cov_n + a.adaptint;
+                    if (a.do_cov) st.t.cov_n = k;
                     if (rc == 1) { st.r_diag = 0; ++st.t.n_adapt; }
                     else if (rc == 2) ++st.t.n_cholfail;
                     st.t.reju = 0;
@@ -2672,6 +2692,8 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
         a.drscale = o->drscale; a.adascale = o->adascale; a.qcovadj = o->qcovadj; a.burnin_scale = o->burnin_scale;
         a.N0 = o->N0; a.S20 = o->S20; a.sigma2_0 = o->sigma2_0; a.seed = o->seed;
         a.nchains = nc; a.ld = ld; a.ldR = ldR; a.do_cov = do_cov ? 1 : 0;
+        // the first block is rows 0 .. isimu-1 of the first adaptation (row 0 is x0, no step): with adaptint = 1 that is 2 rows
+        a.blk_rows = std::max(o->adaptint, 2);
         int *d_cell; unsigned long long *d_uid; double *d;
         CUDA_TRY(up(r.buf, d_cell, (const int *)chain_cell + o0, nc, r.st)); a.chain_cell = d_cell;
         std::vector<unsigned long long> uid(nc);
@@ -2708,8 +2730,8 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
         CUDA_TRY(r.buf.alloc(a.gR, (size_t)nc * ldR));
         if (do_cov) {
             CUDA_TRY(r.buf.alloc(a.gM2, (size_t)nc * ldR));
-            CUDA_TRY(r.buf.alloc(a.gRows, (size_t)nc * o->adaptint * ld));
-            CUDA_TRY(r.buf.alloc(a.gWts, (size_t)nc * o->adaptint));
+            CUDA_TRY(r.buf.alloc(a.gRows, (size_t)nc * a.blk_rows * ld));
+            CUDA_TRY(r.buf.alloc(a.gWts, (size_t)nc * a.blk_rows));
             CUDA_TRY(r.buf.alloc(a.gCmean, (size_t)nc * ld));
         }
         int optin = 0, sms = 0;
@@ -2730,8 +2752,9 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
         if (o->layout == TC_LAYOUT_WARP && !warp_fits)
             return fail(TC_EINVAL, "max(N) = " + std::to_string(Nmax) + " is too large for the chain-per-warp layout");
         const bool use_warp = o->layout == TC_LAYOUT_WARP || (o->layout == TC_LAYOUT_AUTO && warp_fits && !a.big && nc >= TC_WARP_MIN_CHAINS_PER_SM * sms);   // TC_LAYOUT_CTA / _BIG: never
-        // time slices: a multiple of adaptint, ~32 per chain
-        const int unit = o->adaptint > 0 ? o->adaptint : 1;
+        // time slices: ~32 per chain, each ending on an adaptation step (a slice parks no partial covariance block): a multiple
+        // of adaptint, and of 2 when adaptint = 1 (the first adaptation is at isimu = 2, so k = 1 would split the first block)
+        const int unit = o->adaptint > 1 ? o->adaptint : (o->adaptint == 1 ? 2 : 1);
         long long sl = ((long long)o->nsimu + 31) / 32;
         CUDA_TRY(r.buf.alloc(a.smctl, 1024));
         CUDA_TRY(cudaMemsetAsync(a.smctl, 0, sizeof(int) * 1024, r.st));

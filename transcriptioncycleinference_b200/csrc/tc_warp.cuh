@@ -606,7 +606,7 @@ __device__ __noinline__ int wk_adapt(const RunArgs &a, const WkCtx &c, int o_mb,
     const int lane = threadIdx.x & 31, npar = c.npar;
     const int nt4 = (npar + 3) >> 2, T4 = nt4 * (nt4 + 1) / 2;
     if (a.do_cov) {
-        const int m = a.adaptint;
+        const int m = isimu - (int)cov_n;                           // rows of the block (adapt())
         wk_prefetch_l2(c.gM2, T4);                                  // the scatter matrix: HBM -> L2
 #pragma unroll 1
         for (int i = lane; i < npar; i += 32) tc_smem[o_mb + i] = __ldcg(c.mb + i) / m;
@@ -752,8 +752,8 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 c.gWs = a.gW ? a.gW + (size_t)slot * a.ldR : nullptr;
                 c.gR = a.gR + (size_t)ch * a.ldR;
                 c.gM2 = a.gM2 ? a.gM2 + (size_t)ch * a.ldR : nullptr;
-                c.gRows = a.gRows ? a.gRows + (size_t)ch * (size_t)a.adaptint * a.ld : nullptr;
-                c.gWts = a.gWts ? a.gWts + (size_t)ch * (size_t)a.adaptint : nullptr;
+                c.gRows = a.gRows ? a.gRows + (size_t)ch * (size_t)a.blk_rows * a.ld : nullptr;
+                c.gWts = a.gWts ? a.gWts + (size_t)ch * (size_t)a.blk_rows : nullptr;
                 c.cmean = a.gCmean ? a.gCmean + (size_t)ch * a.ld : nullptr;
                 c.mb = a.gMb ? a.gMb + (size_t)ch * a.ld : nullptr;
                 c.wmean = gst + ST_VEC0 + a.ld; c.wM2 = gst + ST_VEC0 + 2 * a.ld; c.rdiag = gst + ST_VEC0 + 3 * a.ld;
@@ -899,7 +899,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 }
                 const double s2 = a.updatesigma ? (n0s20 + ss) * tc_rcp(s_chi) : sig2;
                 if (lane == 0) {
-                    st.t.s2sum += s2; st.t.s2sq += sqrt(s2); st.t.s2cnt += 1.0;
+                    tally_s2(st.t, 1.0, s2, sqrt(s2), 0.0);                 // Welford: a batch of one row
                     st.t.n_ss += nev; st.t.n_oob += noob; if (fl & TC_FL_DR) ++st.t.n_dr;
                     if (acc == 1) ++st.t.n_acc1; else if (acc == 2) ++st.t.n_acc2; else { ++st.t.rej; ++st.t.reju; }
                     store_row(a, ch, k, s2, fl, ss);
@@ -921,7 +921,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                     const int rc = wk_adapt(a, c, ob, k, cov_n, rate, r_diag != 0, nd);
                     if (lane == 0) {
                         st.t.wcnt = wc0 + max(0, k - max(run_r0, c.cc.first_row));
-                        if (a.do_cov) st.t.cov_n = cov_n + a.adaptint;
+                        if (a.do_cov) st.t.cov_n = k;
                         if (rc == 1) ++st.t.n_adapt; else if (rc == 2) ++st.t.n_cholfail;
                         st.t.reju = 0;
                     }
