@@ -197,23 +197,24 @@ def test_time_slices_are_transparent(gpu_cells, cells_npz, orc):
     dict(burnin_cumulative=0),                      # burn-in scaling on the rejection rate since the last adaptation
     dict(adaptint=64, drscale=3.0, qcovadj=1e-6),   # other adaptation interval / DR scale / regulariser
 ])
-def test_replay_option_variants(gpu_cells, cells_npz, orc, variant):
+@pytest.mark.parametrize("layout", [3, 2, 1], ids=["cta", "warp", "big"])   # TC_LAYOUT_CTA, _WARP, _BIG
+def test_replay_option_variants(gpu_cells, cells_npz, orc, variant, layout):
     """Every tc_mcmc_opts field that changes the DRAM arithmetic, replayed against the oracle with the same
-    injected randomness: flags identical, chains equal."""
+    injected randomness on every sampler layout: flags identical, chains equal."""
     from transcriptioncycleinference_b200 import _lib
     co, _ = orc
     chain_cell = np.array([7, 123, 250], dtype=np.int32)
     nsimu, burn = 420, 150
     inputs = _setup(gpu_cells, chain_cell, 61)
     st = _streams(len(chain_cell), nsimu, gpu_cells.ld, cells_npz["N"][chain_cell], 62)
-    opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, replay=1, **SHORT, **variant)
+    opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, replay=1, layout=layout, **SHORT, **variant)
     out = gpu_cells.mcmc_run(opts, chain_cell, *inputs, replay=st, want_flags=True)
     for i, c in enumerate(chain_cell):
         N = int(cells_npz["N"][c]); o = int(cells_npz["off"][c]); npar = 7 + N
         t, ms2, pp7 = (cells_npz[k][o:o + N] for k in ("t", "ms2", "pp7"))
         sti = dict(z1=st["z1"][i][:, :npar], u1=st["u1"][i], z2=st["z2"][i][:, :npar], u2=st["u2"][i], chi2=st["chi2"][i])
         ref = co.dram(orc[1], t, ms2, pp7, co.default_opts(nsimu, burn, **SHORT, **variant), *[x[i, :npar] for x in inputs], streams=sti)
-        assert np.array_equal(out["flags"][i], ref["flags"]), (variant, i)
+        assert np.array_equal(out["flags"][i], ref["flags"]), (variant, layout, i)
         np.testing.assert_allclose(out["chain"][i][:, :npar], ref["chain"], rtol=0, atol=1e-7)
         np.testing.assert_allclose(out["s2chain"][i], ref["s2chain"], rtol=1e-9)
 

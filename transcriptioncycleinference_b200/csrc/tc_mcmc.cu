@@ -192,10 +192,12 @@ struct RunArgs {
 // Ring + per-warp areas are contiguous: during adaptation (when both are idle) they are the workspace of
 // the covariance update and of the Cholesky factorisation.
 __host__ __device__ __forceinline__ int tidx(int nt4, int bi, int bj) { return bi * nt4 - (bi * (bi - 1)) / 2 + (bj - bi); }
+// doubles of an n x n upper triangle in 4x4 tiles (the factor R, the scatter matrix M2, a Cholesky workspace)
+__host__ __device__ __forceinline__ int tri_doubles(int n) { const int nt4 = (n + 3) >> 2; return 16 * (nt4 * (nt4 + 1) / 2); }
 __host__ __device__ inline int chol_ws_doubles(int n)
 {
-    const int nt4 = (n + 3) >> 2, T = nt4 * (nt4 + 1) / 2;
-    return 16 * T + (T + 3) / 4 + 2;                      // tiles + the u16 tile table
+    const int d = tri_doubles(n), T = d / 16;
+    return d + (T + 3) / 4 + 2;                           // tiles + the u16 tile table
 }
 
 // one ring slot = [pad | increments of stage 1: s1 doubles | of stage 2: s1 | pad | 8 per-step scalars]; the two increment
@@ -907,6 +909,88 @@ __device__ __noinline__ void tally_s2(Tally &t, double nb, double s2b, double mb
     t.s2sum += s2b; t.s2cnt = n;
 }
 
+// The rules both samplers decide and count by, each written once.  They take and return scalars (a pointer into shared memory
+// would make every access generic, §3 of DESIGN.md) and keep the association the replay tests pin bit for bit.
+
+// reciprocal prior width: an infinite width is a flat prior
+__device__ __forceinline__ double prior_inv(double sg) { return isinf(sg) ? 0.0 : 1.0 / sg; }
+
+// Slice seg of a chain: steps [k, k_end) (row 0 is x0, no step), and the first step whose isimu is a multiple of adaptint,
+// which triggers an adaptation (kept as a running value afterwards: an integer division per round is ~40 dependent instructions)
+struct Slice { int k, k_end, next_adapt; bool last; };
+__device__ __forceinline__ Slice slice_of(const RunArgs &a, int seg)
+{
+    Slice s;
+    s.k = seg == 0 ? 1 : seg * a.seglen;
+    s.k_end = min(a.nsimu, (seg + 1) * a.seglen);
+    s.last = s.k_end >= a.nsimu;
+    s.next_adapt = a.adaptint > 0 ? ((s.k + a.adaptint) / a.adaptint) * a.adaptint : 0x7fffffff;
+    return s;
+}
+
+// 1 / (N0 S20 + ss): a step that sees sigma2 = (N0 S20 + ss) / chi2 uses 1 / sigma2 = chi2 * rden_of(ss)
+__device__ __forceinline__ double rden_of(double n0s20, double ss) { return tc_rcp(n0s20 + ss); }
+// sigma2 of a row (the draw made from the row's ss and chi2), or the fixed sigma2 without updatesigma
+__device__ __forceinline__ double row_sigma2(int updatesigma, double n0s20, double ss, double chi2, double sig2)
+{
+    return updatesigma ? (n0s20 + ss) * tc_rcp(chi2) : sig2;
+}
+// Stage 1, decided in the log domain: a12 = exp(x12) > u1 <=> x12 >= 0 or x12 > log u1 (no exponential); x12 goes on to resolve_dr
+__device__ __forceinline__ bool stage1_accepts(double ss1, double ss, double is2, double pr1, double pri, double logu, double &x12)
+{
+    x12 = -0.5 * ((ss1 - ss) * is2 + pr1 - pri);
+    return x12 >= 0.0 || x12 > logu;
+}
+
+// A run (the rows [r0, r1), all equal to the state) closes: the rows it adds to the Welford summaries (those >= first_row),
+// and whether it is one more distinct row of the covariance block
+__device__ __forceinline__ int run_rows(int r0, int r1, int first_row) { return max(0, r1 - max(r0, first_row)); }
+__device__ __forceinline__ bool run_distinct(int do_cov, int r0, int r1) { return do_cov && r1 > r0; }
+// Welford weights of m_w rows folded into wcnt rows (mean += d f1, M2 += d^2 f2) through ONE reciprocal (two quotients were
+// ~300 cycles at the head of every accept)
+__device__ __forceinline__ void welford_weights(double wcnt, int m_w, double &f1, double &f2)
+{
+    const double nn = wcnt + m_w, rnn = m_w > 0 ? tc_rcp(nn) : 0.0;
+    f1 = m_w * rnn; f2 = wcnt * m_w * rnn;
+}
+
+// Rejection rate the burn-in scaling looks at after step k: since the start (burnin_cumulative) or since the last adaptation
+__device__ __forceinline__ double adapt_rate(const RunArgs &a, long long rej, long long reju, int k)
+{
+    return a.burnin_cumulative ? (double)rej / k : (double)reju / a.adaptint;
+}
+// Burn-in scales R by this factor (1: R unchanged)
+__device__ __forceinline__ double burnin_factor(double rate, double burnin_scale)
+{
+    double f = 1.0;
+    if (rate > 0.95) f = 1.0 / burnin_scale;
+    else if (rate < 0.05) f = burnin_scale;
+    return f;
+}
+// The covariance block closed at isimu, when the covariance holds cov_n rows: its m rows (adaptint; rows 0 .. isimu-1 for the
+// first block, which is 2 rows when adaptint = 1), the rows of its scatter update (ndist distinct rows + Chan's mean-shift row,
+// once there is a covariance) with the weight fcorr of the mean-shift row, and the share `shift` of the block's mean in the new
+// covariance mean
+struct CovBlock { int m, nrows; double fcorr, shift; };
+__device__ __forceinline__ CovBlock cov_block(int isimu, double cov_n, int ndist)
+{
+    CovBlock b;
+    b.m = isimu - (int)cov_n;
+    b.fcorr = cov_n * b.m / (cov_n + b.m);
+    b.nrows = ndist + (cov_n > 0.0 ? 1 : 0);
+    b.shift = b.m / (cov_n + b.m);
+    return b;
+}
+// The tally after the adaptation at isimu = k that returned rc (1: new factor, 2: Cholesky failed); the caller starts a new
+// run and block at k, and leaves the diagonal proposal when rc = 1
+__device__ __forceinline__ void after_adapt(Tally &t, int do_cov, int k, int rc)
+{
+    if (do_cov) t.cov_n = k;
+    if (rc == 1) ++t.n_adapt;
+    else if (rc == 2) ++t.n_cholfail;
+    t.reju = 0;
+}
+
 // A chain between two time slices: its slot of gState (state_doubles(ld) doubles) holds this record, then the vectors
 // x | wmean | wM2 | rdiag, ld doubles each (dram_warp_kernel keeps the last three there all along).  16-byte aligned: the vectors
 // after it stay aligned, and it moves through L2 as 16-byte words.
@@ -1014,17 +1098,16 @@ struct ChainCtx {
 // Fold the run into the summaries (Welford with multiplicity; rows >= n_burn-1 only), the optional chain
 // storage, and the distinct-row buffer of the current covariance block (row + weight); then, when
 // so >= 0, move the state: x += increment at tc_smem[so + i].  Every thread owns the indices i = tid, tid+256, ..
-// so the whole thing is one pass.  The caller accounts for wcnt / ndist with the same formulas.
+// so the whole thing is one pass.
 __device__ __noinline__ void flush_run(const RunArgs &a, const ChainCtx &cx, int r0, int r1, double wcnt, int ndist, int so, int t0)
 {
     // threads t0 .. DRAM_THREADS-1 take part (t0 = 32 at an accept: warp 0 writes the per-row scalars meanwhile)
     const int tid = (int)threadIdx.x - t0, nthr = DRAM_THREADS - t0, npar = cx.npar;
     if (tid < 0) return;
-    const int m_c = r1 - r0, rs = max(r0, cx.cc.first_row), m_w = r1 - rs;
-    const bool cov = a.do_cov && m_c > 0;
-    // Welford weights m_w / nn and wcnt m_w / nn through ONE reciprocal (every thread computes them: two quotients were ~300
-    // cycles at the head of every accept)
-    const double nn = wcnt + m_w, rnn = m_w > 0 ? tc_rcp(nn) : 0.0, f1 = m_w * rnn, f2 = wcnt * m_w * rnn;
+    const int m_c = r1 - r0, rs = max(r0, cx.cc.first_row), m_w = run_rows(r0, r1, cx.cc.first_row);
+    const bool cov = run_distinct(a.do_cov, r0, r1);
+    double f1, f2;
+    welford_weights(wcnt, m_w, f1, f2);
     double *grow = cov ? cx.gRows + (size_t)ndist * cx.ld : nullptr;
     const int ox = cx.o_x, owm = cx.o_wmean, ow2 = cx.o_wM2, omb = cx.o_mb;
 #pragma unroll 1
@@ -1491,9 +1574,9 @@ __device__ __noinline__ int adapt(const RunArgs &a, const ChainCtx &cx, int isim
                                                        // (offset arithmetic on tc_smem compiles to LDS / STS, cx.ring would be generic)
     SUBP_BEGIN;
     if (a.do_cov) {
-        const int m = isimu - (int)cov_n;                              // rows of the block: adaptint (rows 0 and 1 when adaptint = 1)
-        const double fcorr = cov_n * m / (cov_n + m);
-        const int nrows = ndist + (cov_n > 0.0 ? 1 : 0);              // + the mean-shift row
+        const CovBlock blk = cov_block(isimu, cov_n, ndist);
+        const int m = blk.m, nrows = blk.nrows;
+        const double fcorr = blk.fcorr;
 #pragma unroll 1
         for (int i = tid; i < npar; i += DRAM_THREADS) {
             const double mbi = cx.mb[i] / m;
@@ -1574,30 +1657,28 @@ __device__ __noinline__ int adapt(const RunArgs &a, const ChainCtx &cx, int isim
         SUBP(8);
         __syncthreads();
 #pragma unroll 1
-        for (int i = tid; i < npar; i += DRAM_THREADS) { cx.cmean[i] = __ldcg(cx.cmean + i) + cx.dm[i] * (m / (cov_n + m)); cx.mb[i] = 0.0; }
+        for (int i = tid; i < npar; i += DRAM_THREADS) { cx.cmean[i] = __ldcg(cx.cmean + i) + cx.dm[i] * blk.shift; cx.mb[i] = 0.0; }
         cov_n += m;
         __syncthreads();
         SUBP(9);
     }
     int ret = 0;
     if (isimu < a.burnintime) {
-        double f = 1.0;
-        if (rate > 0.95) f = 1.0 / a.burnin_scale;
-        else if (rate < 0.05) f = a.burnin_scale;
+        const double f = burnin_factor(rate, a.burnin_scale);
         if (f != 1.0) {
             if (r_diag) {
 #pragma unroll 1
                 for (int i = tid; i < npar; i += DRAM_THREADS) cx.rdiag[i] *= f;
             } else {
 #pragma unroll 1
-                for (int i = tid; i < 16 * (((npar + 3) >> 2) * (((npar + 3) >> 2) + 1) / 2); i += DRAM_THREADS) cx.gRb[i] = __ldcg(cx.gRb + i) * f;
+                for (int i = tid; i < tri_doubles(npar); i += DRAM_THREADS) cx.gRb[i] = __ldcg(cx.gRb + i) * f;
                 if (a.big) fence_async_proxy();
             }
         }
     } else {
         // R = chol(cov + qcovadj I) * adascale, factorised in shared memory (tiled layout), kept in HBM/L2
         const double invn = 1.0 / (cov_n - 1.0);
-        const int nt4 = (npar + 3) >> 2, T4 = nt4 * (nt4 + 1) / 2;
+        const int nt4 = (npar + 3) >> 2, T4 = tri_doubles(npar) / 16;
         // mcmcstat: [Ra,is] = chol(cov); only when that fails ("try to blow it") chol(cov + qcovadj I)  [U]; qcovadj_always = 1
         // factors cov + qcovadj I at once
         if (a.big) {
@@ -1777,8 +1858,6 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
         if (ch < 0) break;                                  // every chain is finished (own is false here)
         start = (ch + 1) % a.nchains;
         __threadfence();
-        const int k_end = min(a.nsimu, (seg + 1) * a.seglen);
-        const bool last_seg = k_end >= a.nsimu;
         const int cid = a.chain_cell[ch];
         const int N = a.cells.N[cid];
         const int npar = 7 + N;
@@ -1834,8 +1913,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                 cx.hi[i] = a.upp[g];
                 cx.mu[i] = a.pmu[g];
             }
-            const double sg = a.psig[g];
-            cx.pinv[i] = isinf(sg) ? 0.0 : 1.0 / sg;
+            cx.pinv[i] = prior_inv(a.psig[g]);
             cx.mb[i] = 0.0;
             if (seg == 0) {
                 cx.x[i] = a.theta0[g];
@@ -1853,7 +1931,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
         if (seg == 0) {
             if (a.do_cov) {
 #pragma unroll 1
-                for (int i = tid; i < 16 * (((npar + 3) >> 2) * (((npar + 3) >> 2) + 1) / 2); i += DRAM_THREADS) cx.gM2[i] = 0.0;
+                for (int i = tid; i < tri_doubles(npar); i += DRAM_THREADS) cx.gM2[i] = 0.0;
             }
             // ring slot 0 = zero increments: row 0 evaluates ss(x0) through the same theta view as every step
 #pragma unroll 1
@@ -1872,9 +1950,8 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             diff = __syncthreads_or(diff);
             if (tid == 0) {
                 const size_t g = (size_t)ch * a.ld + 7;
-                const double s7 = a.psig[g];
                 cx.uni = diff ? 0 : 1;
-                cx.blk[0] = a.low[g]; cx.blk[1] = a.upp[g]; cx.blk[2] = a.pmu[g]; cx.blk[3] = isinf(s7) ? 0.0 : 1.0 / s7;
+                cx.blk[0] = a.low[g]; cx.blk[1] = a.upp[g]; cx.blk[2] = a.pmu[g]; cx.blk[3] = prior_inv(a.psig[g]);
             }
         }
         if (tid == 0) {
@@ -1888,7 +1965,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                 // is off and nothing reads it)
                 const ParkedChain p = resume_chain(gst);
                 st.ss = p.ss; st.pri = p.pri; st.sigma2 = p.sigma2; st.rsig = p.rsig; st.r_diag = p.r_diag;
-                st.rden = tc_rcp(a.N0 * a.S20 + p.ss);
+                st.rden = rden_of(a.N0 * a.S20, p.ss);
                 st.t = p.t;
                 st.run_r0 = seg * a.seglen;
             }
@@ -1909,16 +1986,15 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             sp = warp_sum(sp);
             const bool bad = !isfinite(ss0);
             if (tid == 0) {
-                st.ss = ss0; st.pri = sp; st.bad0 = bad ? 1 : 0; st.rden = tc_rcp(a.N0 * a.S20 + ss0); st.rsig = 1.0 / a.sigma2_0;
+                st.ss = ss0; st.pri = sp; st.bad0 = bad ? 1 : 0; st.rden = rden_of(a.N0 * a.S20, ss0); st.rsig = 1.0 / a.sigma2_0;
                 if (!bad) record_row0(a, ch, ss0, st.t);
             }
             __syncthreads();
         }
 
-        int k = seg == 0 ? 1 : seg * a.seglen;      // next step to decide
-        // the step whose isimu = k is the next multiple of adaptint triggers the adaptation (kept as a running value:
-        // an integer division per round is ~40 dependent instructions)
-        int next_adapt = a.adaptint > 0 ? ((k + a.adaptint) / a.adaptint) * a.adaptint : 0x7fffffff;
+        const Slice slice = slice_of(a, seg);
+        const int k_end = slice.k_end;
+        int k = slice.k, next_adapt = slice.next_adapt;   // next step to decide, next adaptation
         int gen_upto = k;                           // increments are ready for steps [k, gen_upto)
         const bool bad0 = st.bad0 != 0;
 #pragma unroll 1
@@ -1998,8 +2074,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                 pr2 = s_cand[lane].pr2; ss2 = s_ssv[2 * lane + 1];
                 if (!o1) {
                     pr1 = s_cand[lane].pr1; ss1 = s_ssv[2 * lane];
-                    x12 = -0.5 * ((ss1 - ss) * is2p + pr1 - pri);
-                    acc1 = x12 >= 0.0 || x12 > scp[5];
+                    acc1 = stage1_accepts(ss1, ss, is2p, pr1, pri, scp[5], x12);
                 }
             }
             const unsigned m1 = __ballot_sync(0xffffffffu, act && acc1);
@@ -2041,13 +2116,13 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                     const double ss_new = accd ? ssn_a : ss;
                     if (accd) {
                         st.ss = ss_new; st.pri = prin_a;
-                        st.t.wcnt = wcnt + max(0, r_acc - max(run_r0, cx.cc.first_row));
-                        if (a.do_cov && r_acc > run_r0) st.ndist = ndist + 1;
+                        st.t.wcnt = wcnt + run_rows(run_r0, r_acc, cx.cc.first_row);
+                        if (run_distinct(a.do_cov, run_r0, r_acc)) st.ndist = ndist + 1;
                         st.run_r0 = r_acc;
                     }
                     // sigma2 of the next step = (N0 S20 + ss_new) / chi2 of the last committed row, kept as its reciprocal (the
                     // same product chi2 * rden the later steps of a round use: the chain does not depend on where rounds are cut)
-                    const double rd = accd ? tc_rcp(a.N0 * a.S20 + ss_new) : rden;
+                    const double rd = accd ? rden_of(a.N0 * a.S20, ss_new) : rden;
                     if (accd) st.rden = rd;
                     if (a.updatesigma) st.rsig = cx.slot_sc(k + ncommit - 1)[2] * rd;
                 }
@@ -2059,7 +2134,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                 if (lane < ncommit) {
                     const int r = k + lane;
                     const double ssr = lane < first ? ss : ss_new;
-                    s2 = a.updatesigma ? (a.N0 * a.S20 + ssr) * tc_rcp(cx.slot_sc(r)[2]) : sig2;
+                    s2 = row_sigma2(a.updatesigma, a.N0 * a.S20, ssr, cx.slot_sc(r)[2], sig2);
                     sq = sqrt(s2);
                     store_row(a, cx.ch, r, s2, so_.fl, ssr);
                 }
@@ -2098,19 +2173,17 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                 const int rr0 = st.run_r0, nd0 = st.ndist;
                 const double wc0 = st.t.wcnt;
                 flush_run(a, cx, rr0, k, wc0, nd0, -1, 0);                     // close the run at the block boundary
-                const int nd = nd0 + ((a.do_cov && k > rr0) ? 1 : 0);
-                const double rate = a.burnin_cumulative ? (double)st.t.rej / k : (double)st.t.reju / a.adaptint;
+                const int nd = nd0 + (run_distinct(a.do_cov, rr0, k) ? 1 : 0);
+                const double rate = adapt_rate(a, st.t.rej, st.t.reju, k);
                 const double cov_n = st.t.cov_n;
                 const bool rdg = st.r_diag != 0;
                 __syncthreads();
                 const int rc = adapt(a, cx, k, cov_n, rate, rdg, nd);
                 if (tid == 0) {
-                    st.t.wcnt = wc0 + max(0, k - max(rr0, cx.cc.first_row));
+                    st.t.wcnt = wc0 + run_rows(rr0, k, cx.cc.first_row);
                     st.run_r0 = k; st.ndist = 0;
-                    if (a.do_cov) st.t.cov_n = k;
-                    if (rc == 1) { st.r_diag = 0; ++st.t.n_adapt; }
-                    else if (rc == 2) ++st.t.n_cholfail;
-                    st.t.reju = 0;
+                    after_adapt(st.t, a.do_cov, k, rc);
+                    if (rc == 1) st.r_diag = 0;
                 }
                 __syncthreads();
                 next_adapt += a.adaptint;
@@ -2125,10 +2198,10 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             const double wc0 = st.t.wcnt;
             flush_run(a, cx, rr0, k, wc0, st.ndist, -1, 0);
             __syncthreads();
-            if (tid == 0) { st.t.wcnt = wc0 + max(0, k - max(rr0, cx.cc.first_row)); st.run_r0 = k; }
+            if (tid == 0) { st.t.wcnt = wc0 + run_rows(rr0, k, cx.cc.first_row); st.run_r0 = k; }
             __syncthreads();
         }
-        if (!last_seg && !bad0) {
+        if (!slice.last && !bad0) {
             // ---- park the chain: the next slice may run on any CTA
 #pragma unroll 1
             for (int i = tid; i < npar; i += DRAM_THREADS) {
@@ -2633,7 +2706,7 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
     ngpus = std::min(ngpus, nchains);
 
     const int Nmax = c->Nmax, npmax = 7 + Nmax;
-    const int ldR = 16 * (((npmax + 3) / 4) * ((npmax + 3) / 4 + 1) / 2);   // proposal factor / scatter matrix in 4x4 tiles (chol_tiled)
+    const int ldR = tri_doubles(npmax);                   // proposal factor / scatter matrix in 4x4 tiles (chol_tiled)
     // does any adaptation with a covariance ever happen?
     bool do_cov = false;
     if (o->adaptint > 0)
@@ -2762,19 +2835,25 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
         CUDA_TRY(r.buf.alloc(a.gState, (size_t)nc * state_doubles(ld)));
         CUDA_TRY(r.buf.alloc(a.cstate, nc));
         CUDA_TRY(cudaMemsetAsync(a.cstate, 0, sizeof(int) * nc, r.st));
+        if (use_warp) a.big = 0;
+        else a.wsz = dram_wsz(Nmax, a.big);
+        const auto kernel = use_warp ? dram_warp_kernel : dram_kernel;
+        const int threads = use_warp ? WK_THREADS : DRAM_THREADS;
+        const size_t smem = use_warp ? smem_w : sizeof(double) * (size_t)dram_smem_doubles(Nmax, a.big);
+        // (big layout: gen_increments_tma keeps at most GENB_MAXT column tiles of 8 per warp in registers)
+        if (!use_warp && (smem > avail || (npmax + 3) / 4 > 255 || (a.big && npmax > 8 * SPEC * GENB_MAXT)))
+            return fail(TC_EINVAL, "max(N) = " + std::to_string(Nmax) + " is too large for the shared-memory layout of this build "
+                                   "(one CTA per chain: the cell, the chain state, 8 proposal slots and 8 forward-model scratch areas must fit in one SM)");
+        CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int per_sm = 0;
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+        if (per_sm < 1) return fail(TC_EINVAL, use_warp ? "chain-per-warp kernel does not fit on this device" : "sampler kernel does not fit on this device");
+        int grid;
         if (use_warp) {
-            a.big = 0;
-            // (more, shorter slices were measured for the one-wave case — 2 392 chains = 150 groups on 148 SMs — and change
-            // nothing: 0.589 s with 29 slices, 0.599 s with 200; what bounds that case is its slowest group, whose slices
-            // are sequential)
-            sl = ((sl + unit - 1) / unit) * unit;
-            a.seglen = (int)std::max<long long>(sl, unit);
-            CUDA_TRY(cudaFuncSetAttribute(dram_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_w));
-            int per_sm = 0;
-            CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, dram_warp_kernel, WK_THREADS, smem_w));
-            if (per_sm < 1) return fail(TC_EINVAL, "chain-per-warp kernel does not fit on this device");
-            // persistent grid, one item = WK_WARPS consecutive chains
-            const int grid = std::max(1, std::min(per_sm * sms, (nc + WK_WARPS - 1) / WK_WARPS));
+            // persistent grid, one item = WK_WARPS consecutive chains.  (More, shorter slices were measured for the one-wave
+            // case — 2 392 chains = 150 groups on 148 SMs — and change nothing: 0.589 s with 29 slices, 0.599 s with 200; what
+            // bounds that case is its slowest group, whose slices are sequential.)
+            grid = std::max(1, std::min(per_sm * sms, (nc + WK_WARPS - 1) / WK_WARPS));
             const size_t nslots = (size_t)grid * WK_WARPS;
             const int ldp = wk_ldp(Nmax);
             CUDA_TRY(r.buf.alloc(a.gPinv, (size_t)nc * ld));
@@ -2786,38 +2865,23 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
                 CUDA_TRY(r.buf.alloc(a.gMb, (size_t)nc * ld));
                 CUDA_TRY(r.buf.alloc(a.gW, nslots * ldR));
             }
-            CUDA_TRY(cudaEventRecord(r.e0, r.st));
-            dram_warp_kernel<<<grid, WK_THREADS, smem_w, r.st>>>(a);
-            CUDA_TRY(cudaGetLastError());
-            CUDA_TRY(cudaEventRecord(r.e1, r.st));
-            continue;
-        }
-        a.wsz = dram_wsz(Nmax, a.big);
-        const size_t smem = sizeof(double) * (size_t)dram_smem_doubles(Nmax, a.big);
-        // (big layout: gen_increments_tma keeps at most GENB_MAXT column tiles of 8 per warp in registers)
-        if (smem > avail || (npmax + 3) / 4 > 255 || (a.big && npmax > 8 * SPEC * GENB_MAXT))
-            return fail(TC_EINVAL, "max(N) = " + std::to_string(Nmax) + " is too large for the shared-memory layout of this build "
-                                   "(one CTA per chain: the cell, the chain state, 8 proposal slots and 8 forward-model scratch areas must fit in one SM)");
-        CUDA_TRY(cudaFuncSetAttribute(dram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        // persistent grid = resident CTA slots
-        int per_sm = 0;
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, dram_kernel, DRAM_THREADS, smem));
-        if (per_sm < 1) return fail(TC_EINVAL, "sampler kernel does not fit on this device");
-        if (nc >= 4 * 296) sl = o->nsimu;                 // many chains per CTA slot: imbalance averages out, no slicing
-        else if (per_sm == 2 && nc > sms) {
-            // about as many chains as CTA slots, two CTAs per SM: lagging chains get an SM to themselves (dram_kernel's claim
-            // loop); finer slices, so that the neighbour of such a chain gives way soon
-            const char *e1 = getenv("TC_SOLO_LAG"), *e2 = getenv("TC_NSEG");          // development switches
-            a.solo_lag = e1 ? atoi(e1) : TC_SOLO_LAG;
-            const int ns = e2 ? atoi(e2) : TC_SOLO_NSEG;
-            if (a.solo_lag > 0) sl = std::max<long long>(((long long)o->nsimu + ns - 1) / ns, 4LL * unit);
+        } else {
+            if (nc >= 4 * 296) sl = o->nsimu;             // many chains per CTA slot: imbalance averages out, no slicing
+            else if (per_sm == 2 && nc > sms) {
+                // about as many chains as CTA slots, two CTAs per SM: lagging chains get an SM to themselves (dram_kernel's
+                // claim loop); finer slices, so that the neighbour of such a chain gives way soon
+                const char *e1 = getenv("TC_SOLO_LAG"), *e2 = getenv("TC_NSEG");          // development switches
+                a.solo_lag = e1 ? atoi(e1) : TC_SOLO_LAG;
+                const int ns = e2 ? atoi(e2) : TC_SOLO_NSEG;
+                if (a.solo_lag > 0) sl = std::max<long long>(((long long)o->nsimu + ns - 1) / ns, 4LL * unit);
+            }
+            grid = std::min(nc, per_sm * sms);             // persistent grid = resident CTA slots: slices may wait on each other
+            if (a.big && do_cov) CUDA_TRY(r.buf.alloc(a.gW, (size_t)grid * ldR));
         }
         sl = ((sl + unit - 1) / unit) * unit;
         a.seglen = (int)std::max<long long>(sl, unit);
-        const int grid = std::min(nc, per_sm * sms);           // every CTA resident: slices may wait on each other
-        if (a.big && do_cov) CUDA_TRY(r.buf.alloc(a.gW, (size_t)grid * ldR));
         CUDA_TRY(cudaEventRecord(r.e0, r.st));
-        dram_kernel<<<grid, DRAM_THREADS, smem, r.st>>>(a);
+        kernel<<<grid, threads, smem, r.st>>>(a);
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaEventRecord(r.e1, r.st));
     }

@@ -206,7 +206,7 @@ __device__ __noinline__ void wk_generate(const RunArgs &a, const WkCtx &c, int g
     const int lane = threadIdx.x & 31, npar = c.npar;
     const int ldz = wk_ldz(c.ld - 7);
     const bool rep = a.replay != 0;
-    if (!r_diag) { const int nt4 = (npar + 3) >> 2; wk_prefetch_l2(c.gR, nt4 * (nt4 + 1) / 2); }    // R: HBM -> L2 while the normals are drawn
+    if (!r_diag) wk_prefetch_l2(c.gR, tri_doubles(npar) / 16);      // R: HBM -> L2 while the normals are drawn
     if (lane < nnew) {
         const int st = g0 + lane;
         double u1, u2, x2;
@@ -395,9 +395,10 @@ __device__ __forceinline__ bool wk_propose2(const WkCtx &c, int ox, int ob, doub
 __device__ __noinline__ void wk_flush(const RunArgs &a, const WkCtx &c, int ox, int r0, int r1, double wcnt, int ndist)
 {
     const int lane = threadIdx.x & 31, npar = c.npar;
-    const int m_c = r1 - r0, rs = max(r0, c.cc.first_row), m_w = r1 - rs;
-    const bool cov = a.do_cov && m_c > 0;
-    const double nn = wcnt + m_w, rnn = m_w > 0 ? tc_rcp(nn) : 0.0, f1 = m_w * rnn, f2 = wcnt * m_w * rnn;     // as flush_run()
+    const int m_c = r1 - r0, rs = max(r0, c.cc.first_row), m_w = run_rows(r0, r1, c.cc.first_row);
+    const bool cov = run_distinct(a.do_cov, r0, r1);
+    double f1, f2;
+    welford_weights(wcnt, m_w, f1, f2);
     double *grow = cov ? c.gRows + (size_t)ndist * c.ld : nullptr;
 #pragma unroll 1
     for (int i = lane; i < npar; i += 32) {
@@ -424,12 +425,10 @@ __device__ __noinline__ void wk_flush(const RunArgs &a, const WkCtx &c, int ox, 
 // M2 += U'U for the covariance block (ndist distinct rows with weights + Chan's mean-shift row), 8 rows at a time: U staged in
 // shared memory, one DMMA pair per 8x8 block of M2 (two blocks interleaved), read-modify-write of M2 in HBM/L2 (4x4-tile layout).
 // mbar (the block mean) sits in shared memory at o_mb.
-__device__ __noinline__ void wk_scatter(const WkCtx &c, int o_mb, int ndist, double cov_n, int m)
+__device__ __noinline__ void wk_scatter(const WkCtx &c, int o_mb, int ndist, int nrows, double fcorr)
 {
     const int lane = threadIdx.x & 31, npar = c.npar, ar = lane >> 2, ak = lane & 3;
     const int nt4 = (npar + 3) >> 2, NT = (npar + 7) >> 3, ldu = wk_ldu(c.ld - 7);
-    const double fcorr = cov_n * m / (cov_n + m);
-    const int nrows = ndist + (cov_n > 0.0 ? 1 : 0);
     const int oU = c.o_ov;
 #pragma unroll 1
     for (int r0 = 0; r0 < nrows; r0 += 8) {
@@ -599,23 +598,24 @@ __device__ __noinline__ bool wk_chol(int nt4, int npar, const double *gA, double
     return ok;
 }
 
-// Adaptation after the step with isimu (a multiple of adaptint), warp-local: see adapt() of dram_kernel for the algebra.
+// Adaptation after the step with isimu (a multiple of adaptint): adapt() of dram_kernel, warp-local, M2 and R in L2.
 // Returns 0: R unchanged / scaled, 1: new full factor, 2: Cholesky failed.  o_mb: a free vector in shared memory (the idle slot).
 __device__ __noinline__ int wk_adapt(const RunArgs &a, const WkCtx &c, int o_mb, int isimu, double cov_n, double rate, bool r_diag, int ndist)
 {
     const int lane = threadIdx.x & 31, npar = c.npar;
-    const int nt4 = (npar + 3) >> 2, T4 = nt4 * (nt4 + 1) / 2;
+    const int nt4 = (npar + 3) >> 2, T4 = tri_doubles(npar) / 16;
     if (a.do_cov) {
-        const int m = isimu - (int)cov_n;                           // rows of the block (adapt())
+        const CovBlock blk = cov_block(isimu, cov_n, ndist);
+        const int m = blk.m;
         wk_prefetch_l2(c.gM2, T4);                                  // the scatter matrix: HBM -> L2
 #pragma unroll 1
         for (int i = lane; i < npar; i += 32) tc_smem[o_mb + i] = __ldcg(c.mb + i) / m;
         __syncwarp();
-        wk_scatter(c, o_mb, ndist, cov_n, m);
+        wk_scatter(c, o_mb, ndist, blk.nrows, blk.fcorr);
 #pragma unroll 1
         for (int i = lane; i < npar; i += 32) {
             const double cm = __ldcg(c.cmean + i), dm = tc_smem[o_mb + i] - cm;
-            __stcg(c.cmean + i, cm + dm * (m / (cov_n + m)));
+            __stcg(c.cmean + i, cm + dm * blk.shift);
             __stcg(c.mb + i, 0.0);
         }
         cov_n += m;
@@ -623,9 +623,7 @@ __device__ __noinline__ int wk_adapt(const RunArgs &a, const WkCtx &c, int o_mb,
     }
     if (lane == 0) { WkState &st = wk_st[threadIdx.x >> 5]; st.t.pc[PH_SCATTER] += clock64() - st.tprev; }    // sub-phase: scatter update
     if (isimu < a.burnintime) {
-        double f = 1.0;
-        if (rate > 0.95) f = 1.0 / a.burnin_scale;
-        else if (rate < 0.05) f = a.burnin_scale;
+        const double f = burnin_factor(rate, a.burnin_scale);
         if (f != 1.0) {
             if (r_diag) {
 #pragma unroll 1
@@ -772,16 +770,14 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 for (int i = lane; i < npar; i += 32) {
                     const size_t g = (size_t)ch * a.ld + i;
                     tc_smem[ox + i] = a.theta0[g];
-                    const double sg = a.psig[g];
-                    a.gPinv[g] = isinf(sg) ? 0.0 : 1.0 / sg;
+                    a.gPinv[g] = prior_inv(a.psig[g]);
                     __stcg(c.rdiag + i, sqrt(a.qcov_diag[g]));
                     __stcg(c.wmean + i, 0.0); __stcg(c.wM2 + i, 0.0);
                     if (a.do_cov) { __stcg(c.cmean + i, 0.0); __stcg(c.mb + i, 0.0); }
                 }
                 if (a.do_cov) {
-                    const int nt4 = (npar + 3) >> 2;
 #pragma unroll 1
-                    for (int i = lane; i < 16 * (nt4 * (nt4 + 1) / 2); i += 32) __stcg(c.gM2 + i, 0.0);
+                    for (int i = lane; i < tri_doubles(npar); i += 32) __stcg(c.gM2 + i, 0.0);
                 }
                 if (lane == 0) {
                     st.t = Tally{};
@@ -833,6 +829,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
 #endif
 #define WK_PHASE(i) do { if (lane == 0) { const long long tn__ = clock64(); st.t.pc[i] += tn__ - st.tprev; st.tprev = tn__; } } while (0)
 
+        // the slice as slice_of() computes it, written out: through slice_of() this kernel spills more
         int k = seg == 0 ? 1 : seg * a.seglen;
         rden = tc_rcp(n0s20 + ss);                                  // (a function of ss alone: recomputed, not parked)
         int next_adapt = a.adaptint > 0 ? ((k + a.adaptint) / a.adaptint) * a.adaptint : 0x7fffffff;
@@ -867,8 +864,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                     ss1 = ss_eval(a.cons, cv, SmemVecA{ob}, w, a.algo, false, nullptr, nullptr);
                     WK_T1(PH_EVAL);
                     nev = 1;
-                    x12 = -0.5 * ((ss1 - ss) * is2 + pr1 - pri);
-                    if (x12 >= 0.0 || x12 > s_logu) acc = 1;
+                    if (stage1_accepts(ss1, ss, is2, pr1, pri, s_logu, x12)) acc = 1;
                 }
                 double ssn = ss1, prin = pr1;
                 if (!acc && a.ntry >= 2) {
@@ -890,14 +886,14 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                     fl |= TC_FL_ACCEPT;
                     const double wcnt = st.t.wcnt;
                     wk_flush(a, c, ox, run_r0, k, wcnt, ndist);          // close the run of the old state at row k
-                    if (lane == 0) st.t.wcnt = wcnt + max(0, k - max(run_r0, c.cc.first_row));
-                    if (a.do_cov && k > run_r0) ++ndist;
+                    if (lane == 0) st.t.wcnt = wcnt + run_rows(run_r0, k, c.cc.first_row);
+                    if (run_distinct(a.do_cov, run_r0, k)) ++ndist;
                     run_r0 = k;
                     const int t_ = ox; ox = ob; ob = t_;                 // the proposal becomes the state
                     ss = ssn; pri = prin;
-                    rden = tc_rcp(n0s20 + ss);
+                    rden = rden_of(n0s20, ss);
                 }
-                const double s2 = a.updatesigma ? (n0s20 + ss) * tc_rcp(s_chi) : sig2;
+                const double s2 = row_sigma2(a.updatesigma, n0s20, ss, s_chi, sig2);
                 if (lane == 0) {
                     tally_s2(st.t, 1.0, s2, sqrt(s2), 0.0);                 // Welford: a batch of one row
                     st.t.n_ss += nev; st.t.n_oob += noob; if (fl & TC_FL_DR) ++st.t.n_dr;
@@ -915,15 +911,13 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                     WK_PHASE(PH_WAIT);
                     const double wc0 = st.t.wcnt, cov_n = st.t.cov_n;
                     wk_flush(a, c, ox, run_r0, k, wc0, ndist);           // close the run at the block boundary
-                    const int nd = ndist + ((a.do_cov && k > run_r0) ? 1 : 0);
-                    const double rate = a.burnin_cumulative ? (double)st.t.rej / k : (double)st.t.reju / a.adaptint;
+                    const int nd = ndist + (run_distinct(a.do_cov, run_r0, k) ? 1 : 0);
+                    const double rate = adapt_rate(a, st.t.rej, st.t.reju, k);
                     __syncwarp();
                     const int rc = wk_adapt(a, c, ob, k, cov_n, rate, r_diag != 0, nd);
                     if (lane == 0) {
-                        st.t.wcnt = wc0 + max(0, k - max(run_r0, c.cc.first_row));
-                        if (a.do_cov) st.t.cov_n = k;
-                        if (rc == 1) ++st.t.n_adapt; else if (rc == 2) ++st.t.n_cholfail;
-                        st.t.reju = 0;
+                        st.t.wcnt = wc0 + run_rows(run_r0, k, c.cc.first_row);
+                        after_adapt(st.t, a.do_cov, k, rc);
                     }
                     if (rc == 1) r_diag = 0;
                     run_r0 = k; ndist = 0;
@@ -939,7 +933,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
         if (!bad0 && run_r0 < k) {
             const double wc0 = st.t.wcnt;
             wk_flush(a, c, ox, run_r0, k, wc0, ndist);
-            if (lane == 0) st.t.wcnt = wc0 + max(0, k - max(run_r0, c.cc.first_row));
+            if (lane == 0) st.t.wcnt = wc0 + run_rows(run_r0, k, c.cc.first_row);
             run_r0 = k;
             __syncwarp();
         }
