@@ -270,3 +270,49 @@ def test_headless_curation_writes_approvedfits_back(tmp_path):
     f2 = str(tmp_path / "19-Oct-2026-X.mat")
     sio.savemat(f2, dict(MCMCresults=mcmc._struct_array(mcmc.RESULT_FIELDS, [rec(7, 1.0), rec(1, 1.0), rec(9, 1.0)]), DatasetName="X"))
     assert curate.ApproveMCMCResults("file", f2, "LoadPrevious", f, "approve", [3]).tolist() == [-1.0, 1.0, 1.0]
+
+
+@pytest.mark.parametrize("width", [0.5, 2.0, 50.0])
+def test_rate_prior_width_reaches_the_sampler(tmp_path, monkeypatch, width):
+    """TranscriptionCycleMCMC(..., 'ratePriorWidth', w) hands the sampler prior_sig = w on every dR and Inf on the seven head
+    parameters, prior_mu = 0 (TranscriptionCycleMCMC.m:242-255), for cells of different lengths in one padded call."""
+    import scipy.io as sio
+    from transcriptioncycleinference_b200 import engine
+    seen = {}
+
+    class FakeCells(engine.Cells):
+        def __init__(self, t, ms2, pp7, construct=None, devices=(0,)):
+            self.ncells = len(t); self.N = np.array([len(x) for x in t], dtype=np.int32)
+            self.off = np.concatenate([[0], np.cumsum(self.N)]); self.t = np.concatenate(t)
+            self.ms2 = np.concatenate(ms2); self.pp7 = np.concatenate(pp7)
+            self.Nmax = int(self.N.max()); self.ld = 7 + self.Nmax
+
+        def close(self):
+            pass
+
+        def mcmc_run(self, opts, chain_cell, theta0, qcov_diag, low, upp, prior_mu, prior_sig, chain_uid=None, **kw):
+            seen.update(cc=np.array(chain_cell), mu=np.array(prior_mu), sig=np.array(prior_sig), N=self.N.copy())
+            n = len(chain_cell)
+            return dict(mean=np.array(theta0), std=np.ones((n, self.ld)), sig=np.ones((n, 2)))
+
+        def forward(self, cell_id, theta, on_raw_grid=True):
+            return np.zeros((len(cell_id), self.Nmax)), np.zeros((len(cell_id), self.Nmax))
+
+    monkeypatch.setattr(mcmc, "Cells", FakeCells)
+    monkeypatch.setattr(mcmc._lib, "device_count", lambda: 1)
+    rng = np.random.default_rng(0)
+    recs = []
+    for n in (5, 9):
+        t = np.arange(n) * 0.5
+        recs.append(dict(time=t, MS2=rng.random(n), PP7=rng.random(n), name="X"))
+    data = np.empty((1, 2), dtype=[("time", object), ("MS2", object), ("PP7", object), ("name", object)])
+    for k, r in enumerate(recs):
+        data[0, k] = (r["time"], r["MS2"], r["PP7"], r["name"])
+    sio.savemat(str(tmp_path / "d.mat"), dict(data=data))
+    mcmc.TranscriptionCycleMCMC("fileDir", str(tmp_path), "saveLoc", str(tmp_path / "out"), "ratePriorWidth", width,
+                                "n_steps", 10, "n_burn", 5, "saveChains", False, "seed", 1, "numChains", 2)
+    assert seen["N"].tolist() == [5, 9] and seen["cc"].tolist() == [0, 0, 1, 1]
+    for i, c in enumerate(seen["cc"]):
+        npar = 7 + int(seen["N"][c])
+        assert np.all(np.isinf(seen["sig"][i, :7])) and np.all(seen["sig"][i, 7:npar] == width), seen["sig"][i]
+        assert np.all(seen["mu"][i, :npar] == 0)

@@ -160,6 +160,8 @@ struct RunArgs {
     unsigned long long seed;
     // chains
     int nchains, ld, ldR, do_cov, wsz, big;
+    int nmax;                                           // max N over the dataset: sizes the chain-per-warp kernel's shared-memory
+                                                        // regions and increment slots (ld may be larger: a caller's padding)
     int blk_rows;                                       // rows of the largest adaptation block: the distinct-row buffer of a chain
     const int *chain_cell;
     const unsigned long long *chain_uid;
@@ -2764,7 +2766,7 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
         a.store_chain = o->store_chain; a.replay = o->replay; a.algo = o->algo; a.qcovadj_always = o->qcovadj_always;
         a.drscale = o->drscale; a.adascale = o->adascale; a.qcovadj = o->qcovadj; a.burnin_scale = o->burnin_scale;
         a.N0 = o->N0; a.S20 = o->S20; a.sigma2_0 = o->sigma2_0; a.seed = o->seed;
-        a.nchains = nc; a.ld = ld; a.ldR = ldR; a.do_cov = do_cov ? 1 : 0;
+        a.nchains = nc; a.ld = ld; a.nmax = Nmax; a.ldR = ldR; a.do_cov = do_cov ? 1 : 0;
         // the first block is rows 0 .. isimu-1 of the first adaptation (row 0 is x0, no step): with adaptint = 1 that is 2 rows
         a.blk_rows = std::max(o->adaptint, 2);
         int *d_cell; unsigned long long *d_uid; double *d;

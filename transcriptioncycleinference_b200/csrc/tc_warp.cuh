@@ -58,7 +58,8 @@ struct WkCtx {
     // bounds / prior in the reference's own structure (TranscriptionCycleMCMC.m:242-255): seven head parameters with their own
     // bounds, then one block (dR) with common bounds and prior.  uni = 1 when this chain's vectors have that structure: the
     // proposals are then checked against these few values instead of four vectors streamed from L2 every step.
-    int uni, pad_;
+    int uni;
+    int nmax;                                                       // max N over the dataset: the layout of the warp's region
     double head[4][8];                                              // lo, hi, mu, 1/sig of parameters 0..7
     double blk[4];                                                  // ... of the block (parameters >= 7)
 };
@@ -125,7 +126,7 @@ template <typename ZT>
 __device__ __forceinline__ void wk_increments(const WkCtx &c, int nnew)
 {
     const int lane = threadIdx.x & 31, npar = c.npar, ar = lane >> 2, ak = lane & 3;
-    const int ldz = wk_ldz(c.ld - 7), rows = sizeof(ZT) == 4 ? WK_GEN : WK_GENR;
+    const int ldz = wk_ldz(c.nmax), rows = sizeof(ZT) == 4 ? WK_GEN : WK_GENR;
     const ZT *Z1 = reinterpret_cast<const ZT *>(tc_smem + c.o_ov), *Z2 = Z1 + rows * ldz;
     const int NT = (npar + 7) >> 3, nt4 = (npar + 3) >> 2, inner = 4 * ak + (ar & 3);
     const bool rowok = ar < nnew;
@@ -204,7 +205,7 @@ __device__ __forceinline__ void wk_prefetch_l2(const double *p, int nlines)     
 __device__ __noinline__ void wk_generate(const RunArgs &a, const WkCtx &c, int g0, int nnew, bool r_diag)
 {
     const int lane = threadIdx.x & 31, npar = c.npar;
-    const int ldz = wk_ldz(c.ld - 7);
+    const int ldz = wk_ldz(c.nmax);
     const bool rep = a.replay != 0;
     if (!r_diag) wk_prefetch_l2(c.gR, tri_doubles(npar) / 16);      // R: HBM -> L2 while the normals are drawn
     if (lane < nnew) {
@@ -428,7 +429,7 @@ __device__ __noinline__ void wk_flush(const RunArgs &a, const WkCtx &c, int ox, 
 __device__ __noinline__ void wk_scatter(const WkCtx &c, int o_mb, int ndist, int nrows, double fcorr)
 {
     const int lane = threadIdx.x & 31, npar = c.npar, ar = lane >> 2, ak = lane & 3;
-    const int nt4 = (npar + 3) >> 2, NT = (npar + 7) >> 3, ldu = wk_ldu(c.ld - 7);
+    const int nt4 = (npar + 3) >> 2, NT = (npar + 7) >> 3, ldu = wk_ldu(c.nmax);
     const int oU = c.o_ov;
 #pragma unroll 1
     for (int r0 = 0; r0 < nrows; r0 += 8) {
@@ -672,7 +673,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
     const int slot = blockIdx.x * WK_WARPS + warp;
     const int nseg = (a.nsimu + a.seglen - 1) / a.seglen;
     const int ngroups = (a.nchains + WK_WARPS - 1) / WK_WARPS;
-    const int regsz = wk_region(a.ld - 7), ldp = wk_ldp(a.ld - 7);
+    const int regsz = wk_region(a.nmax), ldp = wk_ldp(a.nmax);     // as the host sized them (tc_mcmc_run)
     const int o_reg = warp * regsz;
     WkCtx &c = wk_cx[warp];
     WkState &st = wk_st[warp];
@@ -741,8 +742,8 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
             N = a.cells.N[cid]; npar = 7 + N;
             gst = a.gState + (size_t)ch * state_doubles(a.ld);
             if (lane == 0) {
-                c.N = N; c.npar = npar; c.ld = a.ld; c.ldp = ldp; c.ch = ch;
-                c.o_s0 = o_reg + 1; c.o_ov = o_reg + 2 * ldp + 2; c.o_work = c.o_ov + wk_cell_sz(a.ld - 7);
+                c.N = N; c.npar = npar; c.ld = a.ld; c.nmax = a.nmax; c.ldp = ldp; c.ch = ch;
+                c.o_s0 = o_reg + 1; c.o_ov = o_reg + 2 * ldp + 2; c.o_work = c.o_ov + wk_cell_sz(a.nmax);
                 c.cc = chain_consts(a, ch, N);
                 c.lo = a.low + (size_t)ch * a.ld; c.hi = a.upp + (size_t)ch * a.ld; c.mu = a.pmu + (size_t)ch * a.ld;
                 c.pinv = a.gPinv + (size_t)ch * a.ld;
