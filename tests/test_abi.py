@@ -42,11 +42,12 @@ def test_version_and_defaults():
 
 
 def test_struct_layouts_match_header(tmp_path):
-    """sizeof/offsetof from a C compile of the header == the ctypes mirror."""
+    """sizeof/offsetof and the TC_EINVAL / TC_LAYOUT_* values from a C compile of the header == the ctypes mirror."""
     src = tmp_path / "sz.c"
     src.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "tcmcmc.h"\nint main(){printf("%zu %zu %zu %zu %zu %zu %zu %d\\n",'
                    'sizeof(tc_construct),sizeof(tc_mcmc_opts),sizeof(tc_replay),sizeof(tc_device_info),'
-                   'offsetof(tc_mcmc_opts,drscale),offsetof(tc_mcmc_opts,seed),offsetof(tc_construct,pp7_loopn),TC_NCOUNTERS);return 0;}\n')
+                   'offsetof(tc_mcmc_opts,drscale),offsetof(tc_mcmc_opts,seed),offsetof(tc_construct,pp7_loopn),TC_NCOUNTERS);'
+                   'printf("%d %d %d %d %d\\n",TC_EINVAL,TC_LAYOUT_AUTO,TC_LAYOUT_BIG,TC_LAYOUT_WARP,TC_LAYOUT_CTA);return 0;}\n')
     exe = tmp_path / "sz"
     subprocess.check_call(["/usr/bin/gcc" if os.path.exists("/usr/bin/gcc") else "gcc", "-I", os.path.join(ROOT, "include"),
                            "-o", str(exe), str(src)])
@@ -58,6 +59,7 @@ def test_struct_layouts_match_header(tmp_path):
     assert vals[4] == _lib.McmcOpts.drscale.offset and vals[5] == _lib.McmcOpts.seed.offset
     assert vals[6] == _lib.Construct.pp7_loopn.offset
     assert vals[7] == _lib.NCOUNTERS
+    assert vals[8:] == [_lib.TC_EINVAL, _lib.LAYOUT_AUTO, _lib.LAYOUT_BIG, _lib.LAYOUT_WARP, _lib.LAYOUT_CTA]
 
 
 def test_no_cpu_fallback_without_device(cells_npz):

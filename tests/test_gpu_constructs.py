@@ -4,15 +4,15 @@ import numpy as np
 import pytest
 
 from conftest import random_theta
+from parity import check_chain, make_cells, need_gpu, oracle_chains, replay_streams, series
 
 pytestmark = pytest.mark.gpu
 
 
 def test_two_set_construct_ss_and_forward(cells_npz, orc):
-    from transcriptioncycleinference_b200 import _lib, register_construct
+    from transcriptioncycleinference_b200 import register_construct
     from transcriptioncycleinference_b200.engine import Cells
-    if _lib.device_count() < 1:
-        pytest.skip("no CUDA device")
+    need_gpu()
     co, _ = orc
     d = dict(L_MS2=6.0, L_PP7=6.3, MS2_start=[0.024, 2.0], MS2_end=[1.299, 2.6], MS2_loopn=[24.0, 12.0],
              PP7_start=[4.292, 5.8], PP7_end=[5.758, 6.0], PP7_loopn=[24.0, 6.0])
@@ -49,10 +49,9 @@ def test_two_set_construct_ss_and_forward(cells_npz, orc):
 
 def test_truncated_window_cells(cells_npz, orc):
     """t_start / t_end windows: shorter series, t(1) != 0, their own t_interp."""
-    from transcriptioncycleinference_b200 import _lib, setup_cell
+    from transcriptioncycleinference_b200 import setup_cell
     from transcriptioncycleinference_b200.engine import Cells
-    if _lib.device_count() < 1:
-        pytest.skip("no CUDA device")
+    need_gpu()
     co, cons = orc
     ts, m2s, p7s = [], [], []
     for c in range(0, 299, 15):
@@ -84,47 +83,30 @@ def test_series_length_extremes_replay(orc, N):
     N = 400 (BASELINE config 5's length; npar = 257 / 407: the big layout — ring of 8 slots, bounds read from HBM/L2, proposal
     factor factorised through HBM/L2 by chol_global; 257 has an odd number of 4x4 tile rows), and N = 441, the longest series
     the engine takes (npar = 448: seven column tiles of 8 per warp in gen_increments_tma).  Synthetic irregular time
-    grid with missing data; the DRAM replay must match the oracle flag for flag."""
-    from transcriptioncycleinference_b200 import _lib, setup_cell
-    from transcriptioncycleinference_b200.engine import Cells
-    if _lib.device_count() < 1:
-        pytest.skip("no CUDA device")
-    co, cons = orc
+    grid with missing data; the DRAM replay must match the oracle: flags, rows, s2chain, sschain and every counter."""
+    from transcriptioncycleinference_b200 import setup_cell
+    _lib = need_gpu()
+    co, _ = orc
     rng = np.random.default_rng(100 + N)
-    ts, m2s, p7s = [], [], []
-    for c in range(3):
-        t = np.concatenate([[0.0], np.cumsum(rng.uniform(0.15, 0.35, N - 1))])
-        m2 = rng.uniform(0, 3, N); p7 = rng.uniform(0, 10, N)
-        m2[rng.random(N) < 0.4] = np.nan; p7[rng.random(N) < 0.2] = np.nan
-        ts.append(t); m2s.append(m2); p7s.append(p7)
-    cells = Cells(ts, m2s, p7s)
-    packed = dict(N=cells.N, off=cells.off, t=cells.t, ms2=cells.ms2, pp7=cells.pp7)
+    cells, packed = make_cells(co, [series(co, rng, N) for _ in range(3)])
     cc = np.arange(3, dtype=np.int32)
     inputs = setup_cell.chain_inputs(cells, cc, np.random.default_rng(7))
     nsimu, burn = 330, 100
-    g = np.random.default_rng(8)
-    st = dict(z1=g.standard_normal((3, nsimu, cells.ld)), u1=g.random((3, nsimu)), z2=g.standard_normal((3, nsimu, cells.ld)),
-              u2=g.random((3, nsimu)), chi2=g.chisquare(1 + 2 * N, (3, nsimu)))
+    st = replay_streams(cells.N[cc], nsimu, cells.ld, 8)
     opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, replay=1, qcovadj_always=1)   # singular covariances: see test_gpu_mcmc.py
     out = cells.mcmc_run(opts, cc, *inputs, replay=st, want_flags=True)
-    npar = 7 + N
-    for i in range(3):
-        o = int(cells.off[i])
-        sti = dict(z1=st["z1"][i][:, :npar], u1=st["u1"][i], z2=st["z2"][i][:, :npar], u2=st["u2"][i], chi2=st["chi2"][i])
-        ref = co.dram(cons, packed["t"][o:o + N], packed["ms2"][o:o + N], packed["pp7"][o:o + N], co.default_opts(nsimu, burn, qcovadj_always=1),
-                      *[x[i, :npar] for x in inputs], streams=sti)
-        assert np.array_equal(out["flags"][i], ref["flags"]), (N, i)
-        np.testing.assert_allclose(out["chain"][i][:, :npar], ref["chain"], rtol=0, atol=1e-7)
+    refs = oracle_chains(orc, packed, cc, co.default_opts(nsimu, burn, qcovadj_always=1), inputs, st)
+    for i, ref in enumerate(refs):
+        check_chain("N=%d" % N, out, i, ref, 7 + N)
     cells.close()
 
 
 def test_series_longer_than_the_limit_are_rejected():
     """max(N) = 442 does not fit the one-CTA-per-chain layouts (include/tcmcmc.h): tc_mcmc_run returns TC_EINVAL, it does not
     run a kernel that would silently drop column tiles."""
-    from transcriptioncycleinference_b200 import _lib, setup_cell
+    from transcriptioncycleinference_b200 import setup_cell
     from transcriptioncycleinference_b200.engine import Cells
-    if _lib.device_count() < 1:
-        pytest.skip("no CUDA device")
+    _lib = need_gpu()
     N = 442
     rng = np.random.default_rng(5)
     t = np.concatenate([[0.0], np.cumsum(rng.uniform(0.15, 0.35, N - 1))])
@@ -142,9 +124,8 @@ def test_synthetic_config5_workload_big_layout():
     Philox run on the big layout.  Checks what does not depend on how well the reference's sampler mixes: every adaptation
     factorised (no Cholesky failure), the fit explains the data better than the start (posterior sigma below the initial
     one), chains independent of how they are batched (bit-identical), summaries inside the bounds."""
-    from transcriptioncycleinference_b200 import _lib, setup_cell, synthetic
-    if _lib.device_count() < 1:
-        pytest.skip("no CUDA device")
+    from transcriptioncycleinference_b200 import setup_cell, synthetic
+    _lib = need_gpu()
     cells, truth = synthetic.make_cells(12, 400)
     assert cells.Nmax == 400 and truth.shape == (12, 407)
     assert 0.35 < np.isnan(cells.ms2).mean() < 0.65 and 0.1 < np.isnan(cells.pp7).mean() < 0.3

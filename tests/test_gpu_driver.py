@@ -7,6 +7,8 @@ import numpy as np
 import pytest
 import scipy.io as sio
 
+from parity import need_gpu
+
 pytestmark = pytest.mark.gpu
 
 
@@ -26,9 +28,8 @@ def _write_dataset(path, cells_npz, idx, name="TestData"):
 
 
 def test_driver_outputs_reference_layout(tmp_path, cells_npz, orc):
-    from transcriptioncycleinference_b200 import _lib, mcmc
-    if _lib.device_count() < 1:
-        pytest.skip("no CUDA device")
+    from transcriptioncycleinference_b200 import mcmc
+    need_gpu()
     co, cons = orc
     idx = [0, 9, 100, 250, 298]
     d = tmp_path / "in"; s = tmp_path / "out"; d.mkdir()
@@ -62,9 +63,8 @@ def test_driver_outputs_reference_layout(tmp_path, cells_npz, orc):
 
 
 def test_load_previous_and_custom_construct(tmp_path, cells_npz):
-    from transcriptioncycleinference_b200 import _lib, mcmc, register_construct
-    if _lib.device_count() < 1:
-        pytest.skip("no CUDA device")
+    from transcriptioncycleinference_b200 import mcmc, register_construct
+    need_gpu()
     idx = [3, 4, 5, 6]
     d = tmp_path / "in"; s1 = tmp_path / "o1"; s2 = tmp_path / "o2"; d.mkdir()
     _write_dataset(str(d / "TestData.mat"), cells_npz, idx)
@@ -93,9 +93,8 @@ def test_multiple_chains_per_cell_pool_and_diagnose(tmp_path, cells_npz):
     """'numChains' > 1 (BASELINE config 3 through the drop-in driver): the chains of a cell are pooled into the
     reference's MCMCresults layout (pooled mean / population std = those of the concatenated chains) and the extra
     variable MCMCdiagnostics carries Rhat / n_eff per parameter."""
-    from transcriptioncycleinference_b200 import _lib, mcmc
-    if _lib.device_count() < 1:
-        pytest.skip("no CUDA device")
+    from transcriptioncycleinference_b200 import mcmc
+    need_gpu()
     idx = [3, 77, 200]
     d = tmp_path / "in"; s = tmp_path / "out"; d.mkdir()
     _write_dataset(str(d / "TestData.mat"), cells_npz, idx)

@@ -15,56 +15,19 @@ C oracle (oracle/tc_oracle.c: the literal m x n restatement, sequential, bit-exa
 
 The ABI does not report which layout ran: at N = 213 a replay under TC_LAYOUT_CTA passes whether the regular layout or
 (had it stopped fitting) the big one ran."""
-import concurrent.futures as cf
-
 import numpy as np
 import pytest
 
 from conftest import random_theta
+from parity import DTS, check_chain, check_recorded_ss, cols, make_cells, need_gpu, oracle_chains, replay_streams, series
 from test_counter_ties import COUNT_CONS, adversarial_cases, control_cases, count_theta, oracle_floors
+from transcriptioncycleinference_b200 import _lib
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-10
 LENGTHS = list(range(3, 13)) + [31, 32, 33, 127, 128, 129, 130, 141, 142, 144, 145, 152, 153, 200, 211, 212, 213, 214,
                                 255, 256, 257, 384, 400, 441]
 STREAM_MAX_N = 152            # ss_stream_kernel: two CTAs of 8 warps per SM at max N <= 152 (launch_ss)
-DTS = (0.1, 1.0 / 3.0, 0.3, 0.7)
-
-
-def _gpu():
-    from transcriptioncycleinference_b200 import _lib
-    if _lib.device_count() < 1:
-        pytest.skip("no CUDA device")
-    return _lib
-
-
-def _grid_ok(co, t):
-    try:
-        co.t_interp(t)
-        return True
-    except ValueError:
-        return False
-
-
-def series(co, rng, N, dt=None):
-    """One cell: the irregular grid + NaN mask of test_series_length_extremes_replay, or the regular grid t = k dt (the first
-    of DTS, starting at `dt`, whose t(1):dt:t(end) has N points).  Irregular grids are redrawn until that holds."""
-    if dt is None:
-        while True:
-            t = np.concatenate([[0.0], np.cumsum(rng.uniform(0.15, 0.35, N - 1))])
-            if _grid_ok(co, t):
-                break
-    else:
-        k = DTS.index(dt)
-        for d in DTS[k:] + DTS[:k]:
-            t = np.arange(N) * d
-            if _grid_ok(co, t):
-                break
-        else:
-            raise AssertionError("no regular grid of %d points" % N)
-    m2 = rng.uniform(0, 3, N); p7 = rng.uniform(0, 10, N)
-    m2[rng.random(N) < 0.4] = np.nan; p7[rng.random(N) < 0.2] = np.nan
-    return t, m2, p7
 
 
 def model_cell(co, cons, rng, N):
@@ -74,16 +37,6 @@ def model_cell(co, cons, rng, N):
     tg = co.t_interp(t)
     a, b = co.model_on_grid(cons, thstar, tg)
     return (t, np.where(np.isnan(m2), np.nan, np.interp(t, tg, a)), np.where(np.isnan(p7), np.nan, np.interp(t, tg, b))), thstar
-
-
-def make_cells(co, cols, construct=None):
-    """Cells from (t, ms2, pp7) triples; t_interp of every cell must be the oracle's, bit for bit."""
-    from transcriptioncycleinference_b200.engine import Cells
-    kw = {} if construct is None else dict(construct=construct)
-    cells = Cells([c[0] for c in cols], [c[1] for c in cols], [c[2] for c in cols], **kw)
-    for c, col in enumerate(cols):
-        assert np.array_equal(cells.t_interp(c), co.t_interp(col[0])), c
-    return cells, dict(N=cells.N, off=cells.off, t=cells.t, ms2=cells.ms2, pp7=cells.pp7)
 
 
 def theta_rows(rng, cells, n):
@@ -120,7 +73,7 @@ def _check_ss(tag, got, ref, nrows_cap=60000):
 @pytest.fixture(scope="module")
 def length_sets(orc):
     """N -> (cells, packed, theta*): per length one dataset of 3 cells — irregular grid, regular grid, and the model cell."""
-    _gpu()
+    need_gpu()
     co, cons = orc
     out = {}
     for N in LENGTHS:
@@ -192,7 +145,7 @@ def test_stream_vs_batch_kernel_on_the_same_cells(orc):
     both against the oracle; the Toeplitz SS of ss_stream_kernel, ss_batch_kernel and tc_ss_batch_device (torch device buffers)
     agree to 1e-14 (the same ss_eval on the same operands: a staging or permutation bug would be O(1)); theta with a padded
     leading dimension (7 + max N, +1, +8: ss_stream_kernel rounds it up and may stop fitting) gives identical results."""
-    _gpu()
+    need_gpu()
     co, cons = orc
     (ca, pa), (cb, pb) = _short_plus(co, 152), _short_plus(co, 153)
     rng = np.random.default_rng(11)
@@ -223,7 +176,7 @@ def test_stream_vs_batch_kernel_on_the_same_cells(orc):
 
 def test_config5_generator_is_the_oracle_model(orc):
     """synthetic.make_cells(k, 400, noise=0): MS2 / PP7 = the oracle's model at the truth on t_interp, interpolated to t."""
-    _gpu()
+    need_gpu()
     from transcriptioncycleinference_b200 import synthetic
     co, cons = orc
     cells, truth = synthetic.make_cells(4, 400, noise=0.0)
@@ -255,7 +208,7 @@ MULTI_SETS = {
 def test_multi_set_constructs(orc, name, lengths):
     """3- and 8-set constructs (the per-set basal clamp sits inside the loop over sets): SS of both algorithms and the curves
     on both grids against the oracle."""
-    _gpu()
+    need_gpu()
     from transcriptioncycleinference_b200 import register_construct
     co, _ = orc
     d = MULTI_SETS[name]
@@ -284,7 +237,7 @@ def test_counter_ties_against_the_oracle(orc):
     dataset, max N = 400: ss_batch_kernel; the N <= 129 cases alone: ss_stream_kernel) at 1e-10, the curves on t_interp at
     1e-10 / 1e-12 (a wrong floor moves a whole polymerase), and, under a construct whose curves are the loading counts, the
     counts themselves equal to the oracle's floors."""
-    _gpu()
+    need_gpu()
     from transcriptioncycleinference_b200 import register_construct
     co, cons = orc
     cases = list(adversarial_cases()) + list(control_cases())
@@ -329,16 +282,17 @@ def test_counter_ties_against_the_oracle(orc):
 
 # ------------------------------------------------------------------------------------------------ sampler replays
 NSIMU, BURN = 330, 100          # burn-in, the first covariance adaptation and two more
-AUTO, BIG, WARP, CTA = 0, 1, 2, 3
+AUTO, BIG, WARP, CTA = _lib.LAYOUT_AUTO, _lib.LAYOUT_BIG, _lib.LAYOUT_WARP, _lib.LAYOUT_CTA
 SMALL = tuple(range(3, 13))
 
 
 def replay(orc, cols, layout, nch=None, ld_pad=0, seed=0):
-    """Replay nch chains (chain i on cell i % ncells) with injected randomness and qcovadj_always = 1 against the oracle, flag
-    for flag; the SS the sampler recorded for every stored row must be tc_ss_batch's SS of that row (1e-14 relative)."""
-    _lib = _gpu()
+    """Replay nch chains (chain i on cell i % ncells) with injected randomness and qcovadj_always = 1 against the oracle: flags,
+    rows, s2chain, sschain and every counter; the SS the sampler recorded for every stored row must be tc_ss_batch's SS of
+    that row (1e-14 relative)."""
+    need_gpu()
     from transcriptioncycleinference_b200 import setup_cell
-    co, cons = orc
+    co, _ = orc
     cells, packed = make_cells(co, cols)
     nch = nch or cells.ncells
     cc = (np.arange(nch) % cells.ncells).astype(np.int32)
@@ -347,41 +301,16 @@ def replay(orc, cols, layout, nch=None, ld_pad=0, seed=0):
     if ld_pad:
         fill = (0.0, 1.0, 0.0, 0.0, 0.0, np.inf)                  # chain_inputs' own padding
         ins = tuple(np.concatenate([x, np.full((nch, ld_pad), f)], axis=1) for x, f in zip(ins, fill))
-    g = np.random.default_rng(seed + 1)
-    Ns = cells.N[cc]
-    st = dict(z1=g.standard_normal((nch, NSIMU, ld)), u1=g.random((nch, NSIMU)), z2=g.standard_normal((nch, NSIMU, ld)),
-              u2=g.random((nch, NSIMU)), chi2=np.stack([g.chisquare(1 + 2 * int(N), NSIMU) for N in Ns]))
+    st = replay_streams(cells.N[cc], NSIMU, ld, seed + 1)
     opts = _lib.default_opts(nsimu=NSIMU, burnintime=BURN, n_burn=1, store_chain=1, replay=1, layout=layout, qcovadj_always=1)
     out = cells.mcmc_run(opts, cc, *ins, replay=st, want_flags=True)
-
-    def oracle(i):
-        c = int(cc[i]); N = int(cells.N[c]); o = int(cells.off[c]); npar = 7 + N
-        sti = dict(z1=st["z1"][i][:, :npar], u1=st["u1"][i], z2=st["z2"][i][:, :npar], u2=st["u2"][i], chi2=st["chi2"][i])
-        return co.dram(cons, packed["t"][o:o + N], packed["ms2"][o:o + N], packed["pp7"][o:o + N],
-                       co.default_opts(NSIMU, BURN, qcovadj_always=1), *[x[i, :npar] for x in ins], streams=sti)
-
-    with cf.ThreadPoolExecutor() as ex:                            # the oracle releases the GIL
-        refs = list(ex.map(oracle, range(nch)))
+    refs = oracle_chains(orc, packed, cc, co.default_opts(NSIMU, BURN, qcovadj_always=1), ins, st)
     for i, ref in enumerate(refs):
-        npar = 7 + int(Ns[i])
-        assert np.array_equal(out["flags"][i], ref["flags"]), ("flags", i, int(Ns[i]), int(np.argmax(out["flags"][i] != ref["flags"])))
-        np.testing.assert_allclose(out["chain"][i][:, :npar], ref["chain"], rtol=0, atol=1e-7)
-        np.testing.assert_allclose(out["s2chain"][i], ref["s2chain"], rtol=1e-9)
+        check_chain("layout %d N=%d" % (layout, cells.N[cc[i]]), out, i, ref, 7 + int(cells.N[cc[i]]))
         cnt = out["counters"][i]
-        for k in (_lib.CNT_SS_EVALS, _lib.CNT_ACC_STAGE1, _lib.CNT_ACC_STAGE2, _lib.CNT_ADAPTATIONS):
-            assert cnt[k] == ref["counters"][k], (i, k, cnt[k], ref["counters"][k])
         assert cnt[_lib.CNT_ADAPTATIONS] == 3 and cnt[_lib.CNT_CHOL_FAIL] == 0
-    rows = out["chain"].reshape(-1, ld)
-    ss = cells.ss_batch(np.repeat(cc, NSIMU), rows)
-    rel = np.abs(ss - out["sschain"].reshape(-1)) / np.abs(out["sschain"].reshape(-1))
-    assert rel.max() <= 1e-14, rel.max()
+    check_recorded_ss(cells, cc, out, ld)
     cells.close()
-
-
-def _cols(orc, lengths, seed):
-    co, _ = orc
-    rng = np.random.default_rng(seed)
-    return [series(co, rng, N, DTS[k % 4] if k % 2 else None) for k, N in enumerate(lengths)]
 
 
 REPLAYS = ([("cta", (N, N), CTA) for N in SMALL + (141, 142, 211, 212, 213)] +
@@ -396,28 +325,28 @@ REPLAYS = ([("cta", (N, N), CTA) for N in SMALL + (141, 142, 211, 212, 213)] +
 def test_replay_at_layout_edges(orc, name, lengths, layout):
     """Each dataset holds these cells (a single length: two cells, one irregular and one regular grid); short chains in a
     mixed dataset run in a layout sized by the longest one."""
-    replay(orc, _cols(orc, lengths, sum(lengths) + layout), layout)
+    replay(orc, cols(orc, lengths, sum(lengths) + layout), layout)
 
 
 def test_replay_warp_mixed_lengths_ragged_groups(orc):
     """Chain-per-warp layout, 20 chains over cells of N = 3, 12, 61, 129, 144: the first 16-chain group mixes lengths, a ragged
     group of 4 follows."""
-    replay(orc, _cols(orc, (3, 12, 61, 129, 144), 5), WARP, nch=20)
+    replay(orc, cols(orc, (3, 12, 61, 129, 144), 5), WARP, nch=20)
 
 
 def test_replay_padded_leading_dimension(orc):
     """ld = 7 + max N + 1 for every array of the run (theta0, bounds, priors, streams, chain)."""
-    replay(orc, _cols(orc, (5, 129, 141), 9), CTA, ld_pad=1)
+    replay(orc, cols(orc, (5, 129, 141), 9), CTA, ld_pad=1)
 
 
 @pytest.mark.parametrize("N", range(145, 151))
 def test_warp_layout_limit(orc, N):
     """Past N = 144 (DESIGN 3: the chain-per-warp layout's promise) a length either runs and replays, or is refused with
     TC_EINVAL "too large for the chain-per-warp layout" — never a kernel that does not fit."""
-    _lib = _gpu()
+    need_gpu()
     try:
-        replay(orc, _cols(orc, (N, N), N), WARP)
+        replay(orc, cols(orc, (N, N), N), WARP)
         print("chain-per-warp layout at N = %d: runs and replays" % N)
     except _lib.TcError as e:
-        assert e.code == -1 and "too large for the chain-per-warp layout" in str(e), str(e)
+        assert e.code == _lib.TC_EINVAL and "too large for the chain-per-warp layout" in str(e), str(e)
         print("chain-per-warp layout at N = %d: refused (TC_EINVAL)" % N)

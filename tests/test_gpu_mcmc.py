@@ -13,6 +13,9 @@ qcovadj_always = 1 (always factor cov + qcovadj I) on both sides.  The default p
 import numpy as np
 import pytest
 
+from parity import LAYOUTS, check_chain, dumped_streams, oracle_chains, raw_run, replay_streams
+from transcriptioncycleinference_b200 import _lib
+
 pytestmark = pytest.mark.gpu
 SHORT = dict(qcovadj_always=1)
 
@@ -23,53 +26,24 @@ def _setup(gpu_cells, chain_cell, seed):
     return setup_cell.chain_inputs(gpu_cells, chain_cell, rng)
 
 
-def _streams(nch, nsimu, ld, N_of_chain, seed):
-    g = np.random.default_rng(seed)
-    st = dict(z1=g.standard_normal((nch, nsimu, ld)), u1=g.random((nch, nsimu)),
-              z2=g.standard_normal((nch, nsimu, ld)), u2=g.random((nch, nsimu)),
-              chi2=np.zeros((nch, nsimu)))
-    for i, N in enumerate(N_of_chain):
-        st["chi2"][i] = g.chisquare(1 + 2 * N, nsimu)
-    return st
-
-
-def _oracle_chain(orc, cells_npz, c, opts_kw, inputs, i, streams=None):
-    co, cons = orc
-    N = int(cells_npz["N"][c]); o = int(cells_npz["off"][c]); npar = 7 + N
-    t, ms2, pp7 = (cells_npz[k][o:o + N] for k in ("t", "ms2", "pp7"))
-    th0, q, lo, hi, mu, sg = (x[i, :npar] for x in inputs)
-    st = None
-    if streams is not None:
-        st = dict(z1=streams["z1"][i][:, :npar], u1=streams["u1"][i], z2=streams["z2"][i][:, :npar],
-                  u2=streams["u2"][i], chi2=streams["chi2"][i])
-    opts = co.default_opts(opts_kw["nsimu"], opts_kw["burnintime"], **opts_kw.get("extra", SHORT))
-    return co.dram(cons, t, ms2, pp7, opts, th0, q, lo, hi, mu, sg, streams=st)
-
-
-@pytest.mark.parametrize("algo,layout", [(1, 0), (0, 0), (1, 2), (0, 2)])
+@pytest.mark.parametrize("algo,layout", [(_lib.ALGO_TOEPLITZ, _lib.LAYOUT_AUTO), (_lib.ALGO_PAIRS, _lib.LAYOUT_AUTO),
+                                         (_lib.ALGO_TOEPLITZ, _lib.LAYOUT_WARP), (_lib.ALGO_PAIRS, _lib.LAYOUT_WARP)])
 def test_replay_accept_reject_identical(gpu_cells, cells_npz, orc, algo, layout):
     """600 steps with burn-in 300: covers burn-in, the first covariance adaptation (Cholesky of
-    the 300-row covariance) and three later ones.  layout 0: one CTA per chain (dram_kernel), 2: one warp per chain
-    (dram_warp_kernel)."""
-    from transcriptioncycleinference_b200 import _lib
+    the 300-row covariance) and three later ones.  TC_LAYOUT_AUTO: one CTA per chain (dram_kernel), TC_LAYOUT_WARP: one warp
+    per chain (dram_warp_kernel)."""
+    co, _ = orc
     chain_cell = np.array([0, 5, 77, 150, 298, 42], dtype=np.int32)
     nsimu, burn = 600, 300
     inputs = _setup(gpu_cells, chain_cell, 11)
-    st = _streams(len(chain_cell), nsimu, gpu_cells.ld, cells_npz["N"][chain_cell], 12)
+    st = replay_streams(cells_npz["N"][chain_cell], nsimu, gpu_cells.ld, 12)
     opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, replay=1, algo=algo, layout=layout, **SHORT)
     out = gpu_cells.mcmc_run(opts, chain_cell, *inputs, replay=st, want_flags=True)
-    for i, c in enumerate(chain_cell):
-        ref = _oracle_chain(orc, cells_npz, int(c), dict(nsimu=nsimu, burnintime=burn), inputs, i, st)
-        npar = 7 + int(cells_npz["N"][c])
-        assert np.array_equal(out["flags"][i], ref["flags"]), "accept/reject sequence differs (chain %d)" % i
-        np.testing.assert_allclose(out["sschain"][i], ref["sschain"], rtol=1e-9)
-        np.testing.assert_allclose(out["chain"][i][:, :npar], ref["chain"], rtol=0, atol=1e-7)
-        np.testing.assert_allclose(out["s2chain"][i], ref["s2chain"], rtol=1e-9)
-        cnt = out["counters"][i]
-        assert cnt[_lib.CNT_SS_EVALS] == ref["counters"][0]
-        assert cnt[_lib.CNT_ACC_STAGE1] == ref["counters"][1]
-        assert cnt[_lib.CNT_ACC_STAGE2] == ref["counters"][2]
-        assert cnt[_lib.CNT_ADAPTATIONS] == ref["counters"][4] == 4
+    refs = oracle_chains(orc, cells_npz, chain_cell, co.default_opts(nsimu, burn, **SHORT), inputs, st)
+    for i, ref in enumerate(refs):
+        npar = 7 + int(cells_npz["N"][chain_cell[i]])
+        check_chain("algo %d layout %d" % (algo, layout), out, i, ref, npar)
+        assert out["counters"][i][_lib.CNT_ADAPTATIONS] == 4
         # summaries = mean / population std of the stored rows (TranscriptionCycleMCMC.m:286-303)
         np.testing.assert_allclose(out["mean"][i][:npar], ref["chain"].mean(axis=0), rtol=1e-9, atol=1e-9)
         np.testing.assert_allclose(out["std"][i][:npar], ref["chain"].std(axis=0), rtol=1e-6, atol=1e-9)
@@ -80,33 +54,28 @@ def test_replay_accept_reject_identical(gpu_cells, cells_npz, orc, algo, layout)
 def test_production_rng_equals_replay_of_its_own_dump(gpu_cells, cells_npz, orc):
     """Philox path: dump the device's streams for (seed, uid), feed them to the ORACLE, compare with
     the production (non-replay) run."""
-    from transcriptioncycleinference_b200 import _lib
+    co, _ = orc
     chain_cell = np.array([3, 200], dtype=np.int32)
     uid = np.array([1000003, 77], dtype=np.uint64)
     nsimu, burn, seed = 400, 200, 987654321
     inputs = _setup(gpu_cells, chain_cell, 21)
     opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, seed=seed, **SHORT)
     out = gpu_cells.mcmc_run(opts, chain_cell, *inputs, chain_uid=uid, want_flags=True)
-    for i, c in enumerate(chain_cell):
-        N = int(cells_npz["N"][c]); npar = 7 + N
-        d = _lib.rng_dump(seed, int(uid[i]), npar, 1 + 2 * N, nsimu)
+    Ns = cells_npz["N"][chain_cell]
+    st = dumped_streams(Ns, uid, seed, nsimu)
+    for i, N in enumerate(Ns):
         # sanity of the streams themselves
-        assert abs(d["z1"][1:].mean()) < 0.02 and abs(d["z1"][1:].std() - 1) < 0.02
-        assert 0 < d["u1"].min() and d["u1"].max() < 1
-        assert abs(d["chi2"][1:].mean() / (1 + 2 * N) - 1) < 0.02
-        st = {k: v[None] for k, v in d.items()}
-        pad = np.zeros((1, nsimu, gpu_cells.ld)); pad[0, :, :npar] = d["z1"]; st["z1"] = pad
-        pad = np.zeros((1, nsimu, gpu_cells.ld)); pad[0, :, :npar] = d["z2"]; st["z2"] = pad
-        ref = _oracle_chain(orc, cells_npz, int(c), dict(nsimu=nsimu, burnintime=burn),
-                            [x[i:i + 1] for x in inputs], 0, st)
-        assert np.array_equal(out["flags"][i], ref["flags"])
-        np.testing.assert_allclose(out["chain"][i][:, :npar], ref["chain"], rtol=0, atol=1e-7)
+        assert abs(st["z1"][i][1:].mean()) < 0.02 and abs(st["z1"][i][1:].std() - 1) < 0.02
+        assert 0 < st["u1"][i].min() and st["u1"][i].max() < 1
+        assert abs(st["chi2"][i][1:].mean() / (1 + 2 * int(N)) - 1) < 0.02
+    refs = oracle_chains(orc, cells_npz, chain_cell, co.default_opts(nsimu, burn, **SHORT), inputs, st)
+    for i, ref in enumerate(refs):
+        check_chain("philox", out, i, ref, 7 + int(Ns[i]))
 
 
 def test_results_independent_of_partition(gpu_cells):
     """Philox draws are keyed by (seed, chain_uid): running a chain alone or inside a larger batch
     gives bit-identical output (this is what makes the output independent of the GPU count)."""
-    from transcriptioncycleinference_b200 import _lib
     cc = np.array([10, 20, 30, 40], dtype=np.int32)
     uid = np.array([10, 20, 30, 40], dtype=np.uint64)
     inputs = _setup(gpu_cells, cc, 31)
@@ -122,7 +91,6 @@ def test_solo_sm_scheduling_is_transparent(gpu_cells, monkeypatch):
     gives way at its next slice boundary, csrc/tc_mcmc.cu: smctl).  That is scheduling only: 299 chains x 6 000 steps give
     bit-identical summaries and counters with the rule off (TC_SOLO_LAG=0), at its default, and at its most eager setting
     with many short slices."""
-    from transcriptioncycleinference_b200 import _lib
     cc = np.arange(299, dtype=np.int32)
     inputs = _setup(gpu_cells, cc, 77)
     opts = _lib.default_opts(nsimu=6000, burnintime=1000, n_burn=1000)
@@ -144,7 +112,6 @@ def test_solo_sm_scheduling_is_transparent(gpu_cells, monkeypatch):
 def test_chain_layout_and_bounds(gpu_cells, cells_npz):
     """Row 1 = x0, s2chain(1) = sigma2_0 = 1, n_steps - n_burn + 1 stored rows, samples inside the
     bounds (SURVEY 0.1 #7, 4.2)."""
-    from transcriptioncycleinference_b200 import _lib
     cc = np.arange(0, 299, 23, dtype=np.int32)
     inputs = _setup(gpu_cells, cc, 41)
     th0, q, lo, hi, mu, sg = inputs
@@ -172,7 +139,7 @@ def test_time_slices_are_transparent(gpu_cells, cells_npz, orc):
     nsimu = 3300 a slice is 200 steps = two adaptation intervals, and there are 17 park/resume
     cycles: the production run must still be the oracle's chain on the device's own Philox streams
     (regression: the parked phase clocks once overlapped x[0])."""
-    from transcriptioncycleinference_b200 import _lib
+    co, _ = orc
     chain_cell = np.array([0, 250], dtype=np.int32)
     uid = np.array([0, 250 << 20], dtype=np.uint64)
     nsimu, burn, seed = 3300, 1000, 20201028
@@ -180,15 +147,11 @@ def test_time_slices_are_transparent(gpu_cells, cells_npz, orc):
     opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, seed=seed, **SHORT)
     out = gpu_cells.mcmc_run(opts, chain_cell, *inputs, chain_uid=uid, want_flags=True)
     assert np.all(out["counters"][:, [_lib.CNT_CYCLES0 + 3, _lib.CNT_CYCLES0 + 4, _lib.CNT_CYCLES0 + 6]] == 0)   # phases dram_kernel does not time
-    for i, c in enumerate(chain_cell):
-        N = int(cells_npz["N"][c]); npar = 7 + N
-        d = _lib.rng_dump(seed, int(uid[i]), npar, 1 + 2 * N, nsimu)
-        st = {k: v[None] for k, v in d.items()}
-        ref = _oracle_chain(orc, cells_npz, int(c), dict(nsimu=nsimu, burnintime=burn),
-                            [x[i:i + 1] for x in inputs], 0, st)
-        assert np.array_equal(out["flags"][i], ref["flags"])
-        np.testing.assert_allclose(out["chain"][i][:, :npar], ref["chain"], rtol=0, atol=1e-7)
-        np.testing.assert_allclose(out["s2chain"][i], ref["s2chain"], rtol=1e-9)
+    Ns = cells_npz["N"][chain_cell]
+    refs = oracle_chains(orc, cells_npz, chain_cell, co.default_opts(nsimu, burn, **SHORT), inputs,
+                         dumped_streams(Ns, uid, seed, nsimu))
+    for i, ref in enumerate(refs):
+        check_chain("time slices", out, i, ref, 7 + int(Ns[i]))
 
 
 @pytest.mark.parametrize("variant", [
@@ -197,26 +160,20 @@ def test_time_slices_are_transparent(gpu_cells, cells_npz, orc):
     dict(burnin_cumulative=0),                      # burn-in scaling on the rejection rate since the last adaptation
     dict(adaptint=64, drscale=3.0, qcovadj=1e-6),   # other adaptation interval / DR scale / regulariser
 ])
-@pytest.mark.parametrize("layout", [3, 2, 1], ids=["cta", "warp", "big"])   # TC_LAYOUT_CTA, _WARP, _BIG
+@pytest.mark.parametrize("layout", [l for l, _ in LAYOUTS], ids=[n for _, n in LAYOUTS])
 def test_replay_option_variants(gpu_cells, cells_npz, orc, variant, layout):
     """Every tc_mcmc_opts field that changes the DRAM arithmetic, replayed against the oracle with the same
-    injected randomness on every sampler layout: flags identical, chains equal."""
-    from transcriptioncycleinference_b200 import _lib
+    injected randomness on every sampler layout: flags, rows, s2chain, sschain and every counter."""
     co, _ = orc
     chain_cell = np.array([7, 123, 250], dtype=np.int32)
     nsimu, burn = 420, 150
     inputs = _setup(gpu_cells, chain_cell, 61)
-    st = _streams(len(chain_cell), nsimu, gpu_cells.ld, cells_npz["N"][chain_cell], 62)
+    st = replay_streams(cells_npz["N"][chain_cell], nsimu, gpu_cells.ld, 62)
     opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, replay=1, layout=layout, **SHORT, **variant)
     out = gpu_cells.mcmc_run(opts, chain_cell, *inputs, replay=st, want_flags=True)
-    for i, c in enumerate(chain_cell):
-        N = int(cells_npz["N"][c]); o = int(cells_npz["off"][c]); npar = 7 + N
-        t, ms2, pp7 = (cells_npz[k][o:o + N] for k in ("t", "ms2", "pp7"))
-        sti = dict(z1=st["z1"][i][:, :npar], u1=st["u1"][i], z2=st["z2"][i][:, :npar], u2=st["u2"][i], chi2=st["chi2"][i])
-        ref = co.dram(orc[1], t, ms2, pp7, co.default_opts(nsimu, burn, **SHORT, **variant), *[x[i, :npar] for x in inputs], streams=sti)
-        assert np.array_equal(out["flags"][i], ref["flags"]), (variant, layout, i)
-        np.testing.assert_allclose(out["chain"][i][:, :npar], ref["chain"], rtol=0, atol=1e-7)
-        np.testing.assert_allclose(out["s2chain"][i], ref["s2chain"], rtol=1e-9)
+    refs = oracle_chains(orc, cells_npz, chain_cell, co.default_opts(nsimu, burn, **SHORT, **variant), inputs, st)
+    for i, ref in enumerate(refs):
+        check_chain((variant, layout), out, i, ref, 7 + int(cells_npz["N"][chain_cell[i]]))
 
 
 def test_posterior_means_agree_with_independent_cpu_chains(gpu_cells, cells_npz, orc):
@@ -224,7 +181,6 @@ def test_posterior_means_agree_with_independent_cpu_chains(gpu_cells, cells_npz,
     Carlo standard error — against the only long reference-algorithm chains that can exist here: the CPU oracle's,
     run with ITS OWN random numbers (xorshift, not Philox).  12 chains per side on each of 3 cells, same x0 per
     chain index; the standard error is the between-chain one, the bound is 4 combined standard errors."""
-    from transcriptioncycleinference_b200 import _lib
     co, cons = orc
     cells3 = np.array([12, 150, 270], dtype=np.int32)
     per = 12
@@ -250,21 +206,20 @@ def test_big_layout_matches_oracle_and_regular_layout(gpu_cells, cells_npz, orc)
     (1) replay against the oracle over burn-in + 5 covariance adaptations, flags identical; (2) production Philox run,
     regular vs big layout: the two differ only in the rounding of the Cholesky factor (shared-memory right-looking vs
     left-looking through L2), so the accept/reject sequence and the counters must be identical and the means equal to rounding."""
-    from transcriptioncycleinference_b200 import _lib
+    co, _ = orc
     chain_cell = np.array([0, 57, 130, 298], dtype=np.int32)
     inputs = _setup(gpu_cells, chain_cell, 21)
     nsimu, burn = 600, 200
-    st = _streams(len(chain_cell), nsimu, gpu_cells.ld, [int(cells_npz["N"][c]) for c in chain_cell], 22)
-    opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, replay=1, layout=1, **SHORT)
+    st = replay_streams(cells_npz["N"][chain_cell], nsimu, gpu_cells.ld, 22)
+    opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, replay=1, layout=_lib.LAYOUT_BIG, **SHORT)
     out = gpu_cells.mcmc_run(opts, chain_cell, *inputs, replay=st, want_flags=True)
-    for i, c in enumerate(chain_cell):
-        npar = 7 + int(cells_npz["N"][c])
-        ref = _oracle_chain(orc, cells_npz, int(c), dict(nsimu=nsimu, burnintime=burn), inputs, i, st)
-        assert np.array_equal(out["flags"][i], ref["flags"]), c
-        np.testing.assert_allclose(out["chain"][i][:, :npar], ref["chain"], rtol=0, atol=1e-7)
-        assert out["counters"][i][4] == 5 and out["counters"][i][5] == 0          # adaptations at 200..600, no Cholesky failure
+    refs = oracle_chains(orc, cells_npz, chain_cell, co.default_opts(nsimu, burn, **SHORT), inputs, st)
+    for i, ref in enumerate(refs):
+        check_chain("big", out, i, ref, 7 + int(cells_npz["N"][chain_cell[i]]))
+        cnt = out["counters"][i]
+        assert cnt[_lib.CNT_ADAPTATIONS] == 5 and cnt[_lib.CNT_CHOL_FAIL] == 0        # adaptations at 200..600, no Cholesky failure
     res = []
-    for layout in (0, 1):
+    for layout in (_lib.LAYOUT_AUTO, _lib.LAYOUT_BIG):
         opts = _lib.default_opts(nsimu=3000, burnintime=500, n_burn=500, layout=layout, seed=99, **SHORT)
         res.append(gpu_cells.mcmc_run(opts, chain_cell, *inputs, want_flags=True))
     assert np.array_equal(res[0]["flags"], res[1]["flags"])
@@ -277,68 +232,58 @@ def test_replay_long_default_path(gpu_cells, cells_npz, orc):
     (cumulative burn-in rule, chol(cov) first): burn-in of 5 000 steps (50 scaling decisions), then 150 covariance
     adaptations = 150 Cholesky factorisations of a well-conditioned covariance (>= 5 000 rows).  Flags identical over
     all 20 000 steps, chain equal to 1e-6 (150 factorisations in a different summation order), counters equal."""
-    from transcriptioncycleinference_b200 import _lib
+    co, _ = orc
     nsimu, burn = 20000, 5000
-    for c, layout in ((17, 0), (211, 1), (250, 2)):
+    for c, layout in ((17, _lib.LAYOUT_AUTO), (211, _lib.LAYOUT_BIG), (250, _lib.LAYOUT_WARP)):
         chain_cell = np.array([c], dtype=np.int32)
         inputs = _setup(gpu_cells, chain_cell, 81 + layout)
-        st = _streams(1, nsimu, gpu_cells.ld, cells_npz["N"][chain_cell], 82 + layout)
+        st = replay_streams(cells_npz["N"][chain_cell], nsimu, gpu_cells.ld, 82 + layout)
         opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, replay=1, layout=layout)
         assert opts.burnin_cumulative == 1 and opts.qcovadj_always == 0
         out = gpu_cells.mcmc_run(opts, chain_cell, *inputs, replay=st, want_flags=True)
-        ref = _oracle_chain(orc, cells_npz, c, dict(nsimu=nsimu, burnintime=burn, extra={}), inputs, 0, st)
-        npar = 7 + int(cells_npz["N"][c])
-        ndiff = int(np.sum(out["flags"][0] != ref["flags"]))
-        assert ndiff == 0, "accept/reject differs at %d steps, first at %d" % (ndiff, int(np.argmax(out["flags"][0] != ref["flags"])))
-        np.testing.assert_allclose(out["chain"][0][:, :npar], ref["chain"], rtol=0, atol=1e-6)
-        np.testing.assert_allclose(out["s2chain"][0], ref["s2chain"], rtol=1e-8)
+        ref, = oracle_chains(orc, cells_npz, chain_cell, co.default_opts(nsimu, burn), inputs, st)
+        check_chain("layout %d" % layout, out, 0, ref, 7 + int(cells_npz["N"][c]), atol=1e-6)
         cnt = out["counters"][0]
-        assert cnt[_lib.CNT_ADAPTATIONS] == ref["counters"][4] == 151 and cnt[_lib.CNT_CHOL_FAIL] == 0
-        assert cnt[_lib.CNT_SS_EVALS] == ref["counters"][0]
+        assert cnt[_lib.CNT_ADAPTATIONS] == 151 and cnt[_lib.CNT_CHOL_FAIL] == 0
 
 
 def test_replay_200_adaptations(gpu_cells, cells_npz, orc):
     """20 000 steps with a burn-in of 100: 199 covariance adaptations (VERDICT r1: nothing compared a long run with the
     oracle).  The early covariances are singular, so cov + qcovadj I is factored on both sides (see the module docstring)."""
-    from transcriptioncycleinference_b200 import _lib
+    co, _ = orc
     nsimu, burn, c = 20000, 100, 123
     chain_cell = np.array([c], dtype=np.int32)
     inputs = _setup(gpu_cells, chain_cell, 91)
-    st = _streams(1, nsimu, gpu_cells.ld, cells_npz["N"][chain_cell], 92)
+    st = replay_streams(cells_npz["N"][chain_cell], nsimu, gpu_cells.ld, 92)
     opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, replay=1, **SHORT)
     out = gpu_cells.mcmc_run(opts, chain_cell, *inputs, replay=st, want_flags=True)
-    ref = _oracle_chain(orc, cells_npz, c, dict(nsimu=nsimu, burnintime=burn), inputs, 0, st)
-    npar = 7 + int(cells_npz["N"][c])
-    assert np.array_equal(out["flags"][0], ref["flags"])
-    np.testing.assert_allclose(out["chain"][0][:, :npar], ref["chain"], rtol=0, atol=1e-6)
-    assert out["counters"][0][_lib.CNT_ADAPTATIONS] == ref["counters"][4] == 200
+    ref, = oracle_chains(orc, cells_npz, chain_cell, co.default_opts(nsimu, burn, **SHORT), inputs, st)
+    check_chain("200 adaptations", out, 0, ref, 7 + int(cells_npz["N"][c]), atol=1e-6)
+    assert out["counters"][0][_lib.CNT_ADAPTATIONS] == 200
 
 
 def test_singular_covariance_falls_back(gpu_cells, cells_npz, orc):
     """A chain that cannot move (low = upp = theta0: every proposal is out of bounds) has an exactly zero covariance:
     chol(cov) fails for certain and the default path must fall back to chol(cov + qcovadj I) = sqrt(qcovadj) I, as
     mcmcstat's "try to blow it" branch does — not count a failed adaptation."""
-    from transcriptioncycleinference_b200 import _lib
+    co, _ = orc
     chain_cell = np.array([5], dtype=np.int32)
     th0, q, lo, hi, mu, sg = _setup(gpu_cells, chain_cell, 95)
-    lo, hi = th0.copy(), th0.copy()
+    ins = (th0, q, th0.copy(), th0.copy(), mu, sg)
     nsimu, burn = 400, 200
-    st = _streams(1, nsimu, gpu_cells.ld, cells_npz["N"][chain_cell], 96)
-    for layout in (0, 1, 2):
+    st = replay_streams(cells_npz["N"][chain_cell], nsimu, gpu_cells.ld, 96)
+    ref, = oracle_chains(orc, cells_npz, chain_cell, co.default_opts(nsimu, burn), ins, st)
+    for layout in (_lib.LAYOUT_AUTO, _lib.LAYOUT_BIG, _lib.LAYOUT_WARP):
         opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, replay=1, layout=layout)
-        out = gpu_cells.mcmc_run(opts, chain_cell, th0, q, lo, hi, mu, sg, replay=st, want_flags=True)
-        ref = _oracle_chain(orc, cells_npz, 5, dict(nsimu=nsimu, burnintime=burn, extra={}), (th0, q, lo, hi, mu, sg), 0, st)
-        assert np.array_equal(out["flags"][0], ref["flags"])
-        assert out["counters"][0][_lib.CNT_ADAPTATIONS] == ref["counters"][4] == 3
-        assert out["counters"][0][_lib.CNT_CHOL_FAIL] == ref["counters"][5] == 0
+        out = gpu_cells.mcmc_run(opts, chain_cell, *ins, replay=st, want_flags=True)
+        check_chain("layout %d" % layout, out, 0, ref, 7 + int(cells_npz["N"][5]))
+        assert out["counters"][0][_lib.CNT_ADAPTATIONS] == 3 and out["counters"][0][_lib.CNT_CHOL_FAIL] == 0
 
 
 def test_input_validation_and_device_restored(gpu_cells):
     """mcmcstat refuses an initial value outside its bounds; a zero / NaN prior width would make the prior sum NaN and the
     chain would silently never accept: both are TC_EINVAL with the chain and parameter index.  ss(theta0) not finite is
     reported (TC_ESTATE) even when the caller does not ask for counters.  The caller's current device is left alone."""
-    import ctypes as C
-    from transcriptioncycleinference_b200 import _lib
     cc = np.array([1, 2], dtype=np.int32)
     th0, q, lo, hi, mu, sg = _setup(gpu_cells, cc, 5)
     opts = _lib.default_opts(nsimu=50, burnintime=20, n_burn=1)
@@ -351,12 +296,16 @@ def test_input_validation_and_device_restored(gpu_cells):
     lo2 = lo.copy(); lo2[0, 0] = hi[0, 0] + 1.0
     with pytest.raises(_lib.TcError, match="low must be <= upp"):
         gpu_cells.mcmc_run(opts, cc, th0, q, lo2, hi, mu, sg)
-    # TC_ESTATE without a counters buffer: call the ABI directly with counters = NULL
-    L = _lib.load()
-    nan0 = th0.copy(); nan0[0, 6] = np.nan                      # NaN passes no bound check -> EINVAL, so use an infinite ss instead:
-    with pytest.raises(_lib.TcError):
+    nan0 = th0.copy(); nan0[0, 6] = np.nan                      # NaN lies inside no bounds
+    with pytest.raises(_lib.TcError, match=r"theta0 must lie inside"):
         gpu_cells.mcmc_run(opts, cc, nan0, q, lo, hi, mu, sg)
-    cudart = C.CDLL("libcudart.so.12") if False else None      # the device guard is covered through torch when it is importable
+    # TC_ESTATE without a counters buffer (the ABI called directly with counters = NULL): chain 0 starts at A = 1e200
+    # (upp = 1e300, flat prior on A), so its squared residual overflows and ss(theta0) = inf
+    inf0 = th0.copy(); inf0[0, 5] = 1e200
+    hi0 = hi.copy(); hi0[0, 5] = 1e300
+    assert np.isinf(sg[0, 5])
+    rc, msg, _ = raw_run(gpu_cells, opts, cc, (inf0, q, lo, hi0, mu, sg), np.arange(cc.size, dtype=np.uint64), counters=False)
+    assert rc == _lib.TC_ESTATE and "chain 0" in msg, (rc, msg)
     try:
         import torch
         if torch.cuda.device_count() >= 1:
@@ -374,35 +323,33 @@ def test_warp_kernel_production_path(gpu_cells, cells_npz, orc):
     accept/reject sequence and counters, means equal to rounding (the two kernels factor the covariance in different orders);
     (3) option variants the warp kernel implements separately: ntry = 1, updatesigma = 0, a bounds vector without the
     reference's head + block structure (generic path)."""
-    from transcriptioncycleinference_b200 import _lib
+    co, _ = orc
     cc = np.arange(0, 296, 8, dtype=np.int32)                     # 37 chains of different cells
     uid = cc.astype(np.uint64) * np.uint64(1 << 20) + np.uint64(3)
     nsimu, burn, seed = 3300, 1000, 20201028
     inputs = _setup(gpu_cells, cc, 101)
     res = {}
-    for layout in (2, 0):
+    for layout in (_lib.LAYOUT_WARP, _lib.LAYOUT_AUTO):
         # 1 000-row covariances of ~130 parameters are nearly singular: chol(cov) without the regulariser amplifies the
         # rounding differences between the kernels' factorisations to 1e-3 in the chain (measured), so: SHORT
         opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, n_burn=1, store_chain=1, seed=seed, layout=layout, **SHORT)
         res[layout] = gpu_cells.mcmc_run(opts, cc, *inputs, chain_uid=uid, want_flags=True)
-    assert np.array_equal(res[2]["flags"], res[0]["flags"])
-    assert np.array_equal(res[2]["counters"][:, :8], res[0]["counters"][:, :8])
-    assert np.array_equal(res[2]["counters"][:, _lib.CNT_CYCLES0 + 7], res[2]["counters"][:, _lib.CNT_SS_EVALS])
-    np.testing.assert_allclose(res[2]["mean"], res[0]["mean"], rtol=0, atol=1e-6)
-    np.testing.assert_allclose(res[2]["sig"], res[0]["sig"], rtol=1e-9)
-    for i in (0, 17, 36):
-        c = int(cc[i]); N = int(cells_npz["N"][c]); npar = 7 + N
-        d = _lib.rng_dump(seed, int(uid[i]), npar, 1 + 2 * N, nsimu)
-        st = {k: v[None] for k, v in d.items()}
-        ref = _oracle_chain(orc, cells_npz, c, dict(nsimu=nsimu, burnintime=burn), [x[i:i + 1] for x in inputs], 0, st)
-        assert np.array_equal(res[2]["flags"][i], ref["flags"])
-        np.testing.assert_allclose(res[2]["chain"][i][:, :npar], ref["chain"], rtol=0, atol=1e-7)
-        np.testing.assert_allclose(res[2]["s2chain"][i], ref["s2chain"], rtol=1e-9)
+    warp, auto = res[_lib.LAYOUT_WARP], res[_lib.LAYOUT_AUTO]
+    assert np.array_equal(warp["flags"], auto["flags"])
+    assert np.array_equal(warp["counters"][:, :8], auto["counters"][:, :8])
+    assert np.array_equal(warp["counters"][:, _lib.CNT_CYCLES0 + 7], warp["counters"][:, _lib.CNT_SS_EVALS])
+    np.testing.assert_allclose(warp["mean"], auto["mean"], rtol=0, atol=1e-6)
+    np.testing.assert_allclose(warp["sig"], auto["sig"], rtol=1e-9)
+    sel = [0, 17, 36]
+    refs = oracle_chains(orc, cells_npz, cc[sel], co.default_opts(nsimu, burn, **SHORT), [x[sel] for x in inputs],
+                         dumped_streams(cells_npz["N"][cc[sel]], uid[sel], seed, nsimu))
+    for i, ref in zip(sel, refs):
+        check_chain("warp philox", warp, i, ref, 7 + int(cells_npz["N"][cc[i]]))
     th0, q, lo, hi, mu, sg = [x[:3].copy() for x in inputs]
     lo[:, 40] = -25.0; sg[:, 55] = 10.0                          # breaks the head + block structure
     for variant in (dict(ntry=1), dict(updatesigma=0), dict()):
-        a = gpu_cells.mcmc_run(_lib.default_opts(nsimu=700, burnintime=300, n_burn=1, seed=5, layout=2, **SHORT, **variant), cc[:3], th0, q, lo, hi, mu, sg, want_flags=True)
-        b = gpu_cells.mcmc_run(_lib.default_opts(nsimu=700, burnintime=300, n_burn=1, seed=5, layout=0, **SHORT, **variant), cc[:3], th0, q, lo, hi, mu, sg, want_flags=True)
+        a = gpu_cells.mcmc_run(_lib.default_opts(nsimu=700, burnintime=300, n_burn=1, seed=5, layout=_lib.LAYOUT_WARP, **SHORT, **variant), cc[:3], th0, q, lo, hi, mu, sg, want_flags=True)
+        b = gpu_cells.mcmc_run(_lib.default_opts(nsimu=700, burnintime=300, n_burn=1, seed=5, layout=_lib.LAYOUT_AUTO, **SHORT, **variant), cc[:3], th0, q, lo, hi, mu, sg, want_flags=True)
         assert np.array_equal(a["flags"], b["flags"]), variant
         np.testing.assert_allclose(a["mean"], b["mean"], rtol=0, atol=1e-6)
 
@@ -414,7 +361,6 @@ def test_philox_variates_pass_ks(gpu_cells):
     Kolmogorov-Smirnov at 2.5e5 - 5e6 draws (p > 1e-3), moments within 4 standard errors, tails present up to 4.5 sigma,
     and no correlation between the two stages or consecutive steps."""
     from scipy import stats
-    from transcriptioncycleinference_b200 import _lib
     npar, nsimu, nu = 127, 20000, 241.0
     d = _lib.rng_dump(20201028, 123456789, npar, nu, nsimu)
     for k in ("z1", "z2"):

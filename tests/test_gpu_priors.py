@@ -24,12 +24,11 @@ iteration), on every layout; a dataset with N = 257 (where the big layout is cho
 import numpy as np
 import pytest
 
-from test_gpu_lengths import _cols, make_cells
-from test_gpu_schedule import (LAYOUTS, ORC_OOB, _check_chain, _check_recorded_ss, _dumped_streams, _ld_mean_std,
-                               _lib_or_skip, _oracles, _replay_streams)
+from parity import (LAYOUTS, ORC_OOB, check_chain, check_recorded_ss, cols, dumped_streams, ld_mean_std, make_cells, need_gpu,
+                    oracle_chains, replay_streams)
+from transcriptioncycleinference_b200 import _lib
 
 pytestmark = pytest.mark.gpu
-BIG = 1
 NSIMU, BURN, ADAPT = 600, 200, 100
 POSITIONS = (7, 8, 31, 32, 33, 63, 64, 127, 128)       # and npar - 1
 KEYS = ("th0", "q", "lo", "hi", "mu", "sg")              # the six chain inputs, in tc_mcmc_run's order
@@ -189,19 +188,19 @@ def _fam(*names):
     return [(n, f) for n in names for f in FAMILIES[n]]
 
 
-def _check_run(_lib, tag, cells, cc, out, refs):
-    """_check_chain for every chain, the recorded SS of every row, and mean / population std of the stored rows against a
+def _check_run(tag, cells, cc, out, refs):
+    """check_chain for every chain, the recorded SS of every row, and mean / population std of the stored rows against a
     long-double reduction of the oracle's rows (the rows agree to 1e-7)."""
     for i, ref in enumerate(refs):
         npar = 7 + int(cells.N[cc[i]])
-        _check_chain(_lib, tag, out, i, ref, npar)
-        m, s = _ld_mean_std(ref["chain"])
+        check_chain(tag, out, i, ref, npar)
+        m, s = ld_mean_std(ref["chain"])
         np.testing.assert_allclose(out["mean"][i, :npar], m.astype(np.float64), rtol=0, atol=2e-7, err_msg=str((tag, i)))
         np.testing.assert_allclose(out["std"][i, :npar], s.astype(np.float64), rtol=0, atol=2e-7, err_msg=str((tag, i)))
-    _check_recorded_ss(cells, cc, out, out["chain"].shape[2])
+    check_recorded_ss(cells, cc, out, out["chain"].shape[2])
 
 
-def _replay_opts(_lib, layout, nsimu=NSIMU):
+def _replay_opts(layout, nsimu=NSIMU):
     return _lib.default_opts(nsimu=nsimu, burnintime=BURN, adaptint=ADAPT, n_burn=1, store_chain=1, replay=1, layout=layout,
                              qcovadj_always=1)
 
@@ -213,8 +212,8 @@ def _orc_opts(co, nsimu=NSIMU, burn=BURN):
 @pytest.fixture(scope="module")
 def cells2(orc):
     """N = 12 on an irregular grid, N = 129 on a regular grid."""
-    _lib_or_skip()
-    cells, packed = make_cells(orc[0], _cols(orc, (12, 129), 4243))
+    need_gpu()
+    cells, packed = make_cells(orc[0], cols(orc, (12, 129), 4243))
     assert cells.N.tolist() == [12, 129]
     yield cells, packed
     cells.close()
@@ -223,8 +222,8 @@ def cells2(orc):
 @pytest.fixture(scope="module")
 def cells3(orc):
     """N = 12, 129 and 257 in one dataset (ld = 264: the big layout is the one chosen automatically)."""
-    _lib_or_skip()
-    cells, packed = make_cells(orc[0], _cols(orc, (12, 129, 257), 4244))
+    need_gpu()
+    cells, packed = make_cells(orc[0], cols(orc, (12, 129, 257), 4244))
     assert cells.N.tolist() == [12, 129, 257]
     yield cells, packed
     cells.close()
@@ -232,24 +231,24 @@ def cells3(orc):
 
 # ------------------------------------------------------------------------------------------------ 1. replays
 def _family_replay(orc, cells, packed, names, layouts, seed):
-    _lib = _lib_or_skip()
+    need_gpu()
     co, _ = orc
     cc, mods = plan(cells, _fam(*names))
-    st, per = _replay_streams(cells, cc, NSIMU, cells.ld, seed)
+    st = replay_streams(cells.N[cc], NSIMU, cells.ld, seed)
     ins, base, info = apply(cells, cc, mods, seed + 1, z1=st["z1"][:, 1])
     assert any(u for _, u, _ in info) and (names[0] in "AB" or not all(u for _, u, _ in info))
-    refs = _oracles(orc, cells, packed, cc, _orc_opts(co), ins, per)
+    refs = oracle_chains(orc, packed, cc, _orc_opts(co), ins, st)
     for layout, name in layouts:
-        out = cells.mcmc_run(_replay_opts(_lib, layout), cc, *ins, replay=st, want_flags=True)
-        _check_run(_lib, "%s %s" % ("".join(names), name), cells, cc, out, refs)
-    return cc, ins, base, info, st, per, refs
+        out = cells.mcmc_run(_replay_opts(layout), cc, *ins, replay=st, want_flags=True)
+        _check_run("%s %s" % ("".join(names), name), cells, cc, out, refs)
+    return cc, ins, base, info, st, refs
 
 
-def _guard_tight_prior(orc, cells, packed, cc, base, info, per, refs):
+def _guard_tight_prior(orc, cells, packed, cc, base, info, st, refs):
     """Family A: on the same streams the oracle's flags at width 0.5 differ from its flags at the reference's width 50."""
     co, _ = orc
     idx = [i for i, (fam, _, _) in enumerate(info) if fam == "A"]
-    wide = _oracles(orc, cells, packed, cc[idx], _orc_opts(co), [x[idx] for x in base], [per[i] for i in idx])
+    wide = oracle_chains(orc, packed, cc[idx], _orc_opts(co), [x[idx] for x in base], {k: v[idx] for k, v in st.items()})
     diff = {}
     for k, i in enumerate(idx):
         sg = np.unique(base[5][i][7:7 + int(cells.N[cc[i]])])
@@ -288,9 +287,9 @@ def test_family_replay(orc, cells2, fam):
     """600 steps, burn-in 200, adaptint 100, qcovadj_always = 1, every layout: flags, rows, s2chain, sschain, all counters
     (out-of-bounds proposals and delayed-rejection tries included), the recorded SS of every row, mean and std."""
     cells, packed = cells2
-    cc, ins, base, info, st, per, refs = _family_replay(orc, cells, packed, (fam,), LAYOUTS, 100 + ord(fam))
+    cc, ins, base, info, st, refs = _family_replay(orc, cells, packed, (fam,), LAYOUTS, 100 + ord(fam))
     if fam == "A":
-        _guard_tight_prior(orc, cells, packed, cc, base, info, per, refs)
+        _guard_tight_prior(orc, cells, packed, cc, base, info, st, refs)
     if fam == "E":
         _check_on_bound(cells, cc, ins, info, st, refs)
 
@@ -300,7 +299,7 @@ def test_family_replay_long_cell_big_layout(orc, cells3, fam):
     """The same with a cell of N = 257 in the dataset, under the big layout, where bounds and prior means are read from
     HBM at stride ld = 264 for every chain (npar = 19, 136, 264)."""
     cells, packed = cells3
-    cc, ins, base, info, st, per, refs = _family_replay(orc, cells, packed, (fam,), [(BIG, "big")], 200 + ord(fam))
+    cc, ins, base, info, st, refs = _family_replay(orc, cells, packed, (fam,), [(_lib.LAYOUT_BIG, "big")], 200 + ord(fam))
     if fam == "E":
         _check_on_bound(cells, cc, ins, info, st, refs)
 
@@ -313,20 +312,20 @@ def test_production_families_against_oracle(orc, cells2):
     """Families A, B, D and part of C in one launch on the device's Philox streams, 3300 steps (burn-in 1000, adaptint
     100): many time slices, so the structure check runs again on every slice and dram_warp_kernel reuses the reciprocal
     widths it stored at slice 0.  Every layout against the oracle on tc_rng_dump's streams."""
-    _lib = _lib_or_skip()
+    need_gpu()
     co, _ = orc
     cells, packed = cells2
     nsimu, burn, seed = 3300, 1000, 2718
     cc, mods = plan(cells, _fam("A", "B", "D") + PHILOX_C)
     ins, _, info = apply(cells, cc, mods, 300)
     uid = np.arange(cc.size, dtype=np.uint64) * np.uint64(31) + np.uint64(17)
-    refs = _oracles(orc, cells, packed, cc, _orc_opts(co, nsimu, burn), ins, _dumped_streams(_lib, cells, cc, uid, seed, nsimu))
+    refs = oracle_chains(orc, packed, cc, _orc_opts(co, nsimu, burn), ins, dumped_streams(cells.N[cc], uid, seed, nsimu))
     for layout, name in LAYOUTS:
         opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, adaptint=ADAPT, n_burn=1, store_chain=1, seed=seed,
                                  layout=layout, qcovadj_always=1)
         out = cells.mcmc_run(opts, cc, *ins, chain_uid=uid, want_flags=True)
         for i, ref in enumerate(refs):
-            _check_chain(_lib, "philox %s %s" % (name, info[i][0]), out, i, ref, 7 + int(cells.N[cc[i]]))
+            check_chain("philox %s %s" % (name, info[i][0]), out, i, ref, 7 + int(cells.N[cc[i]]))
 
 
 # ------------------------------------------------------------------------------------------------ 3. padded ld, big layout
@@ -335,19 +334,19 @@ def test_padded_leading_dimension_big_layout(orc, cells2):
     layout each chain's bounds and prior means are read from HBM at ch * ld.  Replayed against the oracle on every layout.
     (This found dram_warp_kernel carving its per-warp shared-memory regions and increment slots for N = ld - 7 while the
     host had sized them for max N: with a padded ld the last warps ran past both.)"""
-    _lib = _lib_or_skip()
+    need_gpu()
     co, _ = orc
     cells, packed = cells2
     fams = _fam("A", "B", "D", "E") + [m for m in _fam("C") if m[1] in FAMILIES["C"][::3]]
     cc, mods = plan(cells, fams, first_plain=True)
     ld = cells.ld + 5
-    st, per = _replay_streams(cells, cc, NSIMU, ld, 400)
+    st = replay_streams(cells.N[cc], NSIMU, ld, 400)
     ins, _, info = apply(cells, cc, mods, 401, z1=st["z1"][:, 1], ld_pad=5)
     assert info[0][0] is None and ins[0].shape[1] == ld
-    refs = _oracles(orc, cells, packed, cc, _orc_opts(co), ins, per)
-    for layout, name in [(BIG, "big")] + [l for l in LAYOUTS if l[0] != BIG]:
-        out = cells.mcmc_run(_replay_opts(_lib, layout), cc, *ins, replay=st, want_flags=True)
-        _check_run(_lib, "ld+5 %s" % name, cells, cc, out, refs)
+    refs = oracle_chains(orc, packed, cc, _orc_opts(co), ins, st)
+    for layout, name in [(_lib.LAYOUT_BIG, "big")] + [l for l in LAYOUTS if l[0] != _lib.LAYOUT_BIG]:
+        out = cells.mcmc_run(_replay_opts(layout), cc, *ins, replay=st, want_flags=True)
+        _check_run("ld+5 %s" % name, cells, cc, out, refs)
     _check_on_bound(cells, cc, ins, info, st, refs)
 
 
@@ -358,7 +357,7 @@ def test_uni_and_generic_paths_bit_for_bit(orc, cells2):
     is exactly 0 and only the path changes (a bound is never used for this: a bound moved out of reach can still be
     reached).  Finite head priors with non-zero means keep the prior sum non-trivial.  Replay and Philox (3300 steps, many
     time slices), every layout: flags, rows, s2chain, sschain, mean, std, sig and the counters are bit-identical."""
-    _lib = _lib_or_skip()
+    need_gpu()
     cells, _ = cells2
     hp = head_priors(1.0, 0.75, 0.5)
     half = []
@@ -376,10 +375,10 @@ def test_uni_and_generic_paths_bit_for_bit(orc, cells2):
             assert hp(x, npar)
             x["sg"][7:npar] = np.inf
         ins[4][2 * i + 1, p] = 2.5
-    sth, _ = _replay_streams(cells, cch, NSIMU, cells.ld, 501)
+    sth = replay_streams(cells.N[cch], NSIMU, cells.ld, 501)
     st = {k: np.ascontiguousarray(np.repeat(v, 2, axis=0)) for k, v in sth.items()}
     uid = np.repeat(np.arange(cch.size, dtype=np.uint64) + np.uint64(900), 2)
-    runs = [("replay", lambda layout: (_replay_opts(_lib, layout), dict(replay=st)))]
+    runs = [("replay", lambda layout: (_replay_opts(layout), dict(replay=st)))]
     runs.append(("philox", lambda layout: (_lib.default_opts(nsimu=3300, burnintime=1000, adaptint=ADAPT, n_burn=1,
                                                                store_chain=1, seed=77, layout=layout, qcovadj_always=1),
                                            dict(chain_uid=uid))))

@@ -17,34 +17,20 @@ adaptint = 1, of 1 when adaptation is off) and park the chain between them; n_bu
   * std(sqrt(s2chain),1) where it is exactly 0 and over 200 000 rows.
 
 Every case runs on two cells, N = 12 on an irregular grid and N = 129 on a regular one."""
-import concurrent.futures as cf
-import ctypes as C
-
 import numpy as np
 import pytest
 
-from test_gpu_lengths import _cols, make_cells
+from parity import (LAYOUTS, ORC_ADAPT, ORC_CHOL_FAIL, ORC_OOB, check_chain, check_recorded_ss, cols, dumped_streams,
+                    ld_mean_std, make_cells, need_gpu, oracle_chains, raw_run, replay_streams)
 
 pytestmark = pytest.mark.gpu
-BIG, WARP, CTA = 1, 2, 3
-LAYOUTS = [(CTA, "cta"), (WARP, "warp"), (BIG, "big")]
-# the oracle's counters (orc_dram): SS evaluations, stage-1 / stage-2 accepts, out-of-bounds proposals, adaptations,
-# Cholesky failures
-ORC_SS, ORC_ACC1, ORC_ACC2, ORC_OOB, ORC_ADAPT, ORC_CHOL_FAIL = range(6)
-
-
-def _lib_or_skip():
-    from transcriptioncycleinference_b200 import _lib
-    if _lib.device_count() < 1:
-        pytest.skip("no CUDA device")
-    return _lib
 
 
 @pytest.fixture(scope="module")
 def two_cells(orc):
     """(cells, packed): N = 12 on an irregular grid, N = 129 on a regular grid."""
-    _lib_or_skip()
-    cells, packed = make_cells(orc[0], _cols(orc, (12, 129), 4242))
+    need_gpu()
+    cells, packed = make_cells(orc[0], cols(orc, (12, 129), 4242))
     assert cells.N.tolist() == [12, 129]
     yield cells, packed
     cells.close()
@@ -60,44 +46,6 @@ def _inputs(cells, cc, seed, v0_chains=()):
         for x, y in zip(ins, one):
             x[i] = y[0]
     return ins
-
-
-def _oracle(orc, cells, packed, c, opts, ins, i, st):
-    """The oracle's chain i (cell c) on the streams st (per-chain arrays, [nsimu, >= npar])."""
-    co, cons = orc
-    N = int(cells.N[c]); o = int(cells.off[c]); npar = 7 + N
-    sti = dict(z1=st["z1"][:, :npar], u1=st["u1"], z2=st["z2"][:, :npar], u2=st["u2"], chi2=st["chi2"])
-    return co.dram(cons, packed["t"][o:o + N], packed["ms2"][o:o + N], packed["pp7"][o:o + N], opts,
-                   *[x[i, :npar] for x in ins], streams=sti)
-
-
-def _oracles(orc, cells, packed, cc, opts, ins, streams):
-    with cf.ThreadPoolExecutor() as ex:                            # the oracle releases the GIL
-        return list(ex.map(lambda i: _oracle(orc, cells, packed, int(cc[i]), opts, ins, i, streams[i]), range(cc.size)))
-
-
-def _check_chain(_lib, tag, out, i, ref, npar, first_row=0):
-    """Flags, rows, s2chain, sschain and all seven counters of device chain i against the oracle's chain."""
-    assert np.array_equal(out["flags"][i], ref["flags"]), (tag, i, int(np.argmax(out["flags"][i] != ref["flags"])))
-    np.testing.assert_allclose(out["chain"][i][:, :npar], ref["chain"][first_row:], rtol=0, atol=1e-7, err_msg=str((tag, i)))
-    np.testing.assert_allclose(out["s2chain"][i], ref["s2chain"], rtol=1e-9, err_msg=str((tag, i)))
-    np.testing.assert_allclose(out["sschain"][i], ref["sschain"], rtol=1e-9, err_msg=str((tag, i)))
-    cnt, rc = out["counters"][i], ref["counters"]
-    want = {_lib.CNT_SS_EVALS: rc[ORC_SS], _lib.CNT_ACC_STAGE1: rc[ORC_ACC1], _lib.CNT_ACC_STAGE2: rc[ORC_ACC2],
-            _lib.CNT_OUT_OF_BOUNDS: rc[ORC_OOB], _lib.CNT_ADAPTATIONS: rc[ORC_ADAPT], _lib.CNT_CHOL_FAIL: rc[ORC_CHOL_FAIL],
-            _lib.CNT_DR_TRIES: int(np.sum((ref["flags"] & _lib.FL_DR) != 0)), _lib.CNT_STATUS: 0}
-    got = {k: int(cnt[k]) for k in want}
-    assert got == {k: int(v) for k, v in want.items()}, (tag, i, got, want)
-
-
-def _check_recorded_ss(cells, cc, out, ld):
-    """The SS the sampler recorded for every stored row (n_burn = 1: row r of the chain is step r) is tc_ss_batch's."""
-    nsimu = out["sschain"].shape[1]
-    rows = out["chain"].reshape(-1, ld)
-    ss = cells.ss_batch(np.repeat(cc, nsimu), rows)
-    ref = out["sschain"].reshape(-1)
-    rel = np.abs(ss - ref) / np.abs(ref)
-    assert rel.max() <= 1e-14, rel.max()
 
 
 # ------------------------------------------------------------------------------------------------ 1. schedule replays
@@ -120,27 +68,19 @@ def _sid(s):
     return "n%d-b%d-a%d%s" % (n, b, m, "".join("-" + k for k in sorted(x)))
 
 
-def _replay_streams(cells, cc, nsimu, ld, seed):
-    g = np.random.default_rng(seed)
-    st = dict(z1=g.standard_normal((cc.size, nsimu, ld)), u1=g.random((cc.size, nsimu)),
-              z2=g.standard_normal((cc.size, nsimu, ld)), u2=g.random((cc.size, nsimu)),
-              chi2=np.stack([g.chisquare(1 + 2 * int(cells.N[c]), nsimu) for c in cc]))
-    return st, [{k: v[i] for k, v in st.items()} for i in range(cc.size)]
-
-
 def _replay_all_layouts(orc, cells, packed, cc, ins, nsimu, burn, adaptint, dev_kw, orc_kw, seed, extra_check=None):
-    _lib = _lib_or_skip()
+    _lib = need_gpu()
     co, _ = orc
     ld = cells.ld
-    st, per = _replay_streams(cells, cc, nsimu, ld, seed)
-    refs = _oracles(orc, cells, packed, cc, co.default_opts(nsimu, burn, adaptint=adaptint, **orc_kw), ins, per)
+    st = replay_streams(cells.N[cc], nsimu, ld, seed)
+    refs = oracle_chains(orc, packed, cc, co.default_opts(nsimu, burn, adaptint=adaptint, **orc_kw), ins, st)
     for layout, name in LAYOUTS:
         opts = _lib.default_opts(nsimu=nsimu, burnintime=burn, adaptint=adaptint, n_burn=1, store_chain=1, replay=1,
                                  layout=layout, **dev_kw)
         out = cells.mcmc_run(opts, cc, *ins, replay=st, want_flags=True)
         for i, ref in enumerate(refs):
-            _check_chain(_lib, name, out, i, ref, 7 + int(cells.N[cc[i]]))
-        _check_recorded_ss(cells, cc, out, ld)
+            check_chain(name, out, i, ref, 7 + int(cells.N[cc[i]]))
+        check_recorded_ss(cells, cc, out, ld)
         if extra_check is not None:
             extra_check(name, out, refs)
     return refs
@@ -150,7 +90,7 @@ def _replay_all_layouts(orc, cells, packed, cc, ins, nsimu, burn, adaptint, dev_
 def test_schedule_replay(orc, two_cells, sched):
     """Four chains (two per cell) replayed with injected randomness and qcovadj_always = 1 on every layout: flags, rows,
     s2chain, sschain, the seven counters, and the recorded SS of every row."""
-    _lib = _lib_or_skip()
+    _lib = need_gpu()
     nsimu, burn, adaptint, extra = sched
     cells, packed = two_cells
     cc = np.array([0, 1, 0, 1], dtype=np.int32)
@@ -186,22 +126,6 @@ def test_frozen_chain_every_factorisation_fails(orc, two_cells):
 
 
 # ------------------------------------------------------------------------------------------------ 2. n_burn and Philox
-def _dumped_streams(_lib, cells, cc, uid, seed, nsimu):
-    per = []
-    for i, c in enumerate(cc):
-        N = int(cells.N[c])
-        per.append(_lib.rng_dump(seed, int(uid[i]), 7 + N, 1 + 2 * N, nsimu))
-    return per
-
-
-def _ld_mean_std(x):
-    """Long-double two-pass mean and population std of the columns of x."""
-    xl = x.astype(np.longdouble)
-    m = xl.sum(axis=0) / x.shape[0]
-    d = xl - m
-    return m, np.sqrt((d * d).sum(axis=0) / x.shape[0])
-
-
 @pytest.mark.parametrize("layout,name", LAYOUTS, ids=[n for _, n in LAYOUTS])
 def test_n_burn_sweep_against_oracle(orc, two_cells, layout, name):
     """One production (Philox) run of nsimu = 100, adaptint = 3, burn-in 30: slices of a few steps on both kernels.  It is the
@@ -209,7 +133,7 @@ def test_n_burn_sweep_against_oracle(orc, two_cells, layout, name):
     leaves flags, s2chain, sig and the counters alone, and reports the mean / population std of those rows (long-double
     two-pass: mean within 1e-13 max|x|, std within 1e-10 relative + 1e-13 max|x|).  Chains 2 and 3 have v confined to
     v0 +- 1e-5 (loadPrevious), so their std / |mean| is ~1e-6."""
-    _lib = _lib_or_skip()
+    _lib = need_gpu()
     co, _ = orc
     cells, packed = two_cells
     cc = np.array([0, 1, 0, 1], dtype=np.int32)
@@ -218,10 +142,10 @@ def test_n_burn_sweep_against_oracle(orc, two_cells, layout, name):
     nsimu, burn, adaptint, seed = 100, 30, 3, 777
     kw = dict(nsimu=nsimu, burnintime=burn, adaptint=adaptint, store_chain=1, seed=seed, layout=layout, qcovadj_always=1)
     base = cells.mcmc_run(_lib.default_opts(n_burn=1, **kw), cc, *ins, chain_uid=uid, want_flags=True)
-    refs = _oracles(orc, cells, packed, cc, co.default_opts(nsimu, burn, adaptint=adaptint, qcovadj_always=1), ins,
-                    _dumped_streams(_lib, cells, cc, uid, seed, nsimu))
+    refs = oracle_chains(orc, packed, cc, co.default_opts(nsimu, burn, adaptint=adaptint, qcovadj_always=1), ins,
+                         dumped_streams(cells.N[cc], uid, seed, nsimu))
     for i, ref in enumerate(refs):
-        _check_chain(_lib, name, base, i, ref, 7 + int(cells.N[cc[i]]))
+        check_chain(name, base, i, ref, 7 + int(cells.N[cc[i]]))
     worst = [0.0, 0.0]
     for nb in range(1, nsimu + 1):
         out = cells.mcmc_run(_lib.default_opts(n_burn=nb, **kw), cc, *ins, chain_uid=uid, want_flags=True)
@@ -232,7 +156,7 @@ def test_n_burn_sweep_against_oracle(orc, two_cells, layout, name):
         for i, c in enumerate(cc):
             npar = 7 + int(cells.N[c])
             rows = base["chain"][i, nb - 1:, :npar]
-            m, s = _ld_mean_std(rows)
+            m, s = ld_mean_std(rows)
             scale = np.abs(rows).max(axis=0)
             em = np.abs(out["mean"][i, :npar] - m).astype(np.float64)
             es = np.abs(out["std"][i, :npar] - s).astype(np.float64)
@@ -253,7 +177,7 @@ def test_production_schedule_against_oracle(orc, two_cells, sched):
     """The production path generates 8 steps per batch on both kernels (dram_warp_kernel's replay batch is 4): schedules of
     section 1 on the device's Philox streams, every layout, against the oracle on tc_rng_dump's streams, with n_burn = 1
     and n_burn in the middle of a slice."""
-    _lib = _lib_or_skip()
+    _lib = need_gpu()
     co, _ = orc
     nsimu, burn, adaptint = sched
     cells, packed = two_cells
@@ -261,8 +185,8 @@ def test_production_schedule_against_oracle(orc, two_cells, sched):
     uid = np.array([5, 6, 7, 8], dtype=np.uint64) + np.uint64(nsimu * 1000 + adaptint)
     ins = _inputs(cells, cc, 40 + nsimu)
     seed = 31337
-    refs = _oracles(orc, cells, packed, cc, co.default_opts(nsimu, burn, adaptint=adaptint, qcovadj_always=1), ins,
-                    _dumped_streams(_lib, cells, cc, uid, seed, nsimu))
+    refs = oracle_chains(orc, packed, cc, co.default_opts(nsimu, burn, adaptint=adaptint, qcovadj_always=1), ins,
+                         dumped_streams(cells.N[cc], uid, seed, nsimu))
     nb = max(1, (2 * nsimu) // 3 + 1)
     for layout, name in LAYOUTS:
         for n_burn in sorted({1, nb}):
@@ -270,36 +194,17 @@ def test_production_schedule_against_oracle(orc, two_cells, sched):
                                      seed=seed, layout=layout, qcovadj_always=1)
             out = cells.mcmc_run(opts, cc, *ins, chain_uid=uid, want_flags=True)
             for i, ref in enumerate(refs):
-                _check_chain(_lib, "%s n_burn=%d" % (name, n_burn), out, i, ref, 7 + int(cells.N[cc[i]]), first_row=n_burn - 1)
+                check_chain("%s n_burn=%d" % (name, n_burn), out, i, ref, 7 + int(cells.N[cc[i]]), first_row=n_burn - 1)
 
 
 # ------------------------------------------------------------------------------------------------ 3. ss(theta0) not finite
-def _raw_run(cells, opts, cc, ins, uid):
-    """tc_mcmc_run through ctypes: (return code, message, outputs) — Cells.mcmc_run raises on TC_ESTATE and drops them."""
-    _lib = _lib_or_skip()
-    nch, ld = cc.size, cells.ld
-    arrs = [_lib.f64(x) for x in ins]
-    out = dict(mean=np.zeros((nch, ld)), std=np.zeros((nch, ld)), sig=np.zeros((nch, 2)),
-               counters=np.zeros((nch, _lib.NCOUNTERS), dtype=np.int64), chain=np.zeros((nch, opts.nsimu - opts.n_burn + 1, ld)),
-               s2chain=np.zeros((nch, opts.nsimu)), flags=np.zeros((nch, opts.nsimu), dtype=np.int32),
-               sschain=np.zeros((nch, opts.nsimu)))
-    rp = _lib.Replay()
-    rp.flags = out["flags"].ctypes.data
-    rp.sschain = out["sschain"].ctypes.data
-    L = _lib.load()
-    rc = L.tc_mcmc_run(cells._h, C.byref(opts), nch, _lib.ptr(_lib.i32(cc)), _lib.ptr(np.ascontiguousarray(uid, dtype=np.uint64)),
-                       ld, *[_lib.ptr(x) for x in arrs], _lib.ptr(out["mean"]), _lib.ptr(out["std"]), _lib.ptr(out["sig"]),
-                       _lib.ptr(out["counters"]), _lib.ptr(out["chain"]), _lib.ptr(out["s2chain"]), C.byref(rp))
-    return rc, L.tc_last_error().decode(), out
-
-
 @pytest.mark.parametrize("layout,name", LAYOUTS, ids=[n for _, n in LAYOUTS])
 def test_nonfinite_ss0_chain_inside_a_group(orc, two_cells, layout, name):
     """Chain 7 of 16 (the middle of one chain-per-warp group) starts at A = 1e200 (upp = 1e300, flat prior on A): its squared
     residual overflows, so ss(theta0) = inf (checked with the oracle).  Over 32 time slices the call returns TC_ESTATE naming
     that chain, the chain reports zeros and status 1, and every other chain's outputs are bit-identical to a run of the
     other 15 chains alone with the same chain_uids."""
-    _lib = _lib_or_skip()
+    _lib = need_gpu()
     co, cons = orc
     cells, packed = two_cells
     bad = 7
@@ -311,12 +216,12 @@ def test_nonfinite_ss0_chain_inside_a_group(orc, two_cells, layout, name):
     c = int(cc[bad]); N = int(cells.N[c]); o = int(cells.off[c])
     assert co.ss(cons, packed["t"][o:o + N], packed["ms2"][o:o + N], packed["pp7"][o:o + N], ins[0][bad, :7 + N]) == np.inf
     opts = _lib.default_opts(nsimu=3200, burnintime=1000, n_burn=1000, store_chain=1, seed=99, layout=layout, qcovadj_always=1)
-    rc, msg, out = _raw_run(cells, opts, cc, ins, uid)
+    rc, msg, out = raw_run(cells, opts, cc, ins, uid)
     assert rc == _lib.TC_ESTATE and ("chain %d" % bad) in msg, (rc, msg)
     assert np.all(out["mean"][bad] == 0) and np.all(out["std"][bad] == 0) and np.all(out["sig"][bad] == 0)
     assert out["counters"][bad, _lib.CNT_STATUS] == 1 and np.all(out["counters"][bad, _lib.CNT_ACC_STAGE1:_lib.CNT_STATUS] == 0), out["counters"][bad]
     keep = np.array([i for i in range(16) if i != bad])
-    rc2, msg2, ref = _raw_run(cells, opts, cc[keep], [x[keep] for x in ins], uid[keep])
+    rc2, msg2, ref = raw_run(cells, opts, cc[keep], [x[keep] for x in ins], uid[keep])
     assert rc2 == 0, msg2
     for k in ("mean", "std", "sig", "chain", "s2chain", "flags", "sschain"):
         assert np.array_equal(out[k][keep], ref[k]), (name, k)
@@ -329,7 +234,7 @@ def test_nonfinite_ss0_chain_inside_a_group(orc, two_cells, layout, name):
 def test_sigma_sigma_is_zero_with_fixed_sigma2(two_cells, sigma2):
     """updatesigma = 0: every row of s2chain is sigma2_0, so std(sqrt(s2chain),1) is 0 and sqrt(mean(s2chain)) is
     sqrt(sigma2_0).  20 000 rows: sig[1] <= 1e-14 sig[0], sig[0] within 1e-11 relative."""
-    _lib = _lib_or_skip()
+    _lib = need_gpu()
     cells, _ = two_cells
     cc = np.array([0, 1], dtype=np.int32)
     ins = _inputs(cells, cc, 600)
@@ -349,7 +254,7 @@ def test_sigma_sigma_long_run(two_cells, N0):
     """updatesigma = 1, 200 000 rows (s2chain stored, n_burn = nsimu so the chain is one row): sig[1] within 1e-12 relative of
     a long-double two-pass std of sqrt(s2chain), sig[0] of sqrt(mean(s2chain)).  N0 = 1e6 (a prior on sigma2 worth 1e6
     observations) makes s2chain narrow: std / mean of sqrt(s2) ~ 1e-3, where a difference of running moments cancels most."""
-    _lib = _lib_or_skip()
+    _lib = need_gpu()
     cells, _ = two_cells
     cc = np.array([0, 1], dtype=np.int32)
     ins = _inputs(cells, cc, 700)
@@ -360,7 +265,7 @@ def test_sigma_sigma_long_run(two_cells, N0):
         out = cells.mcmc_run(opts, cc, *ins)
         for i in range(cc.size):
             s2 = out["s2chain"][i].astype(np.longdouble)
-            m, s = _ld_mean_std(np.sqrt(s2)[:, None])
+            m, s = ld_mean_std(np.sqrt(s2)[:, None])
             rel1 = float(abs(out["sig"][i, 1] - s[0]) / s[0])
             rel0 = float(abs(out["sig"][i, 0] - np.sqrt(s2.mean())) / np.sqrt(s2.mean()))
             print("%s N0 = %g chain %d: sig[1] = %.17g, reference %.17g, rel err %.3g; sig[0] rel err %.3g" % (name, N0, i, out["sig"][i, 1], float(s[0]), rel1, rel0))

@@ -12,6 +12,7 @@ from . import build as _build
 
 MAX_SETS = 8
 MAX_GPUS = 8
+TC_EINVAL = -1        # bad argument (the message says which)
 TC_EDIM = -4          # numel(t(1):dt:t(end)) != numel(t)
 TC_ESTATE = -6        # ss(theta0) not finite for a chain
 NCOUNTERS = 16
@@ -20,6 +21,7 @@ CNT_SS_EVALS, CNT_ACC_STAGE1, CNT_ACC_STAGE2, CNT_OUT_OF_BOUNDS = 0, 1, 2, 3
 CNT_ADAPTATIONS, CNT_CHOL_FAIL, CNT_DR_TRIES, CNT_STATUS = 4, 5, 6, 7
 CNT_CYCLES0 = 8       # + 0..7: per-phase clock readings (include/tcmcmc.h)
 FL_ACCEPT, FL_STAGE2, FL_OOB1, FL_DR, FL_OOB2 = 1, 2, 4, 8, 16
+LAYOUT_AUTO, LAYOUT_BIG, LAYOUT_WARP, LAYOUT_CTA = 0, 1, 2, 3   # tc_mcmc_opts.layout (TC_LAYOUT_*)
 
 EXPORTS = [
     "tc_version", "tc_last_error", "tc_device_count", "tc_device_info_get", "tc_opts_default",
