@@ -93,14 +93,21 @@ typedef struct tc_mcmc_opts {
     double N0;                /* 1 */
     double S20;               /* sigma2_0 */
     double sigma2_0;          /* model.sigma2 = 1 (:212,259) */
-    uint64_t seed;            /* Philox key; draws are addressed by (seed, chain_uid, step, slot) so
-                                 results do not depend on the GPU count */
+    uint64_t seed;            /* Philox key; draws are addressed by (seed, chain_uid, step, slot), never by device or place in
+                                 the launch, so for a given sampler the results are bit-identical for every GPU count and
+                                 partition.  Under TC_LAYOUT_AUTO the sampler is chosen per device (see layout) */
     int32_t layout;           /* TC_LAYOUT_AUTO (0): one CTA per chain (speculative rounds) for up to a few chains per SM, one
                                  WARP per chain beyond that (thousands of chains: BASELINE config 3), the large-series
                                  layout for series with more than ~210 points.  TC_LAYOUT_BIG forces the large-series layout
                                  (ring of 8 proposal slots, proposal factor factorised through HBM/L2), TC_LAYOUT_WARP the
-                                 chain-per-warp kernel, TC_LAYOUT_CTA the CTA-per-chain kernel whatever the chain count.  Same
-                                 chain whichever runs (parity tests) */
+                                 chain-per-warp kernel, TC_LAYOUT_CTA the CTA-per-chain kernel whatever the chain count.  The
+                                 same chain whichever runs, to rounding: the kernels factor the covariance in different
+                                 orders (DESIGN.md 2), so flags and counters agree, means to about 1e-9 after 1 000 steps
+                                 (up to 1e-3 on near-singular covariances at qcovadj_always = 0), not bit for bit.  AUTO
+                                 picks the chain-per-warp kernel from 13 chains per SM on, counted per DEVICE: with ngpus > 1 and 13 S <= nchains < 13 S ngpus
+                                 (S SMs per device) one GPU runs it and several run the CTA-per-chain kernel, so there the
+                                 GPU count changes the last bits of the output.  Force TC_LAYOUT_WARP or TC_LAYOUT_CTA for
+                                 results bit-identical across GPU counts at every chain count */
     int32_t qcovadj_always;   /* 0 (default): R = chol(cov), and chol(cov + qcovadj I) only when that fails — mcmcstat's
                                  "try to blow it" branch [U]; 1: always factor cov + qcovadj I */
 } tc_mcmc_opts;

@@ -122,7 +122,10 @@ def test_multiple_chains_per_cell_pool_and_diagnose(tmp_path, cells_npz):
 def test_two_gpus_same_result_as_one(cells_npz):
     """numParPools = 2 -> two GPUs inside one process (tc_mcmc_opts.ngpus = 2: chains partitioned by cumulative N^2, one
     stream and one drain thread per device): bit-identical to the one-GPU fit, raw chains included (Philox is keyed by chain
-    identity, never by device).  Skipped on a box with fewer than two devices."""
+    identity, never by device).  That holds for a given sampler: 43 chains run dram_kernel on one GPU and on two.  Under
+    TC_LAYOUT_AUTO the sampler is chosen per device, so for 13 S <= nchains < 13 S * ngpus (S SMs per device) one GPU runs
+    dram_warp_kernel and two run dram_kernel, and the fits agree to rounding only (test_gpu_chain_counts.py,
+    DESIGN.md 5).  Skipped on a box with fewer than two devices."""
     from transcriptioncycleinference_b200 import _lib, setup_cell
     from transcriptioncycleinference_b200.engine import Cells
     if _lib.device_count() < 2:
