@@ -57,6 +57,7 @@ struct DeviceGuard {
 #define TC_WARP_MIN_CHAINS_PER_SM 13  // chain-per-warp kernel from this many chains per SM on (measured crossover on B200: ~1 900 chains)
 #define TC_SOLO_LAG 2       // dram_kernel: slices a chain must lag the mean progress by to get its SM to itself (0: never)
 #define TC_SOLO_NSEG 128    // ... and the number of time slices per chain then
+#define TC_UNSLICED_CHAINS (4 * 296)  // dram_kernel from this many chains on: many chains per CTA slot, imbalance averages out, no slicing
 #define COV_CR 32          // weighted rows of the covariance block staged per pass of the scatter update
 
 // development aid: cycle counts of sub-phases, chain 0 only (build with -DTC_SUBPROF; see scripts/subprof.py)
@@ -2512,6 +2513,17 @@ static const DevCells *find_dev(const tc_cells *c, int device)
     return nullptr;
 }
 
+// ss_stream_kernel stages per warp the cell (a.csz doubles, set here), two theta rows (a.ld2, set here) and the
+// forward-model scratch (a.wsz).  It runs where two of its CTAs, each also holding 1 KB of reserved shared memory, fit one
+// SM: returns its dynamic shared memory per CTA then, else 0.
+static size_t ss_stream_smem(SsArgs &a, int Nmax, int ld, int optin)
+{
+    a.csz = (cell_doubles(Nmax) + 1) & ~1;
+    a.ld2 = (ld + 1) & ~1;
+    const size_t smem = sizeof(double) * (size_t)(a.csz + 2 * a.ld2 + 2 + a.wsz) * SS_WARPS;
+    return 2 * (smem + 1024) <= (size_t)optin + 1024 ? smem : 0;
+}
+
 static int launch_ss(const tc_cells *c, const DevCells *dc, long long nbatch, const int *d_cell, const double *d_theta,
                      int ld, int algo, int raw, double *d_ss, double *d_o1, double *d_o2, int ldo, cudaStream_t st)
 {
@@ -2529,12 +2541,9 @@ static int launch_ss(const tc_cells *c, const DevCells *dc, long long nbatch, co
         // SS only, O(N) algorithm (latency-bound): operands staged in shared memory (ss_stream_kernel) when two CTAs per SM
         // fit.  The pairs algorithm is FP64-pipe-bound and prefers the 32 warps/SM of the global-view kernel (measured:
         // 52.7 M evaluations/s there, 34.2 M with 16 warps/SM here).
-        a.csz = (cell_doubles(c->Nmax) + 1) & ~1;
-        a.ld2 = (ld + 1) & ~1;
-        const size_t smem2 = sizeof(double) * (size_t)(a.csz + 2 * a.ld2 + 2 + a.wsz) * SS_WARPS;
         int optin = 0;
         CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dc->device));
-        if (2 * (smem2 + 1024) <= (size_t)optin + 1024) {
+        if (const size_t smem2 = ss_stream_smem(a, c->Nmax, ld, optin)) {
             CUDA_TRY(cudaFuncSetAttribute(ss_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
             const long long want2 = (nbatch + SS_WARPS - 1) / SS_WARPS;
             const int grid2 = (int)std::min<long long>(want2, (long long)sms * 2);
@@ -2639,8 +2648,123 @@ int tc_forward(const tc_cells *c, int64_t nbatch, const int32_t *cell_id, const 
 }  // extern "C"
 
 // ------------------------------------------------------------------------------------- mcmc run
+// The launch plan of one device's share of a fit: sampler kernel, shared-memory layout and schedule.  Pure functions of
+// the device's numbers decide it, so that the policy is checked on the host (tests/stubs/layout_check.cu).
+struct LaunchPlan {
+    bool warp = false;                    // dram_warp_kernel (one warp per chain), else dram_kernel (one CTA per chain)
+    int big = 0, threads = 0, wsz = 0, grid = 0, seglen = 0, solo_lag = 0;
+    size_t smem = 0, nslots = 0;          // dynamic shared memory per CTA; dram_warp_kernel: chain slots (per-warp gInc, gSc, gW)
+    std::string err;                      // non-empty: max(N) fits no layout the options allow (TC_EINVAL)
+};
+
+// Kernel and layout for nc chains on cells of up to Nmax points, on a device of sms SMs with optin bytes of opt-in shared
+// memory per block; static_cta / static_warp: the static shared memory of dram_kernel / dram_warp_kernel.
+static LaunchPlan plan_layout(int Nmax, int nc, int layout, int sms, int optin, size_t static_cta, size_t static_warp)
+{
+    LaunchPlan p;
+    const int npmax = 7 + Nmax;
+    const size_t avail = (size_t)optin > static_cta ? (size_t)optin - static_cta : 0;
+    // regular layout when the Cholesky workspace fits in one SM's shared memory, else the big one
+    p.big = (sizeof(double) * (size_t)dram_smem_doubles(Nmax, 0) > avail || layout == TC_LAYOUT_BIG) ? 1 : 0;
+    // Many chains per SM: one warp per chain (dram_warp_kernel, tc_warp.cuh) instead of one CTA per chain.  The CTA kernel
+    // buys latency with speculation and wins while there are about as many chains as CTA slots (measured crossover on
+    // B200: ~13 chains per SM); beyond that the warp kernel does no wasted evaluations and no CTA barriers.
+    const size_t smem_w = sizeof(double) * (size_t)wk_region(Nmax) * WK_WARPS;
+    const bool warp_fits = smem_w + static_warp <= (size_t)optin && npmax <= 32 * WK_PIT;
+    if (layout == TC_LAYOUT_WARP && !warp_fits) {
+        p.err = "max(N) = " + std::to_string(Nmax) + " is too large for the chain-per-warp layout";
+        return p;
+    }
+    p.warp = layout == TC_LAYOUT_WARP || (layout == TC_LAYOUT_AUTO && warp_fits && !p.big && nc >= TC_WARP_MIN_CHAINS_PER_SM * sms);   // TC_LAYOUT_CTA / _BIG: never
+    if (p.warp) { p.big = 0; p.threads = WK_THREADS; p.smem = smem_w; return p; }
+    p.wsz = dram_wsz(Nmax, p.big);
+    p.threads = DRAM_THREADS;
+    p.smem = sizeof(double) * (size_t)dram_smem_doubles(Nmax, p.big);
+    // (big layout: gen_increments_tma keeps at most GENB_MAXT column tiles of 8 per warp in registers)
+    if (p.smem > avail || (npmax + 3) / 4 > 255 || (p.big && npmax > 8 * SPEC * GENB_MAXT))
+        p.err = "max(N) = " + std::to_string(Nmax) + " is too large for the shared-memory layout of this build "
+                "(one CTA per chain: the cell, the chain state, 8 proposal slots and 8 forward-model scratch areas must fit in one SM)";
+    return p;
+}
+
+// Grid and time slices of the planned kernel for nc chains of nsimu steps, with per_sm of its CTAs resident per SM;
+// solo_lag and nseg: the solo-SM rule's lag and slices per chain (TC_SOLO_LAG, TC_SOLO_NSEG).
+static void plan_schedule(LaunchPlan &p, int nc, int nsimu, int adaptint, int sms, int per_sm, int solo_lag, int nseg)
+{
+    // time slices: ~32 per chain, each ending on an adaptation step (a slice parks no partial covariance block): a multiple
+    // of adaptint, and of 2 when adaptint = 1 (the first adaptation is at isimu = 2, so k = 1 would split the first block)
+    const int unit = adaptint > 1 ? adaptint : (adaptint == 1 ? 2 : 1);
+    long long sl = ((long long)nsimu + 31) / 32;
+    if (p.warp) {
+        // persistent grid, one item = WK_WARPS consecutive chains.  (More, shorter slices were measured for the one-wave
+        // case — 2 392 chains = 150 groups on 148 SMs — and change nothing: 0.589 s with 29 slices, 0.599 s with 200; what
+        // bounds that case is its slowest group, whose slices are sequential.)
+        p.grid = std::max(1, std::min(per_sm * sms, (nc + WK_WARPS - 1) / WK_WARPS));
+        p.nslots = (size_t)p.grid * WK_WARPS;
+    } else {
+        if (nc >= TC_UNSLICED_CHAINS) sl = nsimu;
+        else if (per_sm == 2 && nc > sms) {
+            // about as many chains as CTA slots, two CTAs per SM: lagging chains get an SM to themselves (dram_kernel's
+            // claim loop); finer slices, so that the neighbour of such a chain gives way soon
+            p.solo_lag = solo_lag;
+            if (solo_lag > 0) sl = std::max<long long>(((long long)nsimu + nseg - 1) / nseg, 4LL * unit);
+        }
+        p.grid = std::min(nc, per_sm * sms);             // persistent grid = resident CTA slots: slices may wait on each other
+    }
+    sl = ((sl + unit - 1) / unit) * unit;
+    p.seglen = (int)std::max<long long>(sl, unit);
+}
+
+// Static partition over ngpus devices, at most one per chain: contiguous blocks of ~equal work (work ~ N^2 per step), none
+// empty.  Device g runs chains [b[g], b[g + 1]).
+static std::vector<int> partition_chains(const std::vector<int> &N, const int32_t *chain_cell, int nchains, int ngpus)
+{
+    ngpus = std::min(ngpus, nchains);
+    std::vector<double> wk(nchains + 1, 0.0);
+    for (int i = 0; i < nchains; ++i) { const double n = N[chain_cell[i]]; wk[i + 1] = wk[i] + n * n; }
+    std::vector<int> b(ngpus + 1, nchains);
+    b[0] = 0;
+    for (int g = 0; g + 1 < ngpus; ++g) {
+        const double target = wk[nchains] * (g + 1) / ngpus;
+        const int end = (int)(std::lower_bound(wk.begin(), wk.end(), target) - wk.begin());
+        b[g + 1] = std::min(std::max(end, b[g] + 1), nchains - (ngpus - 1 - g));
+    }
+    return b;
+}
+
+// does any adaptation with a covariance ever happen?
+static bool cov_adaptations(const tc_mcmc_opts *o)
+{
+    if (o->adaptint > 0)
+        for (long long m = o->adaptint; m <= o->nsimu; m += o->adaptint) if (m >= o->burnintime) return true;
+    return false;
+}
+
+// The dataset's scratch pool on dc's device, created on first use; nullptr where the device has no stream-ordered pools.
+static cudaMemPool_t scratch_pool(const DevCells *dc)
+{
+    int pools = 0;
+    if (!dc->pool && cudaDeviceGetAttribute(&pools, cudaDevAttrMemoryPoolsSupported, dc->device) == cudaSuccess && pools) {
+        cudaMemPoolProps props{};
+        props.allocType = cudaMemAllocationTypePinned;
+        props.handleTypes = cudaMemHandleTypeNone;
+        props.location.type = cudaMemLocationTypeDevice;
+        props.location.id = dc->device;
+        cudaMemPool_t pool = nullptr;
+        if (cudaMemPoolCreate(&pool, &props) == cudaSuccess) {
+            unsigned long long keep = ~0ULL;                  // our own pool: keep the scratch between fits
+            cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
+            dc->pool = pool;
+        } else {
+            (void)cudaGetLastError();
+        }
+    }
+    return dc->pool;
+}
+
 struct DevRun {
     int device = -1, c0 = 0, c1 = 0;      // chains [c0, c1)
+    LaunchPlan plan;
     DevBuf buf;
     cudaStream_t st = nullptr;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
@@ -2661,6 +2785,116 @@ static cudaError_t up(DevBuf &b, T *&d, const T *h, size_t n, cudaStream_t st)
     cudaError_t e = b.alloc(d, n);
     if (e != cudaSuccess) return e;
     return cudaMemcpyAsync(d, h, n * sizeof(T), cudaMemcpyHostToDevice, st);
+}
+
+// params{i} = {name, init, lo, hi, mu, sig} (TranscriptionCycleMCMC.m:242-255): mcmcstat refuses an initial value outside
+// its bounds; a prior width that is zero, negative or NaN would make the prior sum NaN and the chain would never accept
+static int check_params(const tc_cells *c, int nchains, const int32_t *chain_cell, int ld, const double *theta0,
+                        const double *qcov_diag, const double *low, const double *upp, const double *prior_mu,
+                        const double *prior_sig)
+{
+    for (size_t i = 0; i < (size_t)nchains; ++i)
+        for (int p = 0; p < 7 + c->N[chain_cell[i]]; ++p) {
+            const size_t e = i * ld + p;
+            const char *what = nullptr;
+            if (!(qcov_diag[e] > 0)) what = "qcov_diag must be > 0";
+            else if (!(low[e] <= upp[e])) what = "low must be <= upp";
+            else if (!(theta0[e] >= low[e] && theta0[e] <= upp[e])) what = "theta0 must lie inside [low, upp]";
+            else if (!(prior_sig[e] > 0)) what = "prior_sig must be > 0 (Inf = flat)";
+            else if (std::isnan(prior_mu[e])) what = "prior_mu is NaN";
+            if (what) return fail(TC_EINVAL, std::string(what) + " (chain " + std::to_string(i) + ", parameter " + std::to_string(p) + ")");
+        }
+    return TC_OK;
+}
+
+// One device's share of a fit, chains [r.c0, r.c1): its stream, events and scratch pool, RunArgs from the options and
+// r.plan, the chains' inputs uploaded, outputs and scratch allocated.
+static int setup_run(DevRun &r, const tc_cells *c, const tc_mcmc_opts *o, int ld, const int32_t *chain_cell,
+                     const uint64_t *chain_uid, const double *theta0, const double *qcov_diag, const double *low,
+                     const double *upp, const double *prior_mu, const double *prior_sig, const tc_replay *rp)
+{
+    const int nc = r.c1 - r.c0, Nmax = c->Nmax, nstore = o->nsimu - (o->n_burn - 1);
+    const size_t o0 = (size_t)r.c0;
+    const int ldR = tri_doubles(7 + Nmax);               // proposal factor / scatter matrix in 4x4 tiles (chol_tiled)
+    const bool do_cov = cov_adaptations(o);
+    const LaunchPlan &p = r.plan;
+    const DevCells *dc = find_dev(c, r.device);
+    CUDA_TRY(cudaSetDevice(r.device));
+    CUDA_TRY(cudaStreamCreateWithFlags(&r.st, cudaStreamNonBlocking));
+    if (cudaMemPool_t pool = scratch_pool(dc)) { r.buf.st = r.st; r.buf.pool = pool; r.buf.pooled = true; }
+    CUDA_TRY(cudaEventCreate(&r.e0));
+    CUDA_TRY(cudaEventCreate(&r.e1));
+    RunArgs &a = r.a;
+    a.cells = dc->d; a.cons = make_consx(c->cons);
+    a.nsimu = o->nsimu; a.burnintime = o->burnintime; a.adaptint = o->adaptint; a.ntry = o->ntry;
+    a.updatesigma = o->updatesigma; a.burnin_cumulative = o->burnin_cumulative; a.n_burn = o->n_burn;
+    a.store_chain = o->store_chain; a.replay = o->replay; a.algo = o->algo; a.qcovadj_always = o->qcovadj_always;
+    a.drscale = o->drscale; a.adascale = o->adascale; a.qcovadj = o->qcovadj; a.burnin_scale = o->burnin_scale;
+    a.N0 = o->N0; a.S20 = o->S20; a.sigma2_0 = o->sigma2_0; a.seed = o->seed;
+    a.nchains = nc; a.ld = ld; a.nmax = Nmax; a.ldR = ldR; a.do_cov = do_cov ? 1 : 0;
+    a.big = p.big; a.wsz = p.wsz; a.seglen = p.seglen; a.solo_lag = p.solo_lag;
+    // the first block is rows 0 .. isimu-1 of the first adaptation (row 0 is x0, no step): with adaptint = 1 that is 2 rows
+    a.blk_rows = std::max(o->adaptint, 2);
+    int *d_cell; unsigned long long *d_uid; double *d;
+    CUDA_TRY(up(r.buf, d_cell, (const int *)chain_cell + o0, nc, r.st)); a.chain_cell = d_cell;
+    std::vector<unsigned long long> uid(nc);
+    for (int i = 0; i < nc; ++i) uid[i] = chain_uid ? chain_uid[o0 + i] : (unsigned long long)(o0 + i);
+    CUDA_TRY(r.buf.alloc(d_uid, nc));
+    CUDA_TRY(cudaMemcpyAsync(d_uid, uid.data(), nc * sizeof(unsigned long long), cudaMemcpyHostToDevice, r.st)); a.chain_uid = d_uid;   // pageable source: staged before the call returns
+    CUDA_TRY(up(r.buf, d, theta0 + o0 * ld, (size_t)nc * ld, r.st)); a.theta0 = d;
+    CUDA_TRY(up(r.buf, d, qcov_diag + o0 * ld, (size_t)nc * ld, r.st)); a.qcov_diag = d;
+    CUDA_TRY(up(r.buf, d, low + o0 * ld, (size_t)nc * ld, r.st)); a.low = d;
+    CUDA_TRY(up(r.buf, d, upp + o0 * ld, (size_t)nc * ld, r.st)); a.upp = d;
+    CUDA_TRY(up(r.buf, d, prior_mu + o0 * ld, (size_t)nc * ld, r.st)); a.pmu = d;
+    CUDA_TRY(up(r.buf, d, prior_sig + o0 * ld, (size_t)nc * ld, r.st)); a.psig = d;
+    CUDA_TRY(r.buf.alloc(a.mean, (size_t)nc * ld)); CUDA_TRY(cudaMemsetAsync(a.mean, 0, (size_t)nc * ld * 8, r.st));
+    CUDA_TRY(r.buf.alloc(a.std, (size_t)nc * ld)); CUDA_TRY(cudaMemsetAsync(a.std, 0, (size_t)nc * ld * 8, r.st));
+    CUDA_TRY(r.buf.alloc(a.sig, (size_t)nc * 2));
+    CUDA_TRY(r.buf.alloc(a.counters, (size_t)nc * TC_NCOUNTERS));
+    if (o->store_chain) {
+        CUDA_TRY(r.buf.alloc(a.chain, (size_t)nc * nstore * ld));
+        CUDA_TRY(cudaMemsetAsync(a.chain, 0, (size_t)nc * nstore * ld * 8, r.st));
+        CUDA_TRY(r.buf.alloc(a.s2chain, (size_t)nc * o->nsimu));
+        CUDA_TRY(cudaMemsetAsync(a.s2chain, 0, (size_t)nc * o->nsimu * 8, r.st));
+    }
+    if (o->replay) {
+        const size_t nz = (size_t)nc * o->nsimu * ld, nu = (size_t)nc * o->nsimu;
+        CUDA_TRY(up(r.buf, d, rp->z1 + o0 * o->nsimu * ld, nz, r.st)); a.z1 = d;
+        CUDA_TRY(up(r.buf, d, rp->z2 + o0 * o->nsimu * ld, nz, r.st)); a.z2 = d;
+        CUDA_TRY(up(r.buf, d, rp->u1 + o0 * o->nsimu, nu, r.st)); a.u1 = d;
+        CUDA_TRY(up(r.buf, d, rp->u2 + o0 * o->nsimu, nu, r.st)); a.u2 = d;
+        CUDA_TRY(up(r.buf, d, rp->chi2 + o0 * o->nsimu, nu, r.st)); a.chi2 = d;
+    }
+    if (rp && rp->flags) CUDA_TRY(r.buf.alloc(a.flags, (size_t)nc * o->nsimu));
+    if (rp && rp->sschain) CUDA_TRY(r.buf.alloc(a.sschain, (size_t)nc * o->nsimu));
+    // scratch
+    CUDA_TRY(r.buf.alloc(a.gR, (size_t)nc * ldR));
+    if (do_cov) {
+        CUDA_TRY(r.buf.alloc(a.gM2, (size_t)nc * ldR));
+        CUDA_TRY(r.buf.alloc(a.gRows, (size_t)nc * a.blk_rows * ld));
+        CUDA_TRY(r.buf.alloc(a.gWts, (size_t)nc * a.blk_rows));
+        CUDA_TRY(r.buf.alloc(a.gCmean, (size_t)nc * ld));
+    }
+    CUDA_TRY(r.buf.alloc(a.smctl, 1024));
+    CUDA_TRY(cudaMemsetAsync(a.smctl, 0, sizeof(int) * 1024, r.st));
+    CUDA_TRY(r.buf.alloc(a.gState, (size_t)nc * state_doubles(ld)));
+    CUDA_TRY(r.buf.alloc(a.cstate, nc));
+    CUDA_TRY(cudaMemsetAsync(a.cstate, 0, sizeof(int) * nc, r.st));
+    if (p.warp) {
+        const int ldp = wk_ldp(Nmax);
+        CUDA_TRY(r.buf.alloc(a.gPinv, (size_t)nc * ld));
+        CUDA_TRY(r.buf.alloc(a.gInc, p.nslots * 2 * WK_GEN * ldp));
+        CUDA_TRY(r.buf.alloc(a.gSc, p.nslots * 8 * WK_GEN));
+        CUDA_TRY(r.buf.alloc(a.wq, 1));
+        CUDA_TRY(cudaMemsetAsync(a.wq, 0, sizeof(unsigned long long), r.st));
+        if (do_cov) {
+            CUDA_TRY(r.buf.alloc(a.gMb, (size_t)nc * ld));
+            CUDA_TRY(r.buf.alloc(a.gW, p.nslots * ldR));
+        }
+    } else if (p.big && do_cov) {
+        CUDA_TRY(r.buf.alloc(a.gW, (size_t)p.grid * ldR));
+    }
+    return TC_OK;
 }
 
 extern "C" {
@@ -2684,212 +2918,51 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
     if (o->store_chain && (!chain || !s2chain)) return fail(TC_EINVAL, "store_chain set but chain/s2chain is NULL");
     for (int i = 0; i < nchains; ++i)
         if (chain_cell[i] < 0 || chain_cell[i] >= c->ncells) return fail(TC_EINVAL, "chain_cell out of range");
-    // params{i} = {name, init, lo, hi, mu, sig} (TranscriptionCycleMCMC.m:242-255): mcmcstat refuses an initial value outside
-    // its bounds; a prior width that is zero, negative or NaN would make the prior sum NaN and the chain would never accept
-    for (size_t i = 0; i < (size_t)nchains; ++i)
-        for (int p = 0; p < 7 + c->N[chain_cell[i]]; ++p) {
-            const size_t e = i * ld + p;
-            const char *what = nullptr;
-            if (!(qcov_diag[e] > 0)) what = "qcov_diag must be > 0";
-            else if (!(low[e] <= upp[e])) what = "low must be <= upp";
-            else if (!(theta0[e] >= low[e] && theta0[e] <= upp[e])) what = "theta0 must lie inside [low, upp]";
-            else if (!(prior_sig[e] > 0)) what = "prior_sig must be > 0 (Inf = flat)";
-            else if (std::isnan(prior_mu[e])) what = "prior_mu is NaN";
-            if (what) return fail(TC_EINVAL, std::string(what) + " (chain " + std::to_string(i) + ", parameter " + std::to_string(p) + ")");
-        }
+    if (const int rc = check_params(c, nchains, chain_cell, ld, theta0, qcov_diag, low, upp, prior_mu, prior_sig)) return rc;
     DeviceGuard guard;                                    // declared before `runs`: restores the caller's device last
 
     // devices: 'numParPools' => GPU count
-    int ngpus = std::max(1, o->ngpus);
+    const int ngpus = std::max(1, o->ngpus);
     std::vector<int> devs;
     for (int g = 0; g < ngpus; ++g) devs.push_back(o->devices[0] >= 0 ? o->devices[g] : c->dev[std::min<size_t>(g, c->dev.size() - 1)].device);
     if (o->devices[0] < 0 && ngpus > (int)c->dev.size()) return fail(TC_EINVAL, "ngpus exceeds the devices the cells were uploaded to");
     for (int d : devs) if (!find_dev(c, d)) return fail(TC_EINVAL, "cells not resident on a requested device");
-    ngpus = std::min(ngpus, nchains);
+    const std::vector<int> part = partition_chains(c->N, chain_cell, nchains, ngpus);
+    std::vector<DevRun> runs(part.size() - 1);
+    for (size_t g = 0; g < runs.size(); ++g) { runs[g].device = devs[g]; runs[g].c0 = part[g]; runs[g].c1 = part[g + 1]; }
 
-    const int Nmax = c->Nmax, npmax = 7 + Nmax;
-    const int ldR = tri_doubles(npmax);                   // proposal factor / scatter matrix in 4x4 tiles (chol_tiled)
-    // does any adaptation with a covariance ever happen?
-    bool do_cov = false;
-    if (o->adaptint > 0)
-        for (long long m = o->adaptint; m <= o->nsimu; m += o->adaptint) if (m >= o->burnintime) { do_cov = true; break; }
-    const int nstore = o->nsimu - (o->n_burn - 1);
-
-    // static partition: contiguous blocks of ~equal work (work ~ N^2 per step)
-    std::vector<double> wk(nchains + 1, 0.0);
-    for (int i = 0; i < nchains; ++i) { const double n = c->N[chain_cell[i]]; wk[i + 1] = wk[i] + n * n; }
-    std::vector<DevRun> runs(ngpus);
-    int prev = 0;
-    for (int g = 0; g < ngpus; ++g) {
-        int end = nchains;
-        if (g + 1 < ngpus) {
-            const double target = wk[nchains] * (g + 1) / ngpus;
-            end = (int)(std::lower_bound(wk.begin(), wk.end(), target) - wk.begin());
-            end = std::max(end, prev + 1);
-            end = std::min(end, nchains - (ngpus - 1 - g));
-        }
-        runs[g].device = devs[g]; runs[g].c0 = prev; runs[g].c1 = end;
-        prev = end;
-    }
-
+    // every device's plan before any device work: a series length no allowed layout takes is refused here
+    const char *e1 = getenv("TC_SOLO_LAG"), *e2 = getenv("TC_NSEG");          // development switches
+    const int solo_lag = e1 ? atoi(e1) : TC_SOLO_LAG, nseg = e2 ? atoi(e2) : TC_SOLO_NSEG;
     for (auto &r : runs) {
-        const int nc = r.c1 - r.c0;
-        const size_t o0 = (size_t)r.c0;
+        int optin = 0, sms = 0, per_sm = 0;
+        cudaFuncAttributes fa, faw;
         CUDA_TRY(cudaSetDevice(r.device));
-        CUDA_TRY(cudaStreamCreateWithFlags(&r.st, cudaStreamNonBlocking));
-        {
-            const DevCells *dcp = find_dev(c, r.device);
-            int pools = 0;
-            if (!dcp->pool && cudaDeviceGetAttribute(&pools, cudaDevAttrMemoryPoolsSupported, r.device) == cudaSuccess && pools) {
-                cudaMemPoolProps props{};
-                props.allocType = cudaMemAllocationTypePinned;
-                props.handleTypes = cudaMemHandleTypeNone;
-                props.location.type = cudaMemLocationTypeDevice;
-                props.location.id = r.device;
-                cudaMemPool_t pool = nullptr;
-                if (cudaMemPoolCreate(&pool, &props) == cudaSuccess) {
-                    unsigned long long keep = ~0ULL;                  // our own pool: keep the scratch between fits
-                    cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
-                    dcp->pool = pool;
-                } else {
-                    (void)cudaGetLastError();
-                }
-            }
-            if (dcp->pool) { r.buf.st = r.st; r.buf.pool = dcp->pool; r.buf.pooled = true; }
-        }
-        CUDA_TRY(cudaEventCreate(&r.e0));
-        CUDA_TRY(cudaEventCreate(&r.e1));
-        RunArgs &a = r.a;
-        a.cells = find_dev(c, r.device)->d; a.cons = make_consx(c->cons);
-        a.nsimu = o->nsimu; a.burnintime = o->burnintime; a.adaptint = o->adaptint; a.ntry = o->ntry;
-        a.updatesigma = o->updatesigma; a.burnin_cumulative = o->burnin_cumulative; a.n_burn = o->n_burn;
-        a.store_chain = o->store_chain; a.replay = o->replay; a.algo = o->algo; a.qcovadj_always = o->qcovadj_always;
-        a.drscale = o->drscale; a.adascale = o->adascale; a.qcovadj = o->qcovadj; a.burnin_scale = o->burnin_scale;
-        a.N0 = o->N0; a.S20 = o->S20; a.sigma2_0 = o->sigma2_0; a.seed = o->seed;
-        a.nchains = nc; a.ld = ld; a.nmax = Nmax; a.ldR = ldR; a.do_cov = do_cov ? 1 : 0;
-        // the first block is rows 0 .. isimu-1 of the first adaptation (row 0 is x0, no step): with adaptint = 1 that is 2 rows
-        a.blk_rows = std::max(o->adaptint, 2);
-        int *d_cell; unsigned long long *d_uid; double *d;
-        CUDA_TRY(up(r.buf, d_cell, (const int *)chain_cell + o0, nc, r.st)); a.chain_cell = d_cell;
-        std::vector<unsigned long long> uid(nc);
-        for (int i = 0; i < nc; ++i) uid[i] = chain_uid ? chain_uid[o0 + i] : (unsigned long long)(o0 + i);
-        CUDA_TRY(r.buf.alloc(d_uid, nc));
-        CUDA_TRY(cudaMemcpyAsync(d_uid, uid.data(), nc * sizeof(unsigned long long), cudaMemcpyHostToDevice, r.st)); a.chain_uid = d_uid;   // pageable source: staged before the call returns
-        CUDA_TRY(up(r.buf, d, theta0 + o0 * ld, (size_t)nc * ld, r.st)); a.theta0 = d;
-        CUDA_TRY(up(r.buf, d, qcov_diag + o0 * ld, (size_t)nc * ld, r.st)); a.qcov_diag = d;
-        CUDA_TRY(up(r.buf, d, low + o0 * ld, (size_t)nc * ld, r.st)); a.low = d;
-        CUDA_TRY(up(r.buf, d, upp + o0 * ld, (size_t)nc * ld, r.st)); a.upp = d;
-        CUDA_TRY(up(r.buf, d, prior_mu + o0 * ld, (size_t)nc * ld, r.st)); a.pmu = d;
-        CUDA_TRY(up(r.buf, d, prior_sig + o0 * ld, (size_t)nc * ld, r.st)); a.psig = d;
-        CUDA_TRY(r.buf.alloc(a.mean, (size_t)nc * ld)); CUDA_TRY(cudaMemsetAsync(a.mean, 0, (size_t)nc * ld * 8, r.st));
-        CUDA_TRY(r.buf.alloc(a.std, (size_t)nc * ld)); CUDA_TRY(cudaMemsetAsync(a.std, 0, (size_t)nc * ld * 8, r.st));
-        CUDA_TRY(r.buf.alloc(a.sig, (size_t)nc * 2));
-        CUDA_TRY(r.buf.alloc(a.counters, (size_t)nc * TC_NCOUNTERS));
-        if (o->store_chain) {
-            CUDA_TRY(r.buf.alloc(a.chain, (size_t)nc * nstore * ld));
-            CUDA_TRY(cudaMemsetAsync(a.chain, 0, (size_t)nc * nstore * ld * 8, r.st));
-            CUDA_TRY(r.buf.alloc(a.s2chain, (size_t)nc * o->nsimu));
-            CUDA_TRY(cudaMemsetAsync(a.s2chain, 0, (size_t)nc * o->nsimu * 8, r.st));
-        }
-        if (o->replay) {
-            const size_t nz = (size_t)nc * o->nsimu * ld, nu = (size_t)nc * o->nsimu;
-            CUDA_TRY(up(r.buf, d, rp->z1 + o0 * o->nsimu * ld, nz, r.st)); a.z1 = d;
-            CUDA_TRY(up(r.buf, d, rp->z2 + o0 * o->nsimu * ld, nz, r.st)); a.z2 = d;
-            CUDA_TRY(up(r.buf, d, rp->u1 + o0 * o->nsimu, nu, r.st)); a.u1 = d;
-            CUDA_TRY(up(r.buf, d, rp->u2 + o0 * o->nsimu, nu, r.st)); a.u2 = d;
-            CUDA_TRY(up(r.buf, d, rp->chi2 + o0 * o->nsimu, nu, r.st)); a.chi2 = d;
-        }
-        if (rp && rp->flags) CUDA_TRY(r.buf.alloc(a.flags, (size_t)nc * o->nsimu));
-        if (rp && rp->sschain) CUDA_TRY(r.buf.alloc(a.sschain, (size_t)nc * o->nsimu));
-        // scratch
-        CUDA_TRY(r.buf.alloc(a.gR, (size_t)nc * ldR));
-        if (do_cov) {
-            CUDA_TRY(r.buf.alloc(a.gM2, (size_t)nc * ldR));
-            CUDA_TRY(r.buf.alloc(a.gRows, (size_t)nc * a.blk_rows * ld));
-            CUDA_TRY(r.buf.alloc(a.gWts, (size_t)nc * a.blk_rows));
-            CUDA_TRY(r.buf.alloc(a.gCmean, (size_t)nc * ld));
-        }
-        int optin = 0, sms = 0;
         CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, r.device));
         CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, r.device));
-        cudaFuncAttributes fa;
         CUDA_TRY(cudaFuncGetAttributes(&fa, dram_kernel));
-        const size_t avail = (size_t)optin > fa.sharedSizeBytes ? (size_t)optin - fa.sharedSizeBytes : 0;
-        // regular layout when the Cholesky workspace fits in one SM's shared memory, else the big one
-        a.big = (sizeof(double) * (size_t)dram_smem_doubles(Nmax, 0) > avail || o->layout == TC_LAYOUT_BIG) ? 1 : 0;
-        // Many chains per SM: one warp per chain (dram_warp_kernel, tc_warp.cuh) instead of one CTA per chain.  The CTA kernel
-        // buys latency with speculation and wins while there are about as many chains as CTA slots (measured crossover on
-        // B200: ~13 chains per SM); beyond that the warp kernel does no wasted evaluations and no CTA barriers.
-        cudaFuncAttributes faw;
         CUDA_TRY(cudaFuncGetAttributes(&faw, dram_warp_kernel));
-        const size_t smem_w = sizeof(double) * (size_t)wk_region(Nmax) * WK_WARPS;
-        const bool warp_fits = smem_w + faw.sharedSizeBytes <= (size_t)optin && npmax <= 32 * WK_PIT;
-        if (o->layout == TC_LAYOUT_WARP && !warp_fits)
-            return fail(TC_EINVAL, "max(N) = " + std::to_string(Nmax) + " is too large for the chain-per-warp layout");
-        const bool use_warp = o->layout == TC_LAYOUT_WARP || (o->layout == TC_LAYOUT_AUTO && warp_fits && !a.big && nc >= TC_WARP_MIN_CHAINS_PER_SM * sms);   // TC_LAYOUT_CTA / _BIG: never
-        // time slices: ~32 per chain, each ending on an adaptation step (a slice parks no partial covariance block): a multiple
-        // of adaptint, and of 2 when adaptint = 1 (the first adaptation is at isimu = 2, so k = 1 would split the first block)
-        const int unit = o->adaptint > 1 ? o->adaptint : (o->adaptint == 1 ? 2 : 1);
-        long long sl = ((long long)o->nsimu + 31) / 32;
-        CUDA_TRY(r.buf.alloc(a.smctl, 1024));
-        CUDA_TRY(cudaMemsetAsync(a.smctl, 0, sizeof(int) * 1024, r.st));
-        a.solo_lag = 0;
-        CUDA_TRY(r.buf.alloc(a.gState, (size_t)nc * state_doubles(ld)));
-        CUDA_TRY(r.buf.alloc(a.cstate, nc));
-        CUDA_TRY(cudaMemsetAsync(a.cstate, 0, sizeof(int) * nc, r.st));
-        if (use_warp) a.big = 0;
-        else a.wsz = dram_wsz(Nmax, a.big);
-        const auto kernel = use_warp ? dram_warp_kernel : dram_kernel;
-        const int threads = use_warp ? WK_THREADS : DRAM_THREADS;
-        const size_t smem = use_warp ? smem_w : sizeof(double) * (size_t)dram_smem_doubles(Nmax, a.big);
-        // (big layout: gen_increments_tma keeps at most GENB_MAXT column tiles of 8 per warp in registers)
-        if (!use_warp && (smem > avail || (npmax + 3) / 4 > 255 || (a.big && npmax > 8 * SPEC * GENB_MAXT)))
-            return fail(TC_EINVAL, "max(N) = " + std::to_string(Nmax) + " is too large for the shared-memory layout of this build "
-                                   "(one CTA per chain: the cell, the chain state, 8 proposal slots and 8 forward-model scratch areas must fit in one SM)");
-        CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        int per_sm = 0;
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
-        if (per_sm < 1) return fail(TC_EINVAL, use_warp ? "chain-per-warp kernel does not fit on this device" : "sampler kernel does not fit on this device");
-        int grid;
-        if (use_warp) {
-            // persistent grid, one item = WK_WARPS consecutive chains.  (More, shorter slices were measured for the one-wave
-            // case — 2 392 chains = 150 groups on 148 SMs — and change nothing: 0.589 s with 29 slices, 0.599 s with 200; what
-            // bounds that case is its slowest group, whose slices are sequential.)
-            grid = std::max(1, std::min(per_sm * sms, (nc + WK_WARPS - 1) / WK_WARPS));
-            const size_t nslots = (size_t)grid * WK_WARPS;
-            const int ldp = wk_ldp(Nmax);
-            CUDA_TRY(r.buf.alloc(a.gPinv, (size_t)nc * ld));
-            CUDA_TRY(r.buf.alloc(a.gInc, nslots * 2 * WK_GEN * ldp));
-            CUDA_TRY(r.buf.alloc(a.gSc, nslots * 8 * WK_GEN));
-            CUDA_TRY(r.buf.alloc(a.wq, 1));
-            CUDA_TRY(cudaMemsetAsync(a.wq, 0, sizeof(unsigned long long), r.st));
-            if (do_cov) {
-                CUDA_TRY(r.buf.alloc(a.gMb, (size_t)nc * ld));
-                CUDA_TRY(r.buf.alloc(a.gW, nslots * ldR));
-            }
-        } else {
-            if (nc >= 4 * 296) sl = o->nsimu;             // many chains per CTA slot: imbalance averages out, no slicing
-            else if (per_sm == 2 && nc > sms) {
-                // about as many chains as CTA slots, two CTAs per SM: lagging chains get an SM to themselves (dram_kernel's
-                // claim loop); finer slices, so that the neighbour of such a chain gives way soon
-                const char *e1 = getenv("TC_SOLO_LAG"), *e2 = getenv("TC_NSEG");          // development switches
-                a.solo_lag = e1 ? atoi(e1) : TC_SOLO_LAG;
-                const int ns = e2 ? atoi(e2) : TC_SOLO_NSEG;
-                if (a.solo_lag > 0) sl = std::max<long long>(((long long)o->nsimu + ns - 1) / ns, 4LL * unit);
-            }
-            grid = std::min(nc, per_sm * sms);             // persistent grid = resident CTA slots: slices may wait on each other
-            if (a.big && do_cov) CUDA_TRY(r.buf.alloc(a.gW, (size_t)grid * ldR));
-        }
-        sl = ((sl + unit - 1) / unit) * unit;
-        a.seglen = (int)std::max<long long>(sl, unit);
+        LaunchPlan &p = r.plan = plan_layout(c->Nmax, r.c1 - r.c0, o->layout, sms, optin, fa.sharedSizeBytes, faw.sharedSizeBytes);
+        if (!p.err.empty()) return fail(TC_EINVAL, p.err);
+        const auto kernel = p.warp ? dram_warp_kernel : dram_kernel;
+        CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, p.threads, p.smem));
+        if (per_sm < 1) return fail(TC_EINVAL, p.warp ? "chain-per-warp kernel does not fit on this device" : "sampler kernel does not fit on this device");
+        plan_schedule(p, r.c1 - r.c0, o->nsimu, o->adaptint, sms, per_sm, solo_lag, nseg);
+    }
+    for (auto &r : runs) {
+        const int rc = setup_run(r, c, o, ld, chain_cell, chain_uid, theta0, qcov_diag, low, upp, prior_mu, prior_sig, rp);
+        if (rc) return rc;
+        const auto kernel = r.plan.warp ? dram_warp_kernel : dram_kernel;
         CUDA_TRY(cudaEventRecord(r.e0, r.st));
-        kernel<<<grid, threads, smem, r.st>>>(a);
+        kernel<<<r.plan.grid, r.plan.threads, r.plan.smem, r.st>>>(r.a);
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaEventRecord(r.e1, r.st));
     }
     // Drain: every device's outputs go back on its own stream; with several devices one host thread per device, so the
     // device -> host copies (raw chains: GBs) of the 8 GPUs overlap instead of queueing behind each other.
     const auto t_drain0 = std::chrono::steady_clock::now();
+    const int nstore = o->nsimu - (o->n_burn - 1);
     std::vector<int64_t> cnt_tmp;
     if (!counters) { cnt_tmp.assign((size_t)nchains * TC_NCOUNTERS, 0); counters = cnt_tmp.data(); }   // TC_CNT_STATUS is always checked
     std::vector<double> ksec(runs.size(), 0.0);
