@@ -283,6 +283,60 @@ __device__ __forceinline__ bool chol8(double (&A)[8][8], double (&dinv)[8])
 // two Newton steps) and the reciprocal square roots are side chains: -2 % on the factorisation of dram_kernel, +4 % on the
 // chain-per-warp kernel's, whose FP64 pipe is shared by 16 factorisations and sees the extra instructions.)
 
+// The panel arithmetic of the three factorisations (chol_tiled, chol_global, wk_chol).  The matrix factorised is
+// cov + adj I = M2 / (n - 1) + adj I inside npar; on the padding the diagonal is 1 and every other entry 0 (M2 is 0 there).
+// (v by reference: adapt()'s diagonal loop then loads it only inside npar)
+__device__ __forceinline__ double cov_diag(const double &v, int i, int npar, double adj) { return i < npar ? v + adj : 1.0; }
+// columns col, col + 1 of matrix row `row`, from the scatter-matrix pair v; in = false (a tile outside the padded upper
+// triangle): v as loaded.  (chol_global passes its tile test as `in`: tested at its call site instead, the diagonal tests
+// compile to selects, and chol_global and dram_kernel spill differently.)
+__device__ __forceinline__ double2 cov_entry(bool in, double2 v, int row, int col, int npar, double invn, double adj)
+{
+    if (in) {
+        v.x *= invn; v.y *= invn;
+        if (row == col) v.x = cov_diag(v.x, row, npar, adj);
+        if (row == col + 1) v.y = cov_diag(v.y, row, npar, adj);
+    }
+    return v;
+}
+// the 8x8 diagonal block of the panel buffer S (row stride ldS); a one-tile-row panel (the last of an odd nt4) is filled out
+// with the identity
+__device__ __forceinline__ void diag_block(const double *S, int ldS, bool two, double (&A)[8][8])
+{
+#pragma unroll
+    for (int r = 0; r < 8; ++r)
+#pragma unroll
+        for (int c = r; c < 8; ++c) A[r][c] = (two || c < 4) ? S[r * ldS + c] : (r == c ? 1.0 : 0.0);
+}
+// forward substitution of one panel column xv against the factored diagonal block (r11[p][r], p < r; reciprocal pivots dinv)
+__device__ __forceinline__ void solve_col(const double (&r11)[8][8], const double (&dinv)[8], double (&xv)[8])
+{
+#pragma unroll
+    for (int r = 0; r < 8; ++r) {
+        double sacc = xv[r];
+#pragma unroll
+        for (int p_ = 0; p_ < r; ++p_) sacc = fma(-r11[p_][r], xv[p_], sacc);
+        xv[r] = sacc * dinv[r];
+    }
+}
+// the panel at tile rows b0, b0 + 1 (two: b0 + 1 < nt4; ntc = nt4 - b0 tile columns) from S to the tiled gW, zeros below the
+// diagonal; thread i0 of NTHR, CG: __stcg stores
+template <int NTHR, bool CG>
+__device__ __forceinline__ void store_panel(const double *S, int ldS, double *gW, int nt4, int b0, int ntc, bool two, int i0)
+{
+    const int nT = ntc + (two ? ntc - 1 : 0);
+#pragma unroll 1
+    for (int e = i0; e < 8 * nT; e += NTHR) {
+        const int u = e >> 3, r = (e >> 1) & 3, c2 = e & 1;
+        const int h = u < ntc ? 0 : 1, tcl = h ? u - ntc + 1 : u;
+        const double2 v = *reinterpret_cast<const double2 *>(S + (4 * h + r) * ldS + 4 * tcl + 2 * c2);
+        const bool dg = tcl == h;
+        const double2 o = make_double2((dg && 2 * c2 < r) ? 0.0 : v.x, (dg && 2 * c2 + 1 < r) ? 0.0 : v.y);
+        double2 *dst = reinterpret_cast<double2 *>(gW + 16 * (size_t)tidx(nt4, b0 + h, b0 + tcl) + 4 * r + 2 * c2);
+        if (CG) __stcg(dst, o); else *dst = o;
+    }
+}
+
 // Factor the 8x8 diagonal block that starts at tile row b0 (one 4x4 tile when it is the last row of an odd nt4): every
 // lane of the calling warp factors it redundantly in registers (a chain of 8 dependent rsqrt's, no communication),
 // lanes 0-2 write the three tiles back, lane 0 the reciprocal pivots.
@@ -417,13 +471,7 @@ __device__ __noinline__ bool chol_tiled(int nt4, int oW, bool prof)
                 double xv[8];
 #pragma unroll
                 for (int r = 0; r < 4; ++r) { xv[r] = u0[4 * r]; xv[4 + r] = u1[4 * r]; }
-#pragma unroll
-                for (int r = 0; r < 8; ++r) {
-                    double sacc = xv[r];
-#pragma unroll
-                    for (int p_ = 0; p_ < r; ++p_) sacc = fma(-r11[p_][r], xv[p_], sacc);
-                    xv[r] = sacc * di[r];
-                }
+                solve_col(r11, di, xv);
 #pragma unroll
                 for (int r = 0; r < 4; ++r) { u0[4 * r] = xv[r]; u1[4 * r] = xv[4 + r]; }
             }
@@ -629,6 +677,19 @@ struct CoopRing {
     }
 };
 
+// CALL with the compile-time constant N_ = n_ (1 .. 7; any other n_: nothing)
+#define DISPATCH_1_7(n_, CALL)                                                                              \
+    switch (n_) {                                                       /* warp-uniform */                  \
+    case 7: { constexpr int N_ = 7; CALL; } break;                                                          \
+    case 6: { constexpr int N_ = 6; CALL; } break;                                                          \
+    case 5: { constexpr int N_ = 5; CALL; } break;                                                          \
+    case 4: { constexpr int N_ = 4; CALL; } break;                                                          \
+    case 3: { constexpr int N_ = 3; CALL; } break;                                                          \
+    case 2: { constexpr int N_ = 2; CALL; } break;                                                          \
+    case 1: { constexpr int N_ = 1; CALL; } break;                                                          \
+    default: break;                                                                                         \
+    }
+
 // chol_global, accumulation over `nr` staged tile rows (stride `rs` doubles) for the NM column blocks of this warp: per row one
 // A fragment and NM B fragments (constant offsets: block m sits 256 m doubles after the warp's first block) + NM MMAs.
 // Lanes whose tile column lies beyond the matrix read whatever follows the row (finite or not): those are columns / rows
@@ -744,16 +805,7 @@ __device__ __noinline__ bool chol_global(int nt4, int npar, const double *gA, do
                 if (si < nst) { CG_ISSUE(b0, ntc, rps, si) ++si; }
                 const int nr = min(rps, b0 - u * rps);
                 const int pa = ring.acquire(gc) + 16 * th + inner, pb = pa + 32 * warp;
-                switch (nmine) {                                                    // warp-uniform
-                case 7: cg_accumulate<7>(pa, pb, nr, 16 * ntc, acc); break;
-                case 6: cg_accumulate<6>(pa, pb, nr, 16 * ntc, acc); break;
-                case 5: cg_accumulate<5>(pa, pb, nr, 16 * ntc, acc); break;
-                case 4: cg_accumulate<4>(pa, pb, nr, 16 * ntc, acc); break;
-                case 3: cg_accumulate<3>(pa, pb, nr, 16 * ntc, acc); break;
-                case 2: cg_accumulate<2>(pa, pb, nr, 16 * ntc, acc); break;
-                case 1: cg_accumulate<1>(pa, pb, nr, 16 * ntc, acc); break;
-                default: break;
-                }
+                DISPATCH_1_7(nmine, cg_accumulate<N_>(pa, pb, nr, 16 * ntc, acc))
                 ring.release(gc);
                 ++gc;
             }
@@ -773,12 +825,7 @@ __device__ __noinline__ bool chol_global(int nt4, int npar, const double *gA, do
                 const int j = warp + SPEC * m;
                 if (j >= nb) continue;
                 const int tcn = b0 + 2 * j + (ak >> 1), col = 4 * tcn + 2 * (ak & 1);
-                double2 v = vin[m];
-                if (tr <= tcn && tcn < nt4 && tr < nt4) {
-                    v.x *= invn; v.y *= invn;
-                    if (row == col) v.x = row < npar ? v.x + qcovadj : 1.0;
-                    if (row == col + 1) v.y = row < npar ? v.y + qcovadj : 1.0;
-                }
+                const double2 v = cov_entry(tr <= tcn && tcn < nt4 && tr < nt4, vin[m], row, col, npar, invn, qcovadj);
                 *reinterpret_cast<double2 *>(S + ar * ldS + 8 * j + 2 * ak) = make_double2(v.x - acc[m][0], v.y - acc[m][1]);
             }
         }
@@ -787,10 +834,7 @@ __device__ __noinline__ bool chol_global(int nt4, int npar, const double *gA, do
         // (2) the diagonal block
         if (warp == 0) {
             double A[8][8], dinv[8];
-#pragma unroll
-            for (int r = 0; r < 8; ++r)
-#pragma unroll
-                for (int c = r; c < 8; ++c) A[r][c] = (two || c < 4) ? S[r * ldS + c] : (r == c ? 1.0 : 0.0);
+            diag_block(S, ldS, two, A);
             const bool bad = chol8(A, dinv);
             if (lane == 0) {
 #pragma unroll
@@ -825,31 +869,14 @@ __device__ __noinline__ bool chol_global(int nt4, int npar, const double *gA, do
                 double xv[8];
 #pragma unroll
                 for (int r = 0; r < 8; ++r) xv[r] = S[r * ldS + cc];
-#pragma unroll
-                for (int r = 0; r < 8; ++r) {
-                    double sacc = xv[r];
-#pragma unroll
-                    for (int p_ = 0; p_ < r; ++p_) sacc = fma(-r11[p_][r], xv[p_], sacc);
-                    xv[r] = sacc * di[r];
-                }
+                solve_col(r11, di, xv);
 #pragma unroll
                 for (int r = 0; r < 8; ++r) S[r * ldS + cc] = xv[r];
             }
             __syncthreads();
         }
-        // (4) the panel goes to gW (tiles (b0, b0..), (b0+1, b0+1..)); zeros below the diagonal
-        {
-            const int nT = ntc + (two ? ntc - 1 : 0);
-#pragma unroll 1
-            for (int e = tid; e < 8 * nT; e += DRAM_THREADS) {
-                const int u = e >> 3, r = (e >> 1) & 3, c2 = e & 1;
-                const int h = u < ntc ? 0 : 1, tcl = h ? u - ntc + 1 : u;
-                const double2 v = *reinterpret_cast<const double2 *>(S + (4 * h + r) * ldS + 4 * tcl + 2 * c2);
-                const bool dg = tcl == h;
-                const double v0 = (dg && 2 * c2 < r) ? 0.0 : v.x, v1 = (dg && 2 * c2 + 1 < r) ? 0.0 : v.y;
-                *reinterpret_cast<double2 *>(gW + 16 * (size_t)tidx(nt4, b0 + h, b0 + tcl) + 4 * r + 2 * c2) = make_double2(v0, v1);
-            }
-        }
+        // (4) the panel goes to gW
+        store_panel<DRAM_THREADS, false>(S, ldS, gW, nt4, b0, ntc, two, tid);
         __syncthreads();                                          // the next panels read these tiles back from L2 (cp.async.cg)
         CGP(15);
     }
@@ -1175,17 +1202,6 @@ __device__ __forceinline__ void genb_rows(int kk, int kend, int &bt, int oa, int
         genb_row<NA, false>(bt, false, za, acc);
     }
 }
-#define GENB_DISPATCH(na_, CALL)                                                                            \
-    switch (na_) {                                                      /* warp-uniform */                  \
-    case 7: { constexpr int NA_ = 7; CALL; } break;                                                         \
-    case 6: { constexpr int NA_ = 6; CALL; } break;                                                         \
-    case 5: { constexpr int NA_ = 5; CALL; } break;                                                         \
-    case 4: { constexpr int NA_ = 4; CALL; } break;                                                         \
-    case 3: { constexpr int NA_ = 3; CALL; } break;                                                         \
-    case 2: { constexpr int NA_ = 2; CALL; } break;                                                         \
-    case 1: { constexpr int NA_ = 1; CALL; } break;                                                         \
-    default: break;                                                                                         \
-    }
 #ifdef TC_SUBPROF
 #define GSP_T0 long long gt__ = clock64()
 #define GSP(i) do { if (threadIdx.x == 0 && cx.ch == 0) { const long long t__ = clock64(); tc_subprof[i] += t__ - gt__; gt__ = t__; } } while (0)
@@ -1242,14 +1258,14 @@ __device__ __noinline__ void gen_increments_tma(const ChainCtx &cx, int g0, int 
         while (k < kend && k < kmax) {
             const int kto = min(kend, min(last, kmax));             // the rows before the next edge row
             if (k < kto) {
-                GENB_DISPATCH(na, genb_rows<NA_>(k, kto, bt, oa, nt4, npar, ak, acc))
+                DISPATCH_1_7(na, genb_rows<N_>(k, kto, bt, oa, nt4, npar, ak, acc))
                 k = kto;
             }
             if (k < kend && k == last && k < kmax) {
                 // the lowest live tile is in its last k-step: the lanes of its first tile column have nothing stored there
                 double2 za = make_double2(0.0, 0.0);
                 if (4 * k + ak < npar) za = *reinterpret_cast<const double2 *>(tc_smem + oa + 8 * k);
-                GENB_DISPATCH(na, (genb_row<NA_, true>(bt, th == 0, za, acc)))
+                DISPATCH_1_7(na, (genb_row<N_, true>(bt, th == 0, za, acc)))
                 bt += 16 * (nt4 - k - 1);
                 ++k; --na; last += 2 * SPEC;
             }
@@ -1701,24 +1717,24 @@ __device__ __noinline__ int adapt(const RunArgs &a, const ChainCtx &cx, int isim
         }
         double *W = tc_smem + cx.o_ring;
         unsigned short *tab = reinterpret_cast<unsigned short *>(W + 16 * T4);
+#pragma unroll 1
+        for (int t = tid; t < T4; t += DRAM_THREADS) {
+            int rem = t, b = 0;
+            while (rem >= nt4 - b) { rem -= nt4 - b; ++b; }
+            tab[t] = (unsigned short)((b << 8) | (b + rem));
+        }
         bool ok = false;
 #pragma unroll 1
         for (int attempt = a.qcovadj_always ? 1 : 0; attempt < 2 && !ok; ++attempt) {
             const double adj = attempt ? a.qcovadj : 0.0;
             __syncthreads();
-#pragma unroll 1
-            for (int t = tid; t < T4; t += DRAM_THREADS) {
-                int rem = t, b = 0;
-                while (rem >= nt4 - b) { rem -= nt4 - b; ++b; }
-                tab[t] = (unsigned short)((b << 8) | (b + rem));
-            }
             scaled_copy_cg(reinterpret_cast<double2 *>(W), reinterpret_cast<const double2 *>(cx.gM2), 8 * T4, invn);
             __syncthreads();
-            // + adj I; identity on the padding rows (the rest of the padding is zero: it only ever accumulated zeros)
+            // the diagonal of cov_entry's matrix (the rest of the padding is zero: it only ever accumulated zeros)
 #pragma unroll 1
             for (int i = tid; i < 4 * nt4; i += DRAM_THREADS) {
                 double *d = W + 16 * tidx(nt4, i >> 2, i >> 2) + 5 * (i & 3);
-                *d = i < npar ? *d + adj : 1.0;
+                *d = cov_diag(*d, i, npar, adj);
             }
             __syncthreads();
             SUBP(10);
