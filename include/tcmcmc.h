@@ -81,7 +81,7 @@ typedef struct tc_mcmc_opts {
                                  `rejected > 0.95*isimu` (SURVEY.md 3.2 / B.3, [U]); 0: rejections since the last adaptation */
     int32_t n_burn;           /* summaries / stored rows start at MATLAB row n_burn: chain(n_burn:end,:)
                                  (:276-283); >= 1 */
-    int32_t store_chain;      /* 0: summaries only; 1: also return rows n_burn..nsimu and s2chain */
+    int32_t store_chain;      /* 0: summaries only; 1: also return rows n_burn..nsimu and s2chain (every thin-th of them) */
     int32_t replay;           /* 1: consume caller-supplied randomness instead of Philox */
     int32_t algo;             /* TC_ALGO_* used for ssfun inside the sampler */
     int32_t ngpus;            /* 'numParPools' reinterpreted: devices 0..ngpus-1 (or devices[]) */
@@ -110,6 +110,11 @@ typedef struct tc_mcmc_opts {
                                  results bit-identical across GPU counts at every chain count */
     int32_t qcovadj_always;   /* 0 (default): R = chol(cov), and chol(cov + qcovadj I) only when that fails — mcmcstat's
                                  "try to blow it" branch [U]; 1: always factor cov + qcovadj I */
+    int32_t thin;             /* store_chain: keep every thin-th row (>= 1; 1, the default: every row).  chain keeps the 0-based
+                                 rows n_burn-1 + j*thin, j < nkeep = (nsimu-n_burn)/thin + 1; s2chain the rows j*thin,
+                                 j < ns2 = (nsimu-1)/thin + 1: a regular subsample of the chain thin = 1 returns, bit for bit.
+                                 mean, std, sig, the counters, flags and sschain still cover every row.  Ignored without
+                                 store_chain */
 } tc_mcmc_opts;
 enum { TC_LAYOUT_AUTO = 0, TC_LAYOUT_BIG = 1, TC_LAYOUT_WARP = 2, TC_LAYOUT_CTA = 3 };
 
@@ -185,7 +190,8 @@ int tc_forward(const tc_cells *cells, int64_t nbatch, const int32_t *cell_id, co
  *   mean, std [nchains x ld]   mean / population std of rows n_burn..nsimu (:286-301)
  *   sig [nchains x 2]          sqrt(mean(s2chain)), std(sqrt(s2chain),1) over ALL rows (:302-303)
  *   counters [nchains x TC_NCOUNTERS] int64
- *   chain [nchains x (nsimu-n_burn+1) x ld], s2chain [nchains x nsimu]   (store_chain = 1)
+ *   chain [nchains x nkeep x ld], s2chain [nchains x ns2]   (store_chain = 1; opts->thin = 1: nkeep = nsimu-n_burn+1,
+ *                              ns2 = nsimu; larger thin: the counts of tc_mcmc_opts.thin)
  * Series length: max(N) <= 441 (one CTA per chain holds the cell, the chain state, the proposal slots and the
  * forward-model scratch in one SM; beyond ~210 points the large-series layout of opts->layout is used); longer series
  * return TC_EINVAL.

@@ -15,12 +15,16 @@ function TranscriptionCycleMCMC(varargin)
 %the extra variable MCMCdiagnostics (cell_index, numChains, Rhat, n_eff,
 %Rhat_max: Gelman-Rubin across the chains of a cell) is saved next to
 %MCMCresults.  With numChains = 1 the outputs are exactly the reference's.
+%'thin' (default 1): MCMCchain keeps every thin-th row (rows n_burn,
+%n_burn+thin, ... and s2chain rows 1, 1+thin, ...), a regular subsample of
+%the same chain stored on the GPU, and the raw-chain file carries the scalar
+%thin; MCMCresults still summarise every row.
 
 %% Variable inputs (defaults of the reference code)
 fileDir = pwd; saveLoc = pwd; numParPools = 8; n_burn = 10000; n_steps = 20000;
 ratePriorWidth = 50; t_start = 0; t_end = Inf; loadPrevious = false;
 construct = 'P2P-MS2v5-LacZ-PP7v4'; files_arg = {}; seed = 20201028; saveChains = true;
-prevFile = ''; numChains = 1;
+prevFile = ''; numChains = 1; thin = 1;
 for i = 1:length(varargin)
     if ~(ischar(varargin{i}) || isstring(varargin{i})), continue; end
     switch lower(char(varargin{i}))
@@ -39,9 +43,13 @@ for i = 1:length(varargin)
         case 'savechains', saveChains = varargin{i+1};
         case 'previousresults', prevFile = varargin{i+1};
         case 'numchains', numChains = varargin{i+1};
+        case 'thin', thin = varargin{i+1};
     end
 end
 C = tcmcmc_constructs(construct);   %same table as GetFluorFromPolPos.m; errors on unknown names
+if ~(isscalar(thin) && isnumeric(thin) && thin >= 1 && thin == round(thin))
+    error('TranscriptionCycleMCMC:thin', '''thin'' must be an integer >= 1');
+end
 
 %% Choose datasets (dialog only when a display exists and no 'files' given)
 files = dir(fullfile(fileDir, '*.mat')); names = {files.name};
@@ -85,7 +93,8 @@ for k = 1:length(s)
         upp(1:np, j) = [vu, 20, 10, 50, 50, 1, 40, 30*ones(1, N)]';
         sg(8:np, j) = ratePriorWidth;
     end
-    opts = struct('n_steps', n_steps, 'n_burn', n_burn, 'numGPUs', numParPools, 'seed', seed, 'saveChains', saveChains);
+    opts = struct('n_steps', n_steps, 'n_burn', n_burn, 'numGPUs', numParPools, 'seed', seed, 'saveChains', saveChains, ...
+        'thin', thin);
     if numChains > 1, opts.chainCell = chainCell; end
     out = tcmcmc_mex('fit', C, cells, opts, x0, J0, low, upp, mu, sg);
 
@@ -125,7 +134,7 @@ for k = 1:length(s)
         N = numel(cells(q).time); m = pm(:, q); sd = ps(:, q);
         if saveChains
             cols = (q-1)*numChains + (1:numChains);
-            ch = reshape(permute(out.chain(:, :, cols), [2 3 1]), [], ld);   %rows n_burn..n_steps, chain after chain
+            ch = reshape(permute(out.chain(:, :, cols), [2 3 1]), [], ld);   %rows n_burn:thin:n_steps, chain after chain
             s2 = reshape(out.s2chain(:, cols), [], 1);
             MCMCchain(q) = struct('v_chain', ch(:,1), 'ton_chain', ch(:,3), 'A_chain', ch(:,6), 'tau_chain', ch(:,2), ...
                 'MS2_basal_chain', ch(:,4), 'PP7_basal_chain', ch(:,5), 'R_chain', ch(:,7), 'dR_chain', ch(:,8:7+N), ...
@@ -148,8 +157,10 @@ for k = 1:length(s)
     end
     if saveChains
         w = whos('MCMCchain');
+        extra = {};
+        if thin > 1, extra = {'thin'}; end                           %the reference's variables alone when every row is kept
         if w.bytes < 2^31 - 2^24
-            save(fullfile(saveLoc, [filename, '_RawChain.mat']), 'MCMCchain');    %the reference's file (MAT v5/v7)
+            save(fullfile(saveLoc, [filename, '_RawChain.mat']), 'MCMCchain', extra{:});    %the reference's file (MAT v5/v7)
         else
             %plain save cannot hold a variable of 2 GiB (the reference's own defaults on TestData give 3.1 GB): parts of
             %whole cells below the limit + an index, the layout of the Python host (LoadRawChains.m reads both)
@@ -160,11 +171,11 @@ for k = 1:length(s)
                 while last < numel(full) && acc + sz(last+1) <= lim, last = last + 1; acc = acc + sz(last); end
                 k = k + 1; MCMCchain = full(first:last); firstCell = first; lastCell = last; part = k; %#ok<NASGU>
                 parts{k, 1} = sprintf('%s_RawChain_part%d.mat', filename, k); %#ok<AGROW>
-                save(fullfile(saveLoc, parts{k}), 'MCMCchain', 'firstCell', 'lastCell', 'part');
+                save(fullfile(saveLoc, parts{k}), 'MCMCchain', 'firstCell', 'lastCell', 'part', extra{:});
                 partOf(first:last) = k; first = last + 1;
             end
             MCMCchainParts = parts; MCMCchainPartOfCell = partOf; nParts = k; %#ok<NASGU>
-            save(fullfile(saveLoc, [filename, '_RawChain.mat']), 'MCMCchainParts', 'MCMCchainPartOfCell', 'nParts');
+            save(fullfile(saveLoc, [filename, '_RawChain.mat']), 'MCMCchainParts', 'MCMCchainPartOfCell', 'nParts', extra{:});
         end
     end
 end

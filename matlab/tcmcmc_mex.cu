@@ -14,12 +14,14 @@
 //              (the quantities of src/GetFluorFromPolPos.m:18-30; vectors = one entry per loop set)
 //   cells      1 x Ncells struct array with fields time, MS2, PP7 (already truncated to [t_start,t_end))
 //   opts       struct: n_steps, n_burn, numGPUs, seed, saveChains  (+ optional mcmcstat overrides); chainCell: optional
-//              1 x Nchains vector, the (1-based) cell of every chain ('numChains' > 1); default one chain per cell
+//              1 x Nchains vector, the (1-based) cell of every chain ('numChains' > 1); default one chain per cell; thin:
+//              optional, store every thin-th row of the raw chains (default 1: every row)
 //   x0 .. prior_sig   npar_max x Nchains double (column c = chain c, zero padded)
 //
 //   out        struct: mean, std (npar_max x Nchains), sig (2 x Nchains), counters (16 x Nchains, int64),
-//              chain (npar_max x (n_steps-n_burn+1) x Nchains), s2chain (n_steps x Nchains)
-//              [chain/s2chain only when opts.saveChains], simMS2/simPP7 (Nmax x Ncells; only with one chain per cell)
+//              chain (npar_max x nkeep x Nchains), s2chain (ns2 x Nchains) [chain/s2chain only when opts.saveChains; rows
+//              n_burn, n_burn+thin, .. of the chain, nkeep = floor((n_steps-n_burn)/thin)+1, and rows 1, 1+thin, .. of
+//              s2chain, ns2 = ceil(n_steps/thin)], simMS2/simPP7 (Nmax x Ncells; only with one chain per cell)
 //   sim        struct: simMS2, simPP7 (Nmax x Ncells) for theta (npar_max x Ncells)
 #include <cstring>
 #include <vector>
@@ -130,6 +132,7 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
     o.burnin_cumulative = (int32_t)field_scalar(prhs[3], "burnin_cumulative", o.burnin_cumulative);
     o.N0 = field_scalar(prhs[3], "N0", o.N0);
     o.layout = (int32_t)field_scalar(prhs[3], "layout", o.layout);   // TC_LAYOUT_AUTO; 1: large-series layout, 2: one warp per chain
+    o.thin = (int32_t)field_scalar(prhs[3], "thin", 1);
     int ndev = 0;
     check(tc_device_count(&ndev));
     if (o.ngpus > ndev) o.ngpus = ndev;
@@ -159,10 +162,11 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
     mxArray *cnt = mxCreateNumericMatrix(TC_NCOUNTERS, nchains, mxINT64_CLASS, mxREAL);
     mxArray *chain = nullptr, *s2 = nullptr;
     if (o.store_chain) {
-        // MATLAB is column-major: [ld x nrows x nchains] here is the engine's row-major [nchains][nrows][ld]
-        const mwSize dims[3] = {(mwSize)ld, (mwSize)(o.nsimu - o.n_burn + 1), (mwSize)nchains};
+        if (o.thin < 1) mexErrMsgIdAndTxt("tcmcmc:opts", "opts.thin must be an integer >= 1");
+        // MATLAB is column-major: [ld x nkeep x nchains] here is the engine's row-major [nchains][nkeep][ld]
+        const mwSize dims[3] = {(mwSize)ld, (mwSize)((o.nsimu - o.n_burn) / o.thin + 1), (mwSize)nchains};
         chain = mxCreateNumericArray(3, dims, mxDOUBLE_CLASS, mxREAL);
-        s2 = mxCreateDoubleMatrix(o.nsimu, nchains, mxREAL);
+        s2 = mxCreateDoubleMatrix((o.nsimu - 1) / o.thin + 1, nchains, mxREAL);
     }
     const int rc = tc_mcmc_run(cells, &o, nchains, chain_cell.data(), uid.data(), ld, mxGetPr(prhs[4]), mxGetPr(prhs[5]),
                                mxGetPr(prhs[6]), mxGetPr(prhs[7]), mxGetPr(prhs[8]), mxGetPr(prhs[9]), mxGetPr(mean),

@@ -53,7 +53,7 @@ class McmcOpts(C.Structure):
         ("devices", C.c_int32 * MAX_GPUS),
         ("drscale", C.c_double), ("adascale", C.c_double), ("qcovadj", C.c_double),
         ("burnin_scale", C.c_double), ("N0", C.c_double), ("S20", C.c_double), ("sigma2_0", C.c_double),
-        ("seed", C.c_uint64), ("layout", C.c_int32), ("qcovadj_always", C.c_int32),
+        ("seed", C.c_uint64), ("layout", C.c_int32), ("qcovadj_always", C.c_int32), ("thin", C.c_int32),
     ]
 
 
@@ -177,6 +177,13 @@ def device_info(device=0):
     check(load().tc_device_info_get(device, C.byref(info)))
     return dict(name=info.name.decode(), cc=(info.cc_major, info.cc_minor), sm_count=info.sm_count,
                 total_mem=info.total_mem, smem_per_block_optin=info.smem_per_block_optin)
+
+
+def stored_rows(opts):
+    """(nkeep, ns2): the chain rows and s2chain rows a fit with these options stores per chain (include/tcmcmc.h,
+    tc_mcmc_opts.thin).  A thin below 1 is sized as 1: tc_mcmc_run refuses it."""
+    k = max(int(opts.thin), 1)
+    return (opts.nsimu - opts.n_burn) // k + 1, (opts.nsimu - 1) // k + 1
 
 
 def default_opts(**kw):

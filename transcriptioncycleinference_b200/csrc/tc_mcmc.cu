@@ -182,10 +182,13 @@ struct RunArgs {
     unsigned long long *wq;
     // time slicing
     int seglen;
+    int thin;                                           // store_chain: every thin-th row is stored.  (thin and nkeep fill the
+                                                        // alignment holes before the pointers: the fields keep their offsets)
     int *cstate;
     // dram_kernel, two CTAs per SM: a chain that lags the mean progress by solo_lag slices or more gets its SM to itself
     // (smctl[%smid] = 1 + blockIdx of the owner; 0: shared); solo_lag <= 0: off
     int solo_lag;
+    int nkeep;                                          // store_chain: chain rows stored per chain (thin_nkeep)
     int *smctl;
 };
 
@@ -894,10 +897,15 @@ struct StepOut { double ssn, prin; int acc, fl, nev, noob; };
 
 // ---- chain book-keeping shared by dram_kernel and dram_warp_kernel (tc_warp.cuh)
 
+// Rows a fit stores with store_chain, keeping every thin-th: chain rows first_row + j thin (j < thin_nkeep), s2chain rows j thin
+// (j < thin_ns2).  Ceilings as (x - 1) / thin + 1: no overflow at thin = 2^31 - 1.
+static int thin_nkeep(int nsimu, int n_burn, int thin) { return (nsimu - n_burn) / thin + 1; }
+__host__ __device__ inline int thin_ns2(int nsimu, int thin) { return (nsimu - 1) / thin + 1; }
+
 // Constants of a chain that both samplers derive their per-step arithmetic from
 struct ChainConsts {
     unsigned long long uid;                             // Philox identity
-    int first_row, nstore;                              // first row of the summaries and of the stored chain (n_burn - 1), rows stored
+    int first_row, nkeep;                               // first row of the summaries and of the stored chain (n_burn - 1), rows stored
     double inv_dr, adascale, chi_d, chi_c;              // chi_d, chi_c: Marsaglia-Tsang constants of chi2(N0 + 2 N)
 };
 __device__ __forceinline__ ChainConsts chain_consts(const RunArgs &a, int ch, int N)
@@ -905,7 +913,7 @@ __device__ __forceinline__ ChainConsts chain_consts(const RunArgs &a, int ch, in
     ChainConsts k;
     k.uid = a.chain_uid ? a.chain_uid[ch] : (unsigned long long)ch;
     k.first_row = a.n_burn - 1;
-    k.nstore = a.nsimu - (a.n_burn - 1);
+    k.nkeep = a.nkeep;
     k.inv_dr = 1.0 / a.drscale;
     k.adascale = a.adascale > 0.0 ? a.adascale : 2.4 / sqrt((double)(7 + N));
     chi2_consts(a.N0 + 2.0 * N, k.chi_d, k.chi_c);
@@ -975,6 +983,19 @@ __device__ __forceinline__ bool stage1_accepts(double ss1, double ss, double is2
 // A run (the rows [r0, r1), all equal to the state) closes: the rows it adds to the Welford summaries (those >= first_row),
 // and whether it is one more distinct row of the covariance block
 __device__ __forceinline__ int run_rows(int r0, int r1, int first_row) { return max(0, r1 - max(r0, first_row)); }
+// The stored rows of a run's m_w summarised rows [rs, rs + m_w), rs >= first_row, when every thin-th row is stored: chain rows
+// j0 .. j0 + return value - 1, the rows first_row + j thin among them.  Two divisions per run, computed before the run
+// writer's per-parameter loop; none per row.
+//
+// The samplers are compiled twice, THIN = false (every row; thin = 1 or no stored rows) and THIN = true (thin > 1): the run
+// writers sit on the path of every accept, and the code and registers of the thinned writes cost config 2 ~0.7 % of kernel
+// time (B200) even where they never run.
+__device__ __forceinline__ int kept_rows(int rs, int m_w, int first_row, int thin, int &j0)
+{
+    const int x = rs - first_row;
+    j0 = x == 0 ? 0 : (x - 1) / thin + 1;
+    return m_w > 0 ? (x + m_w - 1) / thin - j0 + 1 : 0;
+}
 __device__ __forceinline__ bool run_distinct(int do_cov, int r0, int r1) { return do_cov && r1 > r0; }
 // Welford weights of m_w rows folded into wcnt rows (mean += d f1, M2 += d^2 f2) through ONE reciprocal (two quotients were
 // ~300 cycles at the head of every accept)
@@ -1050,19 +1071,27 @@ __device__ __forceinline__ ParkedChain resume_chain(const double *gst)
     return p;
 }
 
-// The optional per-row outputs of row r: s2chain (store_chain), flags and sschain (replay / parity harness)
+// The optional per-row outputs of row r: s2chain (store_chain; THIN: rows 0, thin, 2 thin, ..), flags and sschain (replay /
+// parity harness; every row)
+template <bool THIN>
 __device__ __forceinline__ void store_row(const RunArgs &a, int ch, int r, double s2, int fl, double ss)
 {
     const size_t g = (size_t)ch * a.nsimu + r;
-    if (a.store_chain && a.s2chain) a.s2chain[g] = s2;
+    if (THIN) {
+        const int j = r / a.thin;
+        if (a.store_chain && a.s2chain && j * a.thin == r) a.s2chain[(size_t)ch * thin_ns2(a.nsimu, a.thin) + j] = s2;
+    } else if (a.store_chain && a.s2chain) {
+        a.s2chain[g] = s2;
+    }
     if (a.flags) a.flags[g] = fl;
     if (a.sschain) a.sschain[g] = ss;
 }
 // Row 0 = x0 with a finite ss0: s2 = sigma2_0 (TranscriptionCycleMCMC.m:259), no flags.  One thread.
+template <bool THIN>
 __device__ __forceinline__ void record_row0(const RunArgs &a, int ch, double ss0, Tally &t)
 {
     tally_s2(t, 1.0, a.sigma2_0, sqrt(a.sigma2_0), 0.0);
-    store_row(a, ch, 0, a.sigma2_0, 0, ss0);
+    store_row<THIN>(a, ch, 0, a.sigma2_0, 0, ss0);
 }
 
 // a Welford vector: shared memory (dram_kernel) or L2 (dram_warp_kernel: written by other SMs, so past L1)
@@ -1129,6 +1158,7 @@ struct ChainCtx {
 // storage, and the distinct-row buffer of the current covariance block (row + weight); then, when
 // so >= 0, move the state: x += increment at tc_smem[so + i].  Every thread owns the indices i = tid, tid+256, ..
 // so the whole thing is one pass.
+template <bool THIN>
 __device__ __noinline__ void flush_run(const RunArgs &a, const ChainCtx &cx, int r0, int r1, double wcnt, int ndist, int so, int t0)
 {
     // threads t0 .. DRAM_THREADS-1 take part (t0 = 32 at an accept: warp 0 writes the per-row scalars meanwhile)
@@ -1139,6 +1169,8 @@ __device__ __noinline__ void flush_run(const RunArgs &a, const ChainCtx &cx, int
     double f1, f2;
     welford_weights(wcnt, m_w, f1, f2);
     double *grow = cov ? cx.gRows + (size_t)ndist * cx.ld : nullptr;
+    int j0 = rs - cx.cc.first_row, nkr = m_w;
+    if (THIN && a.store_chain && a.chain) nkr = kept_rows(rs, m_w, cx.cc.first_row, a.thin, j0);
     const int ox = cx.o_x, owm = cx.o_wmean, ow2 = cx.o_wM2, omb = cx.o_mb;
 #pragma unroll 1
     for (int i = tid; i < npar; i += nthr) {
@@ -1148,9 +1180,9 @@ __device__ __noinline__ void flush_run(const RunArgs &a, const ChainCtx &cx, int
             tc_smem[owm + i] = fma(d1, f1, wm);
             tc_smem[ow2 + i] = fma(d1 * d1, f2, tc_smem[ow2 + i]);
             if (a.store_chain && a.chain) {
-                double *dst = a.chain + ((size_t)cx.ch * cx.cc.nstore + (rs - cx.cc.first_row)) * cx.ld + i;
+                double *dst = a.chain + ((size_t)cx.ch * cx.cc.nkeep + j0) * cx.ld + i;
 #pragma unroll 1
-                for (int r = 0; r < m_w; ++r) dst[(size_t)r * cx.ld] = xo;
+                for (int r = 0; r < nkr; ++r) dst[(size_t)r * cx.ld] = xo;
             }
         }
         if (cov) {
@@ -1773,6 +1805,7 @@ __device__ __noinline__ int adapt(const RunArgs &a, const ChainCtx &cx, int isim
 // Book-keeping works on RUNS (an accepted state and the rejections that follow it): a rejected step
 // only lengthens the current run; summaries, chain storage and the covariance block see a run once,
 // with its length as weight.
+template <bool THIN>
 __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_constant__ RunArgs ga)
 {
     // The out-of-line phases take the launch arguments by reference: a reference to the kernel parameter
@@ -2006,7 +2039,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             const bool bad = !isfinite(ss0);
             if (tid == 0) {
                 st.ss = ss0; st.pri = sp; st.bad0 = bad ? 1 : 0; st.rden = rden_of(a.N0 * a.S20, ss0); st.rsig = 1.0 / a.sigma2_0;
-                if (!bad) record_row0(a, ch, ss0, st.t);
+                if (!bad) record_row0<THIN>(a, ch, ss0, st.t);
             }
             __syncthreads();
         }
@@ -2125,7 +2158,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             SUBP(20);
             if (accd) {
                 // close the run of the old state at row r_acc and move x by the accepted increment
-                flush_run(a, cx, run_r0, r_acc, wcnt, ndist, cx.slot_i(r_acc) + (acc_t == 2 ? cx.s1 : 0), 32);
+                flush_run<THIN>(a, cx, run_r0, r_acc, wcnt, ndist, cx.slot_i(r_acc) + (acc_t == 2 ? cx.s1 : 0), 32);
             }
             SUBP(21);
             if (warp == 0) {
@@ -2155,7 +2188,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
                     const double ssr = lane < first ? ss : ss_new;
                     s2 = row_sigma2(a.updatesigma, a.N0 * a.S20, ssr, cx.slot_sc(r)[2], sig2);
                     sq = sqrt(s2);
-                    store_row(a, cx.ch, r, s2, so_.fl, ssr);
+                    store_row<THIN>(a, cx.ch, r, s2, so_.fl, ssr);
                 }
                 // the round's sum of s2, and mean of sqrt(s2) and squared deviations from it (rows = lanes < ncommit <= RING / 2)
                 double s2b = s2, mb = sq;
@@ -2191,7 +2224,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             if (k == next_adapt) {
                 const int rr0 = st.run_r0, nd0 = st.ndist;
                 const double wc0 = st.t.wcnt;
-                flush_run(a, cx, rr0, k, wc0, nd0, -1, 0);                     // close the run at the block boundary
+                flush_run<THIN>(a, cx, rr0, k, wc0, nd0, -1, 0);                     // close the run at the block boundary
                 const int nd = nd0 + (run_distinct(a.do_cov, rr0, k) ? 1 : 0);
                 const double rate = adapt_rate(a, st.t.rej, st.t.reju, k);
                 const double cov_n = st.t.cov_n;
@@ -2215,7 +2248,7 @@ __global__ void __launch_bounds__(DRAM_THREADS, 2) dram_kernel(const __grid_cons
             // close the last run (the fit or the slice does not end on an adaptation boundary)
             const int rr0 = st.run_r0;
             const double wc0 = st.t.wcnt;
-            flush_run(a, cx, rr0, k, wc0, st.ndist, -1, 0);
+            flush_run<THIN>(a, cx, rr0, k, wc0, st.ndist, -1, 0);
             __syncthreads();
             if (tid == 0) { st.t.wcnt = wc0 + run_rows(rr0, k, cx.cc.first_row); st.run_r0 = k; }
             __syncthreads();
@@ -2404,7 +2437,7 @@ void tc_opts_default(tc_mcmc_opts *o)
     std::memset(o, 0, sizeof(*o));
     o->nsimu = 20000; o->burnintime = 10000; o->adaptint = 100; o->ntry = 2; o->updatesigma = 1;
     o->burnin_cumulative = 1; o->qcovadj_always = 0; o->n_burn = 10000; o->store_chain = 0; o->replay = 0; o->algo = TC_ALGO_TOEPLITZ;
-    o->ngpus = 1;
+    o->ngpus = 1; o->thin = 1;
     for (int i = 0; i < TC_MAX_GPUS; ++i) o->devices[i] = -1;
     o->drscale = 5.0; o->adascale = 0.0; o->qcovadj = 1e-8; o->burnin_scale = 10.0; o->N0 = 1.0; o->S20 = 1.0;
     o->sigma2_0 = 1.0; o->seed = 20201028ULL;
@@ -2823,13 +2856,25 @@ static int check_params(const tc_cells *c, int nchains, const int32_t *chain_cel
     return TC_OK;
 }
 
+// The thinning of the stored rows: thin, validated by tc_mcmc_run when rows are stored, and ignored (1) when they are not
+static int stored_thin(const tc_mcmc_opts *o) { return o->store_chain ? o->thin : 1; }
+
+// The sampler of a launch: dram_warp_kernel or dram_kernel, compiled for thinned rows when thin > 1 is stored
+static void (*sampler_kernel(bool warp, bool thin))(RunArgs)
+{
+    if (warp) return thin ? dram_warp_kernel<true> : dram_warp_kernel<false>;
+    return thin ? dram_kernel<true> : dram_kernel<false>;
+}
+
 // One device's share of a fit, chains [r.c0, r.c1): its stream, events and scratch pool, RunArgs from the options and
 // r.plan, the chains' inputs uploaded, outputs and scratch allocated.
 static int setup_run(DevRun &r, const tc_cells *c, const tc_mcmc_opts *o, int ld, const int32_t *chain_cell,
                      const uint64_t *chain_uid, const double *theta0, const double *qcov_diag, const double *low,
                      const double *upp, const double *prior_mu, const double *prior_sig, const tc_replay *rp)
 {
-    const int nc = r.c1 - r.c0, Nmax = c->Nmax, nstore = o->nsimu - (o->n_burn - 1);
+    const int nc = r.c1 - r.c0, Nmax = c->Nmax;
+    const int thin = stored_thin(o);
+    const size_t nkeep = thin_nkeep(o->nsimu, o->n_burn, thin), ns2 = thin_ns2(o->nsimu, thin);
     const size_t o0 = (size_t)r.c0;
     const int ldR = tri_doubles(7 + Nmax);               // proposal factor / scatter matrix in 4x4 tiles (chol_tiled)
     const bool do_cov = cov_adaptations(o);
@@ -2845,6 +2890,7 @@ static int setup_run(DevRun &r, const tc_cells *c, const tc_mcmc_opts *o, int ld
     a.nsimu = o->nsimu; a.burnintime = o->burnintime; a.adaptint = o->adaptint; a.ntry = o->ntry;
     a.updatesigma = o->updatesigma; a.burnin_cumulative = o->burnin_cumulative; a.n_burn = o->n_burn;
     a.store_chain = o->store_chain; a.replay = o->replay; a.algo = o->algo; a.qcovadj_always = o->qcovadj_always;
+    a.thin = thin; a.nkeep = (int)nkeep;
     a.drscale = o->drscale; a.adascale = o->adascale; a.qcovadj = o->qcovadj; a.burnin_scale = o->burnin_scale;
     a.N0 = o->N0; a.S20 = o->S20; a.sigma2_0 = o->sigma2_0; a.seed = o->seed;
     a.nchains = nc; a.ld = ld; a.nmax = Nmax; a.ldR = ldR; a.do_cov = do_cov ? 1 : 0;
@@ -2868,10 +2914,10 @@ static int setup_run(DevRun &r, const tc_cells *c, const tc_mcmc_opts *o, int ld
     CUDA_TRY(r.buf.alloc(a.sig, (size_t)nc * 2));
     CUDA_TRY(r.buf.alloc(a.counters, (size_t)nc * TC_NCOUNTERS));
     if (o->store_chain) {
-        CUDA_TRY(r.buf.alloc(a.chain, (size_t)nc * nstore * ld));
-        CUDA_TRY(cudaMemsetAsync(a.chain, 0, (size_t)nc * nstore * ld * 8, r.st));
-        CUDA_TRY(r.buf.alloc(a.s2chain, (size_t)nc * o->nsimu));
-        CUDA_TRY(cudaMemsetAsync(a.s2chain, 0, (size_t)nc * o->nsimu * 8, r.st));
+        CUDA_TRY(r.buf.alloc(a.chain, (size_t)nc * nkeep * ld));
+        CUDA_TRY(cudaMemsetAsync(a.chain, 0, (size_t)nc * nkeep * ld * 8, r.st));
+        CUDA_TRY(r.buf.alloc(a.s2chain, (size_t)nc * ns2));
+        CUDA_TRY(cudaMemsetAsync(a.s2chain, 0, (size_t)nc * ns2 * 8, r.st));
     }
     if (o->replay) {
         const size_t nz = (size_t)nc * o->nsimu * ld, nu = (size_t)nc * o->nsimu;
@@ -2926,6 +2972,7 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
     if (ld < 7 + c->Nmax) return fail(TC_EINVAL, "ld < 7 + max(N)");
     if (o->nsimu < 1) return fail(TC_EINVAL, "nsimu < 1");
     if (o->n_burn < 1 || o->n_burn > o->nsimu) return fail(TC_EINVAL, "n_burn must be in [1, nsimu]");
+    if (o->store_chain && o->thin < 1) return fail(TC_EINVAL, "thin must be >= 1");
     if (o->ntry < 1 || o->ntry > 2) return fail(TC_EINVAL, "ntry must be 1 or 2");
     if (!(o->drscale > 0)) return fail(TC_EINVAL, "drscale must be > 0");
     if (o->algo != TC_ALGO_PAIRS && o->algo != TC_ALGO_TOEPLITZ) return fail(TC_EINVAL, "unknown algo");
@@ -2956,11 +3003,11 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
         CUDA_TRY(cudaSetDevice(r.device));
         CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, r.device));
         CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, r.device));
-        CUDA_TRY(cudaFuncGetAttributes(&fa, dram_kernel));
-        CUDA_TRY(cudaFuncGetAttributes(&faw, dram_warp_kernel));
+        CUDA_TRY(cudaFuncGetAttributes(&fa, dram_kernel<false>));
+        CUDA_TRY(cudaFuncGetAttributes(&faw, dram_warp_kernel<false>));
         LaunchPlan &p = r.plan = plan_layout(c->Nmax, r.c1 - r.c0, o->layout, sms, optin, fa.sharedSizeBytes, faw.sharedSizeBytes);
         if (!p.err.empty()) return fail(TC_EINVAL, p.err);
-        const auto kernel = p.warp ? dram_warp_kernel : dram_kernel;
+        const auto kernel = sampler_kernel(p.warp, stored_thin(o) > 1);
         CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
         CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, p.threads, p.smem));
         if (per_sm < 1) return fail(TC_EINVAL, p.warp ? "chain-per-warp kernel does not fit on this device" : "sampler kernel does not fit on this device");
@@ -2969,7 +3016,7 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
     for (auto &r : runs) {
         const int rc = setup_run(r, c, o, ld, chain_cell, chain_uid, theta0, qcov_diag, low, upp, prior_mu, prior_sig, rp);
         if (rc) return rc;
-        const auto kernel = r.plan.warp ? dram_warp_kernel : dram_kernel;
+        const auto kernel = sampler_kernel(r.plan.warp, stored_thin(o) > 1);
         CUDA_TRY(cudaEventRecord(r.e0, r.st));
         kernel<<<r.plan.grid, r.plan.threads, r.plan.smem, r.st>>>(r.a);
         CUDA_TRY(cudaGetLastError());
@@ -2978,7 +3025,8 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
     // Drain: every device's outputs go back on its own stream; with several devices one host thread per device, so the
     // device -> host copies (raw chains: GBs) of the 8 GPUs overlap instead of queueing behind each other.
     const auto t_drain0 = std::chrono::steady_clock::now();
-    const int nstore = o->nsimu - (o->n_burn - 1);
+    const int thin = stored_thin(o);
+    const size_t nkeep = thin_nkeep(o->nsimu, o->n_burn, thin), ns2 = thin_ns2(o->nsimu, thin);
     std::vector<int64_t> cnt_tmp;
     if (!counters) { cnt_tmp.assign((size_t)nchains * TC_NCOUNTERS, 0); counters = cnt_tmp.data(); }   // TC_CNT_STATUS is always checked
     std::vector<double> ksec(runs.size(), 0.0);
@@ -2996,8 +3044,8 @@ int tc_mcmc_run(const tc_cells *c, const tc_mcmc_opts *o, int nchains, const int
         if (sig) CUDA_TRY(cudaMemcpyAsync(sig + o0 * 2, a.sig, (size_t)nc * 2 * 8, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaMemcpyAsync(counters + o0 * TC_NCOUNTERS, a.counters, (size_t)nc * TC_NCOUNTERS * 8, cudaMemcpyDeviceToHost, st));
         if (o->store_chain) {
-            CUDA_TRY(cudaMemcpyAsync(chain + o0 * nstore * ld, a.chain, (size_t)nc * nstore * ld * 8, cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(cudaMemcpyAsync(s2chain + o0 * o->nsimu, a.s2chain, (size_t)nc * o->nsimu * 8, cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaMemcpyAsync(chain + o0 * nkeep * ld, a.chain, (size_t)nc * nkeep * ld * 8, cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaMemcpyAsync(s2chain + o0 * ns2, a.s2chain, (size_t)nc * ns2 * 8, cudaMemcpyDeviceToHost, st));
         }
         if (rp && rp->flags) CUDA_TRY(cudaMemcpyAsync(rp->flags + o0 * o->nsimu, a.flags, (size_t)nc * o->nsimu * 4, cudaMemcpyDeviceToHost, st));
         if (rp && rp->sschain) CUDA_TRY(cudaMemcpyAsync(rp->sschain + o0 * o->nsimu, a.sschain, (size_t)nc * o->nsimu * 8, cudaMemcpyDeviceToHost, st));

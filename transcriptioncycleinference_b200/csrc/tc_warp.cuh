@@ -393,6 +393,7 @@ __device__ __forceinline__ bool wk_propose2(const WkCtx &c, int ox, int ob, doub
 // The chain rows [r0, r1) all equal the state x (slot ox): Welford summaries with multiplicity (rows >= first_row), optional
 // chain storage, and the distinct-row buffer of the current covariance block.  (flush_run of dram_kernel, warp-local, the
 // summary vectors in L2.)
+template <bool THIN>
 __device__ __noinline__ void wk_flush(const RunArgs &a, const WkCtx &c, int ox, int r0, int r1, double wcnt, int ndist)
 {
     const int lane = threadIdx.x & 31, npar = c.npar;
@@ -401,6 +402,8 @@ __device__ __noinline__ void wk_flush(const RunArgs &a, const WkCtx &c, int ox, 
     double f1, f2;
     welford_weights(wcnt, m_w, f1, f2);
     double *grow = cov ? c.gRows + (size_t)ndist * c.ld : nullptr;
+    int j0 = rs - c.cc.first_row, nkr = m_w;
+    if (THIN && a.store_chain && a.chain) nkr = kept_rows(rs, m_w, c.cc.first_row, a.thin, j0);
 #pragma unroll 1
     for (int i = lane; i < npar; i += 32) {
         const double xo = tc_smem[ox + i];
@@ -409,9 +412,9 @@ __device__ __noinline__ void wk_flush(const RunArgs &a, const WkCtx &c, int ox, 
             __stcg(c.wmean + i, fma(d1, f1, wm));
             __stcg(c.wM2 + i, fma(d1 * d1, f2, __ldcg(c.wM2 + i)));
             if (a.store_chain && a.chain) {
-                double *dst = a.chain + ((size_t)c.ch * c.cc.nstore + (rs - c.cc.first_row)) * c.ld + i;
+                double *dst = a.chain + ((size_t)c.ch * c.cc.nkeep + j0) * c.ld + i;
 #pragma unroll 1
-                for (int r = 0; r < m_w; ++r) dst[(size_t)r * c.ld] = xo;
+                for (int r = 0; r < nkr; ++r) dst[(size_t)r * c.ld] = xo;
             }
         }
         if (cov) {
@@ -636,6 +639,7 @@ __device__ __noinline__ int wk_adapt(const RunArgs &a, const WkCtx &c, int o_mb,
 // generation, in the step loop or in adaptation at the same time — each phase's code fits the SM's instruction cache, the
 // union does not (measured without the barriers: instruction-cache hit rate 61 %, 46 % of the stall cycles waiting for
 // instructions).  Parked state between slices: scalars + counters + x in gState (the summary vectors live in L2 all along).
+template <bool THIN>
 __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_constant__ RunArgs ga)
 {
     __shared__ RunArgs a;
@@ -769,7 +773,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 for (int i = lane; i < npar; i += 32) { const double e = (tc_smem[ox + i] - __ldg(c.mu + i)) * __ldcg(c.pinv + i); sp += e * e; }
                 pri = warp_sum(sp);
                 bad0 = !isfinite(ss);
-                if (!bad0 && lane == 0) record_row0(a, ch, ss, st.t);
+                if (!bad0 && lane == 0) record_row0<THIN>(a, ch, ss, st.t);
             } else {
 #pragma unroll 1
                 for (int i = lane; i < npar; i += 32) tc_smem[ox + i] = __ldcg(gst + ST_VEC0 + i);
@@ -863,7 +867,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 if (acc) {
                     fl |= TC_FL_ACCEPT;
                     const double wcnt = st.t.wcnt;
-                    wk_flush(a, c, ox, run_r0, k, wcnt, ndist);          // close the run of the old state at row k
+                    wk_flush<THIN>(a, c, ox, run_r0, k, wcnt, ndist);          // close the run of the old state at row k
                     if (lane == 0) st.t.wcnt = wcnt + run_rows(run_r0, k, c.cc.first_row);
                     if (run_distinct(a.do_cov, run_r0, k)) ++ndist;
                     run_r0 = k;
@@ -876,7 +880,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                     tally_s2(st.t, 1.0, s2, sqrt(s2), 0.0);                 // Welford: a batch of one row
                     st.t.n_ss += nev; st.t.n_oob += noob; if (fl & TC_FL_DR) ++st.t.n_dr;
                     if (acc == 1) ++st.t.n_acc1; else if (acc == 2) ++st.t.n_acc2; else { ++st.t.rej; ++st.t.reju; }
-                    store_row(a, ch, k, s2, fl, ss);
+                    store_row<THIN>(a, ch, k, s2, fl, ss);
                 }
                 if (a.updatesigma) { sig2 = s2; is2 = s_chi * rden; }
                 __syncwarp();
@@ -888,7 +892,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
                 if (active) {
                     WK_PHASE(PH_WAIT);
                     const double wc0 = st.t.wcnt, cov_n = st.t.cov_n;
-                    wk_flush(a, c, ox, run_r0, k, wc0, ndist);           // close the run at the block boundary
+                    wk_flush<THIN>(a, c, ox, run_r0, k, wc0, ndist);           // close the run at the block boundary
                     const int nd = ndist + (run_distinct(a.do_cov, run_r0, k) ? 1 : 0);
                     const double rate = adapt_rate(a, st.t.rej, st.t.reju, k);
                     __syncwarp();
@@ -910,7 +914,7 @@ __global__ void __launch_bounds__(WK_THREADS, 1) dram_warp_kernel(const __grid_c
         __syncwarp();
         if (!bad0 && run_r0 < k) {
             const double wc0 = st.t.wcnt;
-            wk_flush(a, c, ox, run_r0, k, wc0, ndist);
+            wk_flush<THIN>(a, c, ox, run_r0, k, wc0, ndist);
             if (lane == 0) st.t.wcnt = wc0 + run_rows(run_r0, k, c.cc.first_row);
             run_r0 = k;
             __syncwarp();

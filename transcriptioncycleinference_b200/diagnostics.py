@@ -57,7 +57,8 @@ def split_rhat(chains):
 
 def ess(chains):
     """chains [m, n, p] -> effective sample size [p] of the pooled m*n draws, from the autocorrelation: rho_t = 1 -
-    (W - mean_c acov_c(t)) / V+ (BDA3 11.5), summed over Geyer's initial positive, monotone sequence of pair sums."""
+    (W - mean_c acov_c(t)) / V+ (BDA3 11.5), summed over Geyer's initial positive, monotone sequence of pair sums.
+    The draws are the rows given: for chains stored with 'thin' = k (every k-th row) it counts stored draws, at most m*n."""
     x = np.asarray(chains, dtype=np.float64)
     m, n, p = x.shape
     if n < 4:

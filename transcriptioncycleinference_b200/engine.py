@@ -95,9 +95,10 @@ class Cells:
     # ---- the DRAM fit: mcmcrun(model,data,params,options) for many chains at once
     def mcmc_run(self, opts, chain_cell, theta0, qcov_diag, low, upp, prior_mu, prior_sig, chain_uid=None,
                  replay=None, want_flags=False, chain_out=None, s2chain_out=None):
-        """chain_out / s2chain_out: optional caller-owned destinations of the raw chains ([nch, n_steps-n_burn+1, ld] and
-        [nch, n_steps] float64, C-contiguous; ideally from _lib.pinned_empty, which a caller fitting repeatedly allocates once:
-        page-locking GBs costs about as much as copying them)."""
+        """chain_out / s2chain_out: optional caller-owned destinations of the raw chains ([nch, nkeep, ld] and [nch, ns2]
+        float64, C-contiguous, with (nkeep, ns2) = _lib.stored_rows(opts): n_steps-n_burn+1 and n_steps at opts.thin = 1;
+        ideally from _lib.pinned_empty, which a caller fitting repeatedly allocates once: page-locking GBs costs about as much
+        as copying them)."""
         chain_cell = _lib.i32(chain_cell)
         nch = chain_cell.size
         arrs = [_lib.f64(x) for x in (theta0, qcov_diag, low, upp, prior_mu, prior_sig)]
@@ -108,12 +109,12 @@ class Cells:
         cnt = np.zeros((nch, _lib.NCOUNTERS), dtype=np.int64)
         chain = s2 = None
         if opts.store_chain:
-            nstore = opts.nsimu - opts.n_burn + 1
+            nkeep, ns2 = _lib.stored_rows(opts)
             # raw chains are GBs: page-locked destinations, so that the device -> host copy runs at PCIe speed (every row is
             # written by the kernel: the buffers need no zero fill)
-            chain = chain_out if chain_out is not None else _lib.pinned_empty((nch, nstore, ld))
-            s2 = s2chain_out if s2chain_out is not None else _lib.pinned_empty((nch, opts.nsimu))
-            assert chain.shape == (nch, nstore, ld) and s2.shape == (nch, opts.nsimu)
+            chain = chain_out if chain_out is not None else _lib.pinned_empty((nch, nkeep, ld))
+            s2 = s2chain_out if s2chain_out is not None else _lib.pinned_empty((nch, ns2))
+            assert chain.shape == (nch, nkeep, ld) and s2.shape == (nch, ns2)
             assert chain.dtype == np.float64 and s2.dtype == np.float64 and chain.flags.c_contiguous and s2.flags.c_contiguous
         uid = None if chain_uid is None else np.ascontiguousarray(chain_uid, dtype=np.uint64)
         rp = None

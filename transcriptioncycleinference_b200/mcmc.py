@@ -18,8 +18,12 @@ Differences that are deliberate and documented (DESIGN.md):
   * raw chains beyond MAT v5's 2 GiB per variable (the reference's own defaults on TestData are 3.1 GB) are written as
     MATLAB-readable parts `<date>-<name>_RawChain_part<K>.mat` + an index (save_raw_chains, matlab/LoadRawChains.m).
   * new optional arguments: 'files', 'previousResults', 'numChains' (default 1), 'seed',
-    'saveChains' (default True), 'verbose', 'returnResults'.  With numChains > 1 the chains of a cell are
-    pooled in MCMCresults and an extra variable MCMCdiagnostics (Rhat, n_eff per parameter) is saved.
+    'saveChains' (default True), 'thin' (default 1), 'verbose', 'returnResults'.  With numChains > 1 the chains of a
+    cell are pooled in MCMCresults and an extra variable MCMCdiagnostics (Rhat, n_eff per parameter) is saved.
+  * 'thin', k: MCMCchain keeps every k-th row — rows n_burn, n_burn + k, ... of the chain, and s2chain rows 1, 1 + k, ...
+    (MATLAB numbering) — stored on the device as a regular subsample of the same chain, so raw chains fit in memory at
+    sizes where every row would not; the raw-chain file then carries the scalar `thin`.  MCMCresults still summarise
+    every row.
 """
 import datetime
 import glob
@@ -37,7 +41,7 @@ RESULT_FIELDS = ("mean_v", "sigma_v", "mean_ton", "sigma_ton", "mean_A", "sigma_
 PLOT_FIELDS = ("t_plot", "MS2_plot", "PP7_plot", "simMS2", "simPP7")                                 # :156-157
 DIAG_FIELDS = ("cell_index", "numChains", "Rhat", "n_eff", "Rhat_max", "split_Rhat", "ESS")   # extension, only with numChains > 1
 # (Rhat, n_eff: from the device summaries, n_eff = the between-chain estimate; split_Rhat, ESS: from the raw chains — split
-# halves, autocorrelation — empty unless saveChains)
+# halves, autocorrelation — empty unless saveChains; with 'thin' > 1 from the stored rows, so ESS counts stored draws)
 CHAIN_FIELDS = ("v_chain", "ton_chain", "A_chain", "tau_chain", "MS2_basal_chain", "PP7_basal_chain", "R_chain",
                 "dR_chain", "s2chain")                                                              # :149-150
 _IDX = dict(v=0, tau=1, ton=2, MS2_basal=3, PP7_basal=4, A=5, R=6)
@@ -48,7 +52,7 @@ def parse_varargin(varargin):
     names are ignored, 'loadPrevious' is presence-only (its value, if any, is not read)."""
     o = dict(fileDir=os.getcwd(), saveLoc=os.getcwd(), numParPools=8, n_burn=10000, n_steps=20000,
              ratePriorWidth=50.0, t_start=0.0, t_end=np.inf, loadPrevious=False, construct=DEFAULT_CONSTRUCT,
-             files=None, previousResults=None, numChains=1, seed=None, saveChains=True, verbose=False,
+             files=None, previousResults=None, numChains=1, seed=None, saveChains=True, thin=1, verbose=False,
              returnResults=False)
     names = {k.lower(): k for k in o}
     for i, v in enumerate(varargin):
@@ -132,21 +136,35 @@ def _struct_array(fields, records):
 MAT5_LIMIT = 2 ** 31 - 2 ** 24          # bytes per MAT v5 variable (2 GiB), with room for the struct headers
 
 
-def save_raw_chains(save_loc, base, chain, limit=MAT5_LIMIT):
+def positive_int(value, name):
+    """An option that must be a whole number >= 1 ('thin'): an int, or a float with an integral value as MATLAB passes it."""
+    try:
+        ok = not isinstance(value, (bool, np.bool_)) and float(value) == int(value) and int(value) >= 1
+    except (TypeError, ValueError, OverflowError):
+        ok = False
+    if not ok:
+        raise ValueError("'%s' must be an integer >= 1, got %r" % (name, value))
+    return int(value)
+
+
+def save_raw_chains(save_loc, base, chain, limit=MAT5_LIMIT, thin=1):
     """`save([saveLoc,'\',filename,'_RawChain.mat'],'MCMCchain')` (:377-378).  Plain `save` writes MAT v5, whose variables
     are limited to 2 GiB — the reference's own defaults on TestData (299 cells x 10 001 rows x ~128 doubles = 3.1 GB) already
     exceed that (SURVEY 0.1 #17).  Up to the limit: the reference's single file.  Beyond it: MATLAB-readable PARTS
     `<base>_RawChain_part<K>.mat`, each a v5 file below the limit holding `MCMCchain` for a run of whole cells
     (plus `firstCell`, `lastCell`: positions in the full 1 x Ncells array), and the index `<base>_RawChain.mat` with
     `MCMCchainParts` (file names), `MCMCchainPartOfCell` (1 x Ncells) and `nParts`; matlab/LoadRawChains.m puts them back
-    together.  Returns the list of files written."""
+    together.  thin > 1 (rows thinned on the device, 'thin') adds the scalar `thin` next to `MCMCchain` in every file that
+    holds it and in the index; thin = 1 writes the variables above and nothing else.  Returns the list of files written."""
     import scipy.io as sio
     sizes = [sum(np.asarray(v).nbytes for v in c.values()) for c in chain]
     if any(b > limit for b in sizes):
-        raise ValueError("the raw chain of one cell (%d bytes) exceeds the MAT v5 variable limit: thin it or lower n_steps" % max(sizes))
+        raise ValueError("the raw chain of one cell (%d bytes) exceeds the MAT v5 variable limit: store fewer rows with the "
+                         "option 'thin' or lower n_steps" % max(sizes))
+    extra = dict(thin=float(thin)) if thin > 1 else {}
     path = os.path.join(save_loc, base + "_RawChain.mat")
     if sum(sizes) <= limit:
-        sio.savemat(path, dict(MCMCchain=_struct_array(CHAIN_FIELDS, chain)))
+        sio.savemat(path, dict(MCMCchain=_struct_array(CHAIN_FIELDS, chain), **extra))
         return [path]
     groups, cur, cur_b = [], [], 0
     for i, b in enumerate(sizes):
@@ -158,10 +176,11 @@ def save_raw_chains(save_loc, base, chain, limit=MAT5_LIMIT):
     for k, idx in enumerate(groups, start=1):
         fn = "%s_RawChain_part%d.mat" % (base, k)
         sio.savemat(os.path.join(save_loc, fn), dict(MCMCchain=_struct_array(CHAIN_FIELDS, [chain[i] for i in idx]),
-                                                     firstCell=float(idx[0] + 1), lastCell=float(idx[-1] + 1), part=float(k)))
+                                                     firstCell=float(idx[0] + 1), lastCell=float(idx[-1] + 1), part=float(k),
+                                                     **extra))
         files.append(fn); part_of[0, idx] = k
     sio.savemat(path, dict(MCMCchainParts=np.array(files, dtype=object).reshape(-1, 1), MCMCchainPartOfCell=part_of,
-                           nParts=float(len(groups))))
+                           nParts=float(len(groups)), **extra))
     return [path] + [os.path.join(save_loc, f) for f in files]
 
 
@@ -170,6 +189,7 @@ def fit_dataset(cells_in, o, devices):
     MCMCresults, MCMCplot) as lists of dicts, already stripped of skipped cells (:360-369)."""
     n_burn, n_steps = int(o["n_burn"]), int(o["n_steps"])
     nchains = int(o["numChains"])
+    thin = positive_int(o["thin"], "thin")
     rng = np.random.default_rng(o["seed"])
     prev = o.get("_prev")                                   # {cell_index: (mean_v, ApprovedFits)} or None
     kept, ts, m2s, p7s = [], [], [], []
@@ -193,7 +213,7 @@ def fit_dataset(cells_in, o, devices):
             np.tile(np.arange(nchains, dtype=np.uint64), len(kept))
         opts = _lib.default_opts(nsimu=n_steps, burnintime=n_burn, n_burn=n_burn,
                                  store_chain=1 if o["saveChains"] else 0, ngpus=len(devices),
-                                 seed=int(rng.integers(0, 2 ** 63 - 1)))
+                                 seed=int(rng.integers(0, 2 ** 63 - 1)), thin=thin)
         out = cells.mcmc_run(opts, cc, *inputs, chain_uid=uid)
         # pool the chains of a cell (numChains > 1 is an extension; with 1 chain this is the identity)
         MCMCchain, MCMCresults, MCMCplot = [], [], []
@@ -208,17 +228,20 @@ def fit_dataset(cells_in, o, devices):
             if o["saveChains"]:
                 ch = out["chain"][sl, :, :npar].reshape(-1, npar)
                 s2 = out["s2chain"][sl].reshape(-1)
-                mean_sigma, sigma_sigma = float(np.sqrt(s2.mean())), float(np.sqrt(s2).std())
                 MCMCchain.append(dict(
                     v_chain=ch[:, [_IDX["v"]]], ton_chain=ch[:, [_IDX["ton"]]], A_chain=ch[:, [_IDX["A"]]],
                     tau_chain=ch[:, [_IDX["tau"]]], MS2_basal_chain=ch[:, [_IDX["MS2_basal"]]],
                     PP7_basal_chain=ch[:, [_IDX["PP7_basal"]]], R_chain=ch[:, [_IDX["R"]]], dR_chain=ch[:, 7:],
                     s2chain=s2.reshape(-1, 1)))
             else:
+                MCMCchain.append({f: np.zeros((0, 0)) for f in CHAIN_FIELDS})
+            if o["saveChains"] and thin == 1:
+                mean_sigma, sigma_sigma = float(np.sqrt(s2.mean())), float(np.sqrt(s2).std())
+            else:
+                # sig of every row, from the device (a thinned s2chain holds only some of them)
                 sg = out["sig"][sl]
                 mean_sigma = float(np.sqrt((sg[:, 0] ** 2).mean()))
                 sigma_sigma = float(sg[:, 1].mean()) if nchains == 1 else float(np.sqrt((sg[:, 1] ** 2).mean()))
-                MCMCchain.append({f: np.zeros((0, 0)) for f in CHAIN_FIELDS})
             means.append(mean)
             if nchains > 1:
                 # order of theta: [v, tau, ton, MS2_basal, PP7_basal, A, R, dR_1..dR_N]
@@ -256,6 +279,7 @@ def TranscriptionCycleMCMC(*varargin):
     import scipy.io as sio
     o = parse_varargin(varargin)
     get_construct(o["construct"])                          # unknown construct: fail before any work
+    positive_int(o["thin"], "thin")
     if int(o["n_burn"]) < 1 or int(o["n_burn"]) > int(o["n_steps"]):
         raise IndexError("n_burn must satisfy 1 <= n_burn <= n_steps (chain(n_burn:end,:))")
     ndev = _lib.device_count()
@@ -297,7 +321,7 @@ def TranscriptionCycleMCMC(*varargin):
             mat["MCMCdiagnostics"] = _struct_array(DIAG_FIELDS, diags)
         sio.savemat(os.path.join(save_loc, base + ".mat"), mat)
         if o["saveChains"]:
-            save_raw_chains(save_loc, base, chain)
+            save_raw_chains(save_loc, base, chain, thin=int(o["thin"]))
         ret.append(dict(DatasetName=name, MCMCresults=results, MCMCplot=plot, MCMCchain=chain, MCMCdiagnostics=diags))
     print("MCMC analysis complete. Information stored in: %s" % save_loc)
     return ret if o["returnResults"] else None
